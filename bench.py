@@ -3,6 +3,8 @@
 
     python bench.py --gpus N --steps K --warmup W            our arm (CUDA, through the C ABI)
     python bench.py --impl reference --gpus N --steps K ...   the reference's own CPU code (oracle/_ref), same workload
+    python bench.py ... --dump-outputs DIR                    also write the last timed step's outputs as DIR/*.npy: the inputs
+                                                              are seeded, so two builds can be compared output for output
 
 Workload (BASELINE.json configs[1]): hg38 Micro-C 150-cycle stitched-read SAM ("flash" mode), 100 M read groups per
 GPU, synthetic (microcket_b200/csrc/synth.h), sam2pairs + coordinate dedup + 5 kb binning.  One step = one pass of
@@ -58,8 +60,50 @@ DUP_PER_1024 = 128          # 12.5 % of the read groups re-use the fragment of a
                             # with their own read ids, crossing shard boundaries): ~11 % of the pairs are removed by the dedup
 
 
+DUMP_ROWS = 1 << 19         # --dump-outputs keeps at most this many rows of each array (a quarter of it for each of the nine COOs of
+                            # --config multires): the largest dump (--config multires --sam) is 61.9 MB of .npy files
+
+
 def synth_opts(mk, universe):
     return mk.synth_opts(dup_per_1024=DUP_PER_1024, dup_universe=universe, chimeric_per_1024=WL["chimeric"])
+
+
+def dump_rows(torch, np, t, n, rows=None):
+    """the first n rows of tensor t on the host: all of them when n <= rows (default DUMP_ROWS), else a sample drawn with the
+    workload's seed (so the same n gives the same rows in every run and every build), in output order"""
+    rows = rows or DUMP_ROWS
+    idx = np.arange(n) if n <= rows else np.sort(np.random.default_rng(SEED).choice(n, rows, replace=False))
+    return t[:n][torch.from_numpy(idx).to(t.device)].cpu().numpy()
+
+
+def write_dump(d, np, arrays):
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), a)
+    print(f"[bench] --dump-outputs: {', '.join(f'{k}{list(v.shape)}' for k, v in arrays.items())} -> {d}", file=sys.stderr)
+
+
+def dump_pipeline(d, torch, np, mk, pipe, n_pairs, kept, nnz, st, text_len):
+    """--dump-outputs: what the last timed step handed its caller (rank 0's share when N > 1).  Integers as float64 (positions
+    exceed float32's 24-bit mantissa), text bytes as float32."""
+    kp = pipe.pairs if pipe.src_ptr == pipe.pairs.data_ptr() else pipe.kept_pairs(kept)
+    rec = np.frombuffer(dump_rows(torch, np, kp.view(-1, 16), kept).tobytes(), dtype=mk.PAIR_DTYPE)
+    coo_rows = DUMP_ROWS // 4 if pipe.multires else DUMP_ROWS
+    coo = lambda a, b, c, z: np.stack([dump_rows(torch, np, x, z, coo_rows) for x in (a, b, c)], axis=1).astype(np.float64)
+    arrays = {"counts": np.array([n_pairs, kept, nnz], dtype=np.float64),          # pairs emitted, pairs kept by the dedup, COO cells
+              "s2p_log": np.array([getattr(st, f) for f in ("lowMap", "manyHits", "unpaired", "selfCircle", "trans", "cis10K", "cis1K", "cis0")],
+                                  dtype=np.float64),
+              f"coo_{RES}": coo(pipe.b1, pipe.b2, pipe.cnt, nnz),                    # bin1, bin2, count
+              "kept_pairs": np.stack([rec[f].astype(np.float64) for f in mk.PAIR_DTYPE.names], axis=1),   # columns: PAIR_DTYPE's fields
+              "pairs_text": dump_rows(torch, np, pipe.text, text_len).astype(np.float32)}
+    if SAM_ON:
+        arrays["sam_text"] = dump_rows(torch, np, pipe.samout, pipe.sam_len).astype(np.float32)
+    if pipe.multires:                               # the other eight resolutions: their cell counts and their COOs
+        cells = {r: c for r, c in pipe.multires_cells.items() if c is not None}
+        arrays["multires_cells"] = np.array(sorted(cells.items()), dtype=np.float64)
+        for r, (b1, b2, c) in pipe.mcoo.items():
+            arrays[f"coo_{r}"] = coo(b1, b2, c, cells[r])
+    write_dump(d, np, arrays)
 
 
 def measured_peak():
@@ -275,10 +319,12 @@ class Pipeline:
         ev[1].record()
         cells = {RES: None}
         for k, r in enumerate(self.dense_res):
-            cells[r], _ = self.hist.coo(k, self.m1.data_ptr(), self.m2.data_ptr(), self.mc.data_ptr(), self.cap_pairs, stream=self.stream)
+            b1, b2, c = self.mcoo[r]
+            cells[r], _ = self.hist.coo(k, b1.data_ptr(), b2.data_ptr(), c.data_ptr(), b1.numel(), stream=self.stream)
         ev[2].record()
         for r in self.sparse_res:
-            cells[r] = self.ws.bin(kept_ptr, kept, WL["lens"], r, self.m1.data_ptr(), self.m2.data_ptr(), self.mc.data_ptr(), self.cap_pairs, stream=self.stream)
+            b1, b2, c = self.mcoo[r]
+            cells[r] = self.ws.bin(kept_ptr, kept, WL["lens"], r, b1.data_ptr(), b2.data_ptr(), c.data_ptr(), b1.numel(), stream=self.stream)
         ev[3].record()
         self.multires_events.append(ev)
         self.multires_cells = cells
@@ -289,7 +335,10 @@ class Pipeline:
         self.dense_res = [r for r in DEFAULT_RES if r >= 100000]
         self.sparse_res = [r for r in DEFAULT_RES if r < 100000 and r != RES]
         self.hist = mk.Hist(WL["lens"], self.dense_res, device=self.b1.device.index)
-        self.m1 = torch.empty_like(self.b1); self.m2 = torch.empty_like(self.b1); self.mc = torch.empty_like(self.b1)
+        # COO buffers of their own per resolution (a dense one needs no more rows than its triangle has cells), so that a step
+        # leaves all nine resolutions' counts behind, as a caller receives them
+        rows = lambda r: min(self.cap_pairs, mk.Hist.cells(WL["lens"], r)[1])
+        self.mcoo = {r: [torch.empty(rows(r), dtype=torch.int32, device=self.b1.device) for _ in range(3)] for r in self.dense_res + self.sparse_res}
         self.multires_events, self.multires_cells = [], {}
 
     def kept_pairs(self, kept):
@@ -490,7 +539,7 @@ def run_krmdup(args):
                 break
             a += n1.value; b += n2.value
         stt = kd.finish()
-        return stt, a + b
+        return stt, a, b
 
     def barrier():
         if dist is not None:
@@ -505,10 +554,16 @@ def run_krmdup(args):
         clocks.start()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        stt, out_bytes = once()
+        stt, n_out1, n_out2 = once()
     barrier()
     sec = (time.perf_counter() - t0) / args.steps
     clk = clocks.stop() if rank == 0 else None
+    out_bytes = n_out1 + n_out2
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        write_dump(args.dump_outputs, np, {"krmdup_log": np.array([stt.uniq, stt.dup, stt.discard], dtype=np.float64),
+                                           "read1_fastq": dump_rows(torch, np, out1, n_out1).astype(np.float32),
+                                           "read2_fastq": dump_rows(torch, np, out2, n_out2).astype(np.float32)})
     t = torch.tensor([sec, float(stt.pairs), float(nb), float(out_bytes), float(stt.uniq), float(stt.dup)], dtype=torch.float64, device=dev)
     if dist is not None:
         tmax = t.clone(); dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
@@ -559,7 +614,14 @@ def main():
                          "SAM's primary records before grouping - pinned by the reference binaries - then binning")
     ap.add_argument("--no-verify", action="store_true", help="skip the untimed, asserted reduced-size verification of the N-GPU path")
     ap.add_argument("--verify-groups", type=int, default=200_000, help="read groups per GPU of that verification")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to DIR/<name>.npy "
+                                                          "(float64 / float32, a seeded sample of at most %d rows per array, %d per COO "
+                                                          "with --config multires)" % (DUMP_ROWS, DUMP_ROWS // 4))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's outputs: it goes with --impl ours")
     global WL, SAM_ON, DEDUP_SEQ
     WL = WORKLOADS[args.config]; SAM_ON = args.sam; DEDUP_SEQ = args.dedup == "seq"
     if DEDUP_SEQ and args.config == "multires":
@@ -633,6 +695,8 @@ def main():
     launches = s2p.launches() + ws.launches() - launches0
     s2p.enable_timing(False)
     st = s2p.finish(0, 0) if world > 1 else s2p.finish()
+    if args.dump_outputs and rank == 0:
+        dump_pipeline(args.dump_outputs, torch, np, mk, pipe, n_pairs, kept, nnz, st, text_len[0])
     # size-independent properties of the last timed step, at full size (reported, not asserted: the parity tests are tests/):
     # every emitted pair is counted in exactly one class counter; the COO counts add up to the pairs kept by the dedup
     checks = None
@@ -737,7 +801,7 @@ def main():
             path, nb = reference_sample(torch, mk, args.cpu_groups, local, tmpdir, universe)
             threads = max(2, min(host_cores(), 8))
             p, sec, kind = cpu_pipeline_once(path, tmpdir, threads)
-            cpu = {"value": p / sec, "unit": "pairs/s", "cores": threads, "kind": kind, "host_cores": host_cores(),
+            cpu = {"value": p / sec, "unit": "pairs/s", "cores": threads, "kind": kind, "host_cores": host_cores(), "passes": 1,   # not --steps: a pass takes tens of seconds
                    "sample": f"{args.cpu_groups} read groups ({nb / 1e9:.2f} GB SAM) of the same workload, one pass, {sec:.1f} s: "
                              f"reference sam2pairs (T={threads}) + oracle dedup/binning (1 thread)"}
         finally:
@@ -911,7 +975,7 @@ def measure_e2e(torch, mk, np, dist, args, world, rank, local):
         once()
     for k in phases:
         phases[k] = 0.0
-    reps = max(2, min(args.steps, 3))
+    reps = args.steps
     barrier()
     t0 = time.perf_counter()
     for _ in range(reps):
