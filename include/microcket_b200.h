@@ -270,6 +270,43 @@ int  mk_hist_coo_device(mk_hist *, int res_idx, uint32_t *d_bin1, uint32_t *d_bi
 uint64_t mk_hist_dropped(mk_hist *);
 uint64_t mk_hist_launch_count(mk_hist *);
 
+/* ------------------------------------------------------------------ matrix balancing (normalisation vectors) */
+/* The VC, VC_SQRT and KR vectors `juicer_tools pre` stores in a .hic (microcket:525-529), per chromosome, from its
+ * intra-chromosomal matrix A (symmetric, diagonal counted once; bins as in the COO: len / res + 1 per chromosome).
+ *   VC       n_i = sum_j A_ij; VC_SQRT = sqrt(VC); empty rows 0
+ *   KR       Knight-Ruiz bnewt (tol 1e-6, delta 0.1, Delta 3, etamax 0.1, g 0.9) on the rows with a nonzero sum, n_i = 1 / x_i;
+ *            NaN on the rows left out.  A chromosome FAILS when it has not converged after 100 outer steps, some x_i is <= 0
+ *            or not finite, or its matrix has no doubly-stochastic scaling; a failed chromosome's KR entries are all NaN.
+ * Every vector is then multiplied per chromosome by juicer's sum factor sqrt(sum c/(n_x n_y) / sum c) over the entries with
+ * valid norms (off-diagonal entries twice), so that the normalised matrix sums to the raw one.  No floating-point atomics:
+ * the same input gives the same bits.  PARITY UNPINNED (juicer_tools is absent; DESIGN.md §5). */
+typedef struct mk_norm mk_norm;
+#define MK_NORM_VC       1
+#define MK_NORM_VC_SQRT  2
+#define MK_NORM_KR       4
+typedef struct {
+    uint32_t kr_outer_max;      /* most outer (Newton) steps any chromosome took */
+    uint32_t kr_matvecs;        /* lockstep KR steps = products over all unfinished chromosomes at once */
+    uint32_t kr_failed;         /* chromosomes whose KR failed */
+    double   kr_residual_max;   /* largest ||1 - x (A x)||_2 of the balanced chromosomes */
+} mk_norm_stats;
+/* One object per resolution; max_nnz: the most COO entries a call may pass (below 2^30: one radix sort call). */
+int  mk_norm_create(int device, const uint32_t *chrom_len, int n_chrom, uint32_t res, size_t max_nnz, mk_norm **);
+void mk_norm_destroy(mk_norm *);
+/* One resolution's COO as mk_pairs_bin_device / mk_hist_coo_device return it (device, sorted by (bin1, bin2), bin1 <= bin2).
+ * types: MK_NORM_* bits; d_vc / d_vc_sqrt / d_kr: n_bins doubles each on the device, global bin order (may be NULL when the
+ * type is not requested).  chrom_status (host, n_chrom, may be NULL): 0 ok, 1 no intra contacts (no vector of any type),
+ * 2 KR failed.  Refused: nnz > max_nnz (MK_ERR_CAPACITY); bin1 > bin2, a bin past the resolution's bins, an unsorted COO
+ * (MK_ERR_ARG). */
+int  mk_norm_device(mk_norm *, const uint32_t *d_bin1, const uint32_t *d_bin2, const uint32_t *d_cnt, size_t nnz, int types,
+                    double *d_vc, double *d_vc_sqrt, double *d_kr, uint8_t *chrom_status, mk_norm_stats *, void *stream);
+uint64_t mk_norm_launch_count(mk_norm *);
+/* Optional timing (tools/norm_bench.py): CUDA events on the stream, host clock for the KR loop.  ms[k] / count[k], arrays of 8:
+ * 0 CSR build, 1 products inside KR, 2 KR vector kernels (pre + post), 3 KR loop wall time incl. the host round trips
+ * (count = steps), 4 products outside KR (row sums, sum factors), 5 other vector kernels, 6-7 unused. */
+int  mk_norm_enable_timing(mk_norm *, int on);
+int  mk_norm_kernel_times(mk_norm *, double *ms, uint64_t *count);
+
 /* ------------------------------------------------------------------ multi-GPU exchange over NVLink peer memory */
 /* One object per rank (one process per GPU, or several ranks in one process).  Owner bucketing and the all-to-all are ONE
  * kernel: owner = mix(chr1, chr2, pos1 / res) mod world (mk_pairs_owner); every rank writes its pairs straight into the

@@ -6,6 +6,6 @@ bench.py: a ctypes binding that mirrors the C ABI one to one.  There is no CPU f
 every compute call raises if the CUDA library or a GPU is missing.
 """
 from .capi import (MkError, Lib, lib, build, S2PConfig, Sam2Pairs, Krmdup, PairsWorkspace, synth_host,  # noqa: F401
-                   synth_device, synth_opts, SynthOpts, chrom_ranks, Hist, Xchg, LIB_PATH, PAIR_DTYPE)
+                   synth_device, synth_opts, SynthOpts, chrom_ranks, Hist, Norm, NormStats, NORM_TYPES, Xchg, LIB_PATH, PAIR_DTYPE)
 
-__all__ = ["MkError", "Lib", "lib", "build", "S2PConfig", "Sam2Pairs", "Krmdup", "PairsWorkspace", "synth_host", "synth_device", "synth_opts", "SynthOpts", "chrom_ranks", "Hist", "Xchg", "LIB_PATH", "PAIR_DTYPE"]
+__all__ = ["MkError", "Lib", "lib", "build", "S2PConfig", "Sam2Pairs", "Krmdup", "PairsWorkspace", "synth_host", "synth_device", "synth_opts", "SynthOpts", "chrom_ranks", "Hist", "Norm", "NormStats", "NORM_TYPES", "Xchg", "LIB_PATH", "PAIR_DTYPE"]

@@ -54,6 +54,13 @@ def synth_opts(dup_per_1024=0, dup_universe=0, chimeric_per_1024=-1, noise_per_1
     return SynthOpts(dup_per_1024, dup_universe, chimeric_per_1024, noise_per_1024, selfcircle_per_1024)
 
 
+class NormStats(C.Structure):
+    _fields_ = [("kr_outer_max", C.c_uint32), ("kr_matvecs", C.c_uint32), ("kr_failed", C.c_uint32), ("kr_residual_max", C.c_double)]
+
+
+NORM_TYPES = {"VC": 1, "VC_SQRT": 2, "KR": 4}
+
+
 class DedupCfg(C.Structure):
     _fields_ = [("hskip1", C.c_int), ("klen1", C.c_int), ("hskip2", C.c_int), ("klen2", C.c_int), ("device", C.c_int),
                 ("window_bytes", C.c_size_t), ("async_pull", C.c_int)]
@@ -145,7 +152,11 @@ class Lib:
                            ("mk_xchg_launch_count", [vp]), ("mk_xchg_begin", [vp]), ("mk_xchg_end_device", [vp, vp]),
                            ("mk_xchg_scatter_part_device", [vp, vp, vp, C.c_uint32, vp]),
                            ("mk_pairs_partition_device", [vp, vp, sz, i, C.c_uint32, vp, P(u64), vp]),
-                           ("mk_pairs_launch_count", [vp])):
+                           ("mk_pairs_launch_count", [vp]),
+                           ("mk_norm_create", [i, P(C.c_uint32), i, C.c_uint32, sz, P(vp)]), ("mk_norm_destroy", [vp]),
+                           ("mk_norm_device", [vp, vp, vp, vp, sz, i, vp, vp, vp, P(C.c_uint8), P(NormStats), vp]),
+                           ("mk_norm_launch_count", [vp]), ("mk_norm_enable_timing", [vp, i]),
+                           ("mk_norm_kernel_times", [vp, P(C.c_double), P(u64)])):
             if hasattr(L, name):
                 getattr(L, name).argtypes = args
         if hasattr(L, "mk_pairs_owner"):
@@ -155,7 +166,7 @@ class Lib:
             L.mk_pairs_launch_count.restype = u64
         if hasattr(L, "mk_pairs_dropped"):
             L.mk_pairs_dropped.restype = u64
-        for name in ("mk_hist_dropped", "mk_hist_launch_count", "mk_xchg_launch_count"):
+        for name in ("mk_hist_dropped", "mk_hist_launch_count", "mk_xchg_launch_count", "mk_norm_launch_count"):
             if hasattr(L, name):
                 getattr(L, name).restype = u64
 
@@ -550,6 +561,55 @@ class Hist:
 
     def launches(self):
         return self.lib.L.mk_hist_launch_count(self.h)
+
+
+class Norm:
+    """Balancing of one resolution's contact matrices (csrc/norm.cu): VC, VC_SQRT and KR vectors per chromosome from the COO."""
+
+    def __init__(self, chrom_len, res, max_nnz, device=0):
+        self.lib = lib()
+        self.lib.require_gpu()
+        self.chrom_len, self.res = list(chrom_len), res
+        self.n_bins = sum(l // res + 1 for l in self.chrom_len)
+        cl = (C.c_uint32 * len(chrom_len))(*chrom_len)
+        self.h = C.c_void_p()
+        self.lib.check(self.lib.L.mk_norm_create(device, cl, len(chrom_len), res, max_nnz, C.byref(self.h)))
+
+    def run(self, d_bin1, d_bin2, d_cnt, nnz, types=("VC", "VC_SQRT", "KR"), d_vc=0, d_vc_sqrt=0, d_kr=0, stream=0):
+        """device COO in, n_bins doubles per requested type written to the device pointers -> (chrom_status list, NormStats)"""
+        mask = 0
+        for t in types:
+            mask |= NORM_TYPES[t]
+        status = (C.c_uint8 * len(self.chrom_len))()
+        st = NormStats()
+        self.lib.check(self.lib.L.mk_norm_device(self.h, d_bin1, d_bin2, d_cnt, nnz, mask, d_vc or None, d_vc_sqrt or None, d_kr or None,
+                                                 status, C.byref(st), stream))
+        return list(status), st
+
+    def launches(self):
+        return self.lib.L.mk_norm_launch_count(self.h)
+
+    def enable_timing(self, on=True):
+        self.lib.check(self.lib.L.mk_norm_enable_timing(self.h, int(on)))
+
+    def kernel_times(self):
+        """-> {name: (ms, count)}: CUDA events around the kernels, host clock around the KR loop"""
+        ms = (C.c_double * 8)()
+        cnt = (C.c_uint64 * 8)()
+        self.lib.check(self.lib.L.mk_norm_kernel_times(self.h, ms, cnt))
+        names = ("build", "kr_product", "kr_vector", "kr_wall", "product", "vector")
+        return {n: (ms[k], cnt[k]) for k, n in enumerate(names)}
+
+    def close(self):
+        if self.h:
+            self.lib.L.mk_norm_destroy(self.h)
+            self.h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 class Xchg:

@@ -12,6 +12,9 @@
 // -H <out.hic> also packs every resolution's counts into one `.hic` (version 8) container, i.e. the file the driver's
 // `juicer_tools pre` call produces (host code over the arrays copied back for the .coo files: hic_writer.hpp; -g names the
 // genome in its header, default: the .info file's stem).
+// -n <types> (with -H; any of VC,VC_SQRT,KR, comma separated) also balances every resolution's matrices on the GPU (norm.cu,
+// mk_norm_device on the COO while it is still in device memory) and stores the normalisation vectors and the normalised
+// expected values in the container, what `juicer_tools pre` computes by default (and `addNorm` adds to a file without them).
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -27,12 +30,47 @@ using namespace std;
 #define CHECK(call) do { if ((call) != MK_OK) { cerr << "Error: " << mk_last_error() << "\n"; return 20; } } while (0)
 
 static hic::Writer *g_hic = NULL;                                         // -H: every resolution's arrays also go into the container
+static int g_norm_types = 0, g_dev = 0;                                   // -n: MK_NORM_* bits
+static vector<uint32_t> g_len; static vector<string> g_names;
+
+// -n: the resolution's normalisation vectors from its device COO, copied to the host for the writer
+static int balance(uint32_t res, const void *d_b1, const void *d_b2, const void *d_ct, size_t nnz, vector<vector<double>> &vals, vector<hic::NormInput> &norms) {
+    static const char *names[3] = {"VC", "VC_SQRT", "KR"};
+    uint64_t nb = 0; CHECK(mk_hist_cells(g_len.data(), (int)g_len.size(), res, &nb, NULL));
+    mk_norm *nm = NULL;
+    CHECK(mk_norm_create(g_dev, g_len.data(), (int)g_len.size(), res, nnz, &nm));
+    void *d_out[3] = {NULL, NULL, NULL};
+    for (int t = 0; t < 3; ++t) if (g_norm_types & (1 << t)) CHECK(mk_dev_alloc(g_dev, nb * 8 + 8, &d_out[t]));
+    vector<uint8_t> status(g_len.size(), 0); mk_norm_stats st;
+    CHECK(mk_norm_device(nm, (const uint32_t *)d_b1, (const uint32_t *)d_b2, (const uint32_t *)d_ct, nnz, g_norm_types,
+                         (double *)d_out[0], (double *)d_out[1], (double *)d_out[2], status.data(), &st, NULL));
+    mk_norm_destroy(nm);
+    vals.assign(3, vector<double>());
+    for (int t = 0; t < 3; ++t) {
+        if (!d_out[t]) continue;
+        vals[t].resize(nb);
+        CHECK(mk_copy_to_host(vals[t].data(), d_out[t], nb * 8));
+        mk_dev_free(d_out[t]);
+        hic::NormInput q; q.type = names[t]; q.values = vals[t].data();
+        for (size_t c = 0; c < g_len.size(); ++c) q.stored.push_back(status[c] == 0 || (status[c] == 2 && t < 2));
+        norms.push_back(q);
+    }
+    if (g_norm_types & MK_NORM_KR) {
+        string failed;
+        for (size_t c = 0; c < g_len.size(); ++c) if (status[c] == 2) failed += (failed.empty() ? "" : ", ") + g_names[c];
+        cerr << "INFO: KR at " << res << " bp: " << st.kr_matvecs << " steps, " << st.kr_failed << " chromosome(s) failed"
+             << (failed.empty() ? "" : ": " + failed) << ".\n";
+    }
+    return 0;
+}
 
 static int write_coo(const string &prefix, uint32_t res, const void *d_b1, const void *d_b2, const void *d_ct, size_t nnz) {
     const string path = prefix + "." + to_string(res) + ".coo";
+    vector<vector<double>> vals; vector<hic::NormInput> norms;           // before the copy: the device arrays are reused afterwards
+    if (g_norm_types) if (int rc = balance(res, d_b1, d_b2, d_ct, nnz, vals, norms)) return rc;
     vector<uint32_t> b1(nnz + 1), b2(nnz + 1), ct(nnz + 1);
     if (nnz) { CHECK(mk_copy_to_host(b1.data(), d_b1, nnz * 4)); CHECK(mk_copy_to_host(b2.data(), d_b2, nnz * 4)); CHECK(mk_copy_to_host(ct.data(), d_ct, nnz * 4)); }
-    if (g_hic) { string err; if (g_hic->add(res, b1.data(), b2.data(), ct.data(), nnz, &err)) { cerr << "Error: " << err << "\n"; return 10; } }
+    if (g_hic) { string err; if (g_hic->add(res, b1.data(), b2.data(), ct.data(), nnz, &err, g_norm_types ? &norms : NULL)) { cerr << "Error: " << err << "\n"; return 10; } }
     FILE *fo = fopen(path.c_str(), "w");
     if (!fo) { cerr << "Error: cannot write " << path << "\n"; return 10; }
     static char big[1 << 22];
@@ -43,7 +81,7 @@ static int write_coo(const string &prefix, uint32_t res, const void *d_b1, const
 }
 
 int main(int argc, char *argv[]) {
-    bool dedup = false, bins_bed = false; string reslist, hic_path, genome;
+    bool dedup = false, bins_bed = false; string reslist, hic_path, genome, normlist;
     int a = 1;
     while (a < argc && argv[a][0] == '-' && argv[a][1]) {
         if (!strcmp(argv[a], "-d")) { dedup = true; ++a; }
@@ -51,10 +89,20 @@ int main(int argc, char *argv[]) {
         else if (!strcmp(argv[a], "-r") && a + 1 < argc) { reslist = argv[a + 1]; a += 2; }
         else if (!strcmp(argv[a], "-H") && a + 1 < argc) { hic_path = argv[a + 1]; a += 2; }
         else if (!strcmp(argv[a], "-g") && a + 1 < argc) { genome = argv[a + 1]; a += 2; }
+        else if (!strcmp(argv[a], "-n") && a + 1 < argc) { normlist = argv[a + 1]; a += 2; }
         else break;
     }
-    if (argc - a < 3 || reslist.empty()) {
-        cerr << "\nUsage: " << argv[0] << " [-d] [-b] [-H <out.hic>] [-g <genomeId>] -r <res[,res...]> <in.pairs|-> <out.prefix> <genome.info>\n\n";
+    if (!normlist.empty()) {
+        stringstream ss(normlist); string t;
+        while (getline(ss, t, ',')) {
+            if (t == "VC") g_norm_types |= MK_NORM_VC;
+            else if (t == "VC_SQRT") g_norm_types |= MK_NORM_VC_SQRT;
+            else if (t == "KR") g_norm_types |= MK_NORM_KR;
+            else { cerr << "Error: unknown normalisation '" << t << "' (VC, VC_SQRT, KR)\n"; return 2; }
+        }
+    }
+    if (argc - a < 3 || reslist.empty() || (!normlist.empty() && hic_path.empty())) {
+        cerr << "\nUsage: " << argv[0] << " [-d] [-b] [-H <out.hic> [-n VC,VC_SQRT,KR]] [-g <genomeId>] -r <res[,res...]> <in.pairs|-> <out.prefix> <genome.info>\n\n";
         return 2;
     }
     vector<uint32_t> res;
@@ -87,6 +135,7 @@ int main(int argc, char *argv[]) {
     FILE *fp = strcmp(argv[a], "-") ? fopen(argv[a], "rb") : stdin;
     if (!fp) { cerr << "Error: cannot read " << argv[a] << "\n"; return 10; }
     const int dev = getenv("MICROCKET_DEVICE") ? atoi(getenv("MICROCKET_DEVICE")) : 0;
+    g_dev = dev; g_len = chr_len; g_names = names;
     if (mk_device_count() < 1) { cerr << "Error: no CUDA device: microcket_b200 has no CPU fallback\n"; return 20; }
 
     // ---- stream the text to the GPU and parse it there

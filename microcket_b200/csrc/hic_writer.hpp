@@ -2,7 +2,8 @@
 // (SURVEY.md §8(f)-3; stands where the driver runs `java -jar juicer_tools.jar pre -r <res,...> <sid>.final.pairs <sid>.hic
 // <genome>.info`, microcket:525-529).  Host code only: the counting is done on the GPU (pairs.cu / hist.cu), this file
 // lays the counts out in the container: header, one matrix per chromosome pair with every resolution's compressed blocks,
-// footer with the master index and the expected-value vectors.
+// footer with the master index and the expected-value vectors, and — when normalisation vectors are handed in with a
+// resolution (norm.cu) — the normalised expected values and the vectors themselves.
 //
 // PARITY UNPINNED: juicer_tools is a third-party jar that is not in /root/reference and cannot run here (SURVEY §8c); the
 // layout follows the published .hic v8 format description and is read back in tests/ by an independent reader written from
@@ -143,6 +144,10 @@ static inline void expected_values(uint32_t bin_size, const std::vector<uint32_t
     }
 }
 
+// one resolution's normalisation vector of one type (mk_norm_device's output): values in global bin order, and per chromosome
+// whether it has a vector at all (none without intra contacts, none where KR failed)
+struct NormInput { std::string type; const double *values; std::vector<bool> stored; };
+
 class Writer {
 public:
     // chromosomes in .info order; resolutions in any order (the file lists them coarse to fine, as juicer does)
@@ -160,7 +165,10 @@ public:
 
     // one resolution's COO as pairs2bins writes it: global bin ids (bin = offset[chr] + pos / res, len / res + 1 bins per
     // chromosome, .info order), upper triangle, sorted by (bin1, bin2)
-    int add(uint32_t res, const uint32_t *b1, const uint32_t *b2, const uint32_t *ct, size_t nnz, std::string *err) {
+    // norms (may be NULL): the resolution's normalisation vectors; the normalised expected values are made here from the
+    // same entries, with c / (n_x n_y) for the counts and only the entries whose two norms are valid (finite, > 0)
+    int add(uint32_t res, const uint32_t *b1, const uint32_t *b2, const uint32_t *ct, size_t nnz, std::string *err,
+            const std::vector<NormInput> *norms = nullptr) {
         int ri = -1; for (size_t k = 0; k < res_.size(); ++k) if (res_[k] == res) ri = (int)k;
         if (ri < 0) { *err = "resolution " + std::to_string(res) + " was not announced"; return 1; }
         if (done_[ri]) return 0;                                      // a resolution listed twice is stored once
@@ -170,6 +178,8 @@ public:
         for (size_t c = 0; c < nc; ++c) off[c + 1] = off[c] + len_[c] / res + 1;
         std::vector<std::vector<Rec>> per(nc * nc);
         std::vector<double> actual, chr_counts(nc, 0.0);
+        const size_t n_types = norms ? norms->size() : 0;
+        std::vector<std::vector<double>> n_actual(n_types), n_counts(n_types, std::vector<double>(nc, 0.0));
         const bool finest = res == res_.back();
         std::vector<Rec> all;                                        // whole-genome records, merged below
         size_t c1 = 0;
@@ -184,6 +194,14 @@ public:
                 const uint32_t d = y - x;
                 if (d >= actual.size()) actual.resize((size_t)d + 1, 0.0);
                 actual[d] += ct[i]; chr_counts[c1] += ct[i];
+                for (size_t t = 0; t < n_types; ++t) {
+                    const NormInput &q = (*norms)[t];
+                    const double nx = q.values[b1[i]], ny = q.values[b2[i]];
+                    if (!q.stored[c1] || !std::isfinite(nx) || !std::isfinite(ny) || !(nx > 0) || !(ny > 0)) continue;
+                    if (d >= n_actual[t].size()) n_actual[t].resize((size_t)d + 1, 0.0);
+                    const double v = ct[i] / (nx * ny);
+                    n_actual[t][d] += v; n_counts[t][c1] += v;
+                }
             }
             if (finest) {                                             // whole-genome view from the finest resolution's bin starts
                 uint32_t gx = (uint32_t)((cum_[c1] + (uint64_t)x * res) / 1000 / all_bin_), gy = (uint32_t)((cum_[c2] + (uint64_t)y * res) / 1000 / all_bin_);
@@ -192,6 +210,13 @@ public:
             }
         }
         expected_values(res, len_, actual, chr_counts, &exp_[ri]);
+        for (size_t t = 0; t < n_types; ++t) {
+            const NormInput &q = (*norms)[t];
+            norm_exp_.emplace_back(); norm_exp_.back().first = q.type;
+            expected_values(res, len_, n_actual[t], n_counts[t], &norm_exp_.back().second);
+            for (size_t c = 0; c < nc; ++c)
+                if (q.stored[c]) norm_vec_.push_back({q.type, (int)c + 1, res, std::vector<double>(q.values + off[c], q.values + off[c + 1])});
+        }
         // sort + deflate, one matrix per task
         std::vector<size_t> todo; for (size_t k = 0; k < nc * nc; ++k) if (!per[k].empty()) todo.push_back(k);
         std::sort(todo.begin(), todo.end(), [&](size_t a, size_t b) { return per[a].size() > per[b].size(); });
@@ -268,8 +293,25 @@ public:
         }
         Buf tail; tail.i32((int32_t)ft.v.size());                     // nBytesV5: what lies between this int and the normalised section
         tail.raw(ft.v.data(), ft.v.size());
-        tail.i32(0);                                                  // no normalised expected-value vectors
-        tail.i32(0);                                                  // no normalisation vectors (juicer's addNorm can append them later)
+        // normalised section: expected values per (type, resolution), the vectors' index, then the vectors at their positions
+        int nnexp = 0; for (auto &e : norm_exp_) nnexp += !e.second.values.empty();
+        tail.i32(nnexp);
+        for (auto &te : norm_exp_) {
+            const Expected &e = te.second;
+            if (e.values.empty()) continue;
+            tail.str(te.first); tail.str("BP"); tail.i32((int32_t)e.bin_size); tail.i32((int32_t)e.values.size());
+            for (double v : e.values) tail.f64(v);
+            tail.i32((int32_t)e.scale.size()); for (auto &sc : e.scale) { tail.i32(sc.first); tail.f64(sc.second); }
+        }
+        tail.i32((int32_t)norm_vec_.size());
+        int64_t vpos = pos + (int64_t)tail.v.size();
+        for (const NormVec &n : norm_vec_) vpos += (int64_t)(n.type.size() + 1 + 4 + 3 + 4 + 8 + 4);
+        for (const NormVec &n : norm_vec_) {
+            const int32_t nbytes = (int32_t)(4 + 8 * n.values.size());
+            tail.str(n.type); tail.i32(n.chr); tail.str("BP"); tail.i32((int32_t)n.bin_size); tail.i64(vpos); tail.i32(nbytes);
+            vpos += nbytes;
+        }
+        for (const NormVec &n : norm_vec_) { tail.i32((int32_t)n.values.size()); for (double v : n.values) tail.f64(v); }
         fwrite(tail.v.data(), 1, tail.v.size(), f);
         fseek(f, 8, SEEK_SET); fwrite(&pos, 8, 1, f);
         const bool bad = ferror(f); if (fclose(f) || bad) { *err = "write error on " + path; return 1; }
@@ -281,6 +323,9 @@ private:
     std::vector<uint64_t> cum_; uint32_t all_len_ = 0, all_bin_ = 1;
     std::vector<std::vector<Zoom>> zooms_;                           // [c1 * n + c2] -> the resolutions added so far
     std::vector<Expected> exp_; std::vector<bool> done_; Zoom all_zoom_; bool have_all_ = false;
+    struct NormVec { std::string type; int chr; uint32_t bin_size; std::vector<double> values; };
+    std::vector<std::pair<std::string, Expected>> norm_exp_;        // normalised expected values, in the order added
+    std::vector<NormVec> norm_vec_;                                   // chromosome index in the file: 1..n (0 is ALL: no vectors)
 };
 
 }  // namespace hic
