@@ -138,7 +138,8 @@ __global__ void __launch_bounds__(NM_T) k_nm_fill_lower(const RadixPlan *plan, c
     const u32 *v = plan->final_buf ? v1 : v0;
     const u64 m = *n_low;
     for (u64 j = (u64)blockIdx.x * NM_T + threadIdx.x; j < m; j += (u64)gridDim.x * NM_T) {
-        const u32 r = (u32)k[j], idx = v[j];
+        // no pass ran (every key equal: all entries mirror into one column): the values were never written, the order is the input's
+        const u32 r = (u32)k[j], idx = plan->n_exec ? v[j] : (u32)j;
         ents[row_ptr[r] + (j - low_start[r])] = make_uint2(b1[idx], cnt[idx]);
     }
 }

@@ -287,8 +287,16 @@ struct RadixWs {                   // device workspace for sorts of up to max_n 
     }
 };
 
-// Sorts `n` elements.  Input in buffer 0; the result ends in buffer plan->final_buf (device value).
+// Sorts `n` elements, stable, on the scheduled bytes.  Input in buffer 0; the result ends in buffer plan->final_buf (device value).
 // hist_done: the digit histograms are already in ws.plan->hist (zeroed, then filled by the kernel that produced the keys)
+// What a consumer reads back (tests/test_gpu_radix_edges.py checks each point through tests/radix_harness.cu):
+//   - a pass whose digit is the same for every key is skipped; final_buf = parity of plan->n_exec, the passes that ran
+//   - iota_vals: the first pass that runs writes the input index as the value, so values hold the stable permutation.  When
+//     NO pass runs (n_exec == 0: all keys equal on the schedule, or n == 0) the values are never written and buffer 0 keeps
+//     whatever the caller left there: the permutation is the identity and the consumer takes the position itself
+//     (`plan->n_exec ? v[i] : i`, pairs.cu k_mark_first, norm.cu k_nm_fill_lower)
+//   - bytes outside the schedule (the whole value word of Rec16 records included) travel with their key unsorted
+//   - refused before anything is enqueued: n >= 2^30 (30-bit look-back counts) or n > ws.max_n (MK_ERR_CAPACITY)
 template <class P>
 static int radix_sort(typename P::Bufs bufs, u64 n, const RadixSchedule &sch, RadixWs &ws, int iota_vals, int sms,
                       cudaStream_t s, u64 *launches, bool hist_done = false) {
