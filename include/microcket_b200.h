@@ -285,7 +285,7 @@ typedef struct mk_norm mk_norm;
 #define MK_NORM_VC_SQRT  2
 #define MK_NORM_KR       4
 typedef struct {
-    uint32_t kr_outer_max;      /* most outer (Newton) steps any chromosome took */
+    uint32_t kr_outer_max;      /* most outer (Newton) steps any chromosome (segment) took */
     uint32_t kr_matvecs;        /* lockstep KR steps = products over all unfinished chromosomes at once */
     uint32_t kr_failed;         /* chromosomes whose KR failed */
     double   kr_residual_max;   /* largest ||1 - x (A x)||_2 of the balanced chromosomes */
@@ -300,6 +300,17 @@ void mk_norm_destroy(mk_norm *);
  * (MK_ERR_ARG). */
 int  mk_norm_device(mk_norm *, const uint32_t *d_bin1, const uint32_t *d_bin2, const uint32_t *d_cnt, size_t nnz, int types,
                     double *d_vc, double *d_vc_sqrt, double *d_kr, uint8_t *chrom_status, mk_norm_stats *, void *stream);
+/* The genome-wide vectors over every bin at once (juicer's GW_VC / GW_KR and INTER_VC / INTER_KR), same COO and object:
+ * scope MK_NORM_SCOPE_GW balances the whole-genome matrix (every entry), MK_NORM_SCOPE_INTER its inter-chromosomal entries only
+ * (bins in different chromosomes).  One balancing problem over all n_bins rows with the definitions above (KR on the rows
+ * with a nonzero sum, one sum factor for the whole genome).  types: MK_NORM_VC and / or MK_NORM_KR (there is no GW / INTER
+ * VC_SQRT); d_vc / d_kr: n_bins doubles each on the device, global bin order.  *status (host, may be NULL): 0 ok, 1 the
+ * matrix has no entries (no vector of any type), 2 KR failed (no KR vector; VC is still written).  Refused like
+ * mk_norm_device, and also for MK_NORM_VC_SQRT, an unknown type bit or an unknown scope (MK_ERR_ARG). */
+#define MK_NORM_SCOPE_GW     1
+#define MK_NORM_SCOPE_INTER  2
+int  mk_norm_genome_device(mk_norm *, const uint32_t *d_bin1, const uint32_t *d_bin2, const uint32_t *d_cnt, size_t nnz, int scope,
+                           int types, double *d_vc, double *d_kr, uint8_t *status, mk_norm_stats *, void *stream);
 uint64_t mk_norm_launch_count(mk_norm *);
 /* Optional timing (tools/norm_bench.py): CUDA events on the stream, host clock for the KR loop.  ms[k] / count[k], arrays of 8:
  * 0 CSR build, 1 products inside KR, 2 KR vector kernels (pre + post), 3 KR loop wall time incl. the host round trips

@@ -59,6 +59,7 @@ class NormStats(C.Structure):
 
 
 NORM_TYPES = {"VC": 1, "VC_SQRT": 2, "KR": 4}
+NORM_SCOPES = {"GW": 1, "INTER": 2}
 
 
 class DedupCfg(C.Structure):
@@ -155,6 +156,7 @@ class Lib:
                            ("mk_pairs_launch_count", [vp]),
                            ("mk_norm_create", [i, P(C.c_uint32), i, C.c_uint32, sz, P(vp)]), ("mk_norm_destroy", [vp]),
                            ("mk_norm_device", [vp, vp, vp, vp, sz, i, vp, vp, vp, P(C.c_uint8), P(NormStats), vp]),
+                           ("mk_norm_genome_device", [vp, vp, vp, vp, sz, i, i, vp, vp, P(C.c_uint8), P(NormStats), vp]),
                            ("mk_norm_launch_count", [vp]), ("mk_norm_enable_timing", [vp, i]),
                            ("mk_norm_kernel_times", [vp, P(C.c_double), P(u64)])):
             if hasattr(L, name):
@@ -585,6 +587,20 @@ class Norm:
         self.lib.check(self.lib.L.mk_norm_device(self.h, d_bin1, d_bin2, d_cnt, nnz, mask, d_vc or None, d_vc_sqrt or None, d_kr or None,
                                                  status, C.byref(st), stream))
         return list(status), st
+
+    def run_genome(self, d_bin1, d_bin2, d_cnt, nnz, scope="GW", types=("VC", "KR"), d_vc=0, d_kr=0, stream=0):
+        """the genome-wide vectors: scope "GW" (every entry) or "INTER" (inter-chromosomal entries), types from ("VC", "KR");
+        n_bins doubles per requested type written to the device pointers -> (status, NormStats); status 0 ok, 1 empty matrix,
+        2 KR failed.  A scope or type outside these goes to the library as is, which refuses it."""
+        mask = 0
+        for t in types:
+            mask |= NORM_TYPES[t] if isinstance(t, str) else t
+        status = C.c_uint8()
+        st = NormStats()
+        sc = NORM_SCOPES[scope] if isinstance(scope, str) else scope
+        self.lib.check(self.lib.L.mk_norm_genome_device(self.h, d_bin1, d_bin2, d_cnt, nnz, sc, mask, d_vc or None, d_kr or None,
+                                                        C.byref(status), C.byref(st), stream))
+        return status.value, st
 
     def launches(self):
         return self.lib.L.mk_norm_launch_count(self.h)

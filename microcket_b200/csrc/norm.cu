@@ -1,27 +1,36 @@
 // norm.cu — balancing of contact matrices: the VC, VC_SQRT and KR normalisation vectors `juicer_tools pre` stores in a `.hic`
-// (microcket:525-529), per chromosome, from its intra-chromosomal matrix.  Restated from juicer's published behaviour
-// (Knight & Ruiz 2013 `bnewt` for KR, juicer's sum factor); PARITY UNPINNED like the rest of the container (DESIGN.md §5).
+// (microcket:525-529), per chromosome, from its intra-chromosomal matrix; and the GW_VC / GW_KR (whole-genome matrix) and
+// INTER_VC / INTER_KR (inter-chromosomal entries only) vectors, one balancing problem over every bin.  Restated from juicer's
+// published behaviour (Knight & Ruiz 2013 `bnewt` for KR, juicer's sum factor); PARITY UNPINNED like the rest of the
+// container (DESIGN.md §5).
 //
 // The COO of one resolution (sorted by (bin1, bin2), upper triangle: what mk_pairs_bin_device / mk_hist_coo_device return)
-// becomes ONE symmetric CSR of its intra-chromosomal entries, built once and reused by every product:
+// becomes ONE symmetric CSR of the entries in the call's scope, built once and reused by every product:
 //   row r = [mirrored half: (column bin1 < r), bin1 ascending][upper half: (column bin2 >= r), bin2 ascending]
-// The upper half is already CSR by bin1 in the COO; the mirrored half comes from one stable radix sort on bin2
-// (radix_sort.cuh, values = entry index).  Entries are (u32 column, u32 count), row pointers 64-bit.
+// The scope is INTRA (both bins in one chromosome), GENOME (every entry) or INTER (the two bins in different chromosomes).
+// Row r's entries in the COO are one run sorted by column; its INTRA entries are a prefix of the run (up to the end of r's
+// chromosome), its INTER entries the rest.  The upper half is therefore already CSR by bin1 in the COO; the mirrored half
+// comes from one stable radix sort on bin2 (radix_sort.cuh, values = entry index) of the scope's off-diagonal entries.
+// Entries are (u32 column, u32 count), row pointers 64-bit.
 //
-//   k_nm_classify     validation, intra test, where every row's intra entries start / end in the COO, sort keys
+// A segment is one balancing problem: a chromosome for INTRA, every bin for GENOME and INTER (segment 0).  The commands, the
+// results and the row skip of the element-wise kernels are indexed by segment through a bin -> segment table.
+//
+//   k_nm_classify     validation, scope test, where every row's entries in the scope start / end in the COO, sort keys
 //   k_nm_lower_runs   where every row's mirrored entries start / end in the sorted keys
 //   k_nm_row_ptr      row pointers (ticketed tiles, decoupled look-back)
 //   k_nm_fill_upper / k_nm_fill_lower   the CSR entries
 //   k_nm_spmv         y = A u: one warp per row, every lane sums a fixed stride of the row in order, then a fixed
 //                     butterfly: no floating-point atomics, so the vectors are bitwise reproducible from run to run
 //   k_nm_pre          per row, the vector that goes into the next product, from its chromosome's command
-//   k_nm_post         one CTA per chromosome: the vector updates and segmented reductions after a product
+//   k_nm_post         one CTA per chromosome: the vector updates and segmented reductions after a product (INTRA)
+//   k_nm_gpost        the same work for the one segment of GENOME / INTER, over fixed slices of NM_GS rows in 1 or 3 phases
 //   k_nm_finish       1 / x (KR) or sqrt (VC_SQRT) into the output vectors; k_nm_scale: the sum factors
 //
-// KR runs for all chromosomes in lockstep: every step is k_nm_pre -> k_nm_spmv -> k_nm_post, and the per-chromosome scalars
-// come back in ONE small copy; the host advances every chromosome's state machine (plain C++ below) and sends the next
-// step's commands in one copy.  Each unfinished chromosome needs exactly one product per step: A (x∘p) inside CG, A x after
-// an outer update.  Finished chromosomes' rows are skipped by the product.
+// KR runs for all segments in lockstep: every step is k_nm_pre -> k_nm_spmv -> k_nm_post (k_nm_gpost), and the per-segment
+// scalars come back in ONE small copy; the host advances every segment's state machine (plain C++ below) and sends the next
+// step's commands in one copy.  Each unfinished segment needs exactly one product per step: A (x∘p) inside CG, A x after
+// an outer update.  Finished segments' rows are skipped by the product.
 #include <algorithm>
 #include <chrono>
 #include <cmath>
@@ -33,6 +42,7 @@
 #define NM_RT 1024               // per-chromosome kernels: one CTA per chromosome (32 warps: the block reductions rely on it)
 #define NP_T 256                 // row pointer scan
 #define NP_ITEMS 16
+#define NM_GS 2048               // rows per slice of a GENOME / INTER segment: fixed, so the bits depend neither on the card nor on the grid
 
 // Knight-Ruiz parameters (bnewt defaults, as juicer uses them)
 #define KR_TOL 1e-6
@@ -45,16 +55,25 @@
 
 enum { OP_IDLE = 0, OP_ONES, OP_KR_INIT, OP_KR_OUTER, OP_CG_FIRST, OP_CG_NEXT, OP_SUMF };
 enum { ST_CG_CONT = 0, ST_CG_BREAK = 1, ST_FAIL = 2 };
+enum { NM_INTRA = 0, NM_GENOME = MK_NORM_SCOPE_GW, NM_INTER = MK_NORM_SCOPE_INTER };
 
 struct NormCmd { int op, pad; double beta, rho; };             // host -> device, one per chromosome and step
 struct NormRes { double a, b, c; int flag, pad; };             // device -> host
+struct NormPart { double a, b, c, d; };                         // one slice's partials of one k_nm_gpost phase
+static_assert(sizeof(NormRes) == sizeof(NormPart), "k_nm_gpost's result sits behind its final partials, copied in one piece");
 
 struct NormVecs { double *x, *v, *rk, *y, *z, *p, *w, *u, *au, *rs; u8 *kept; };   // rs: row sums (au is every product's output)
 
 // ---------------------------------------------------------------- CSR build
 __device__ __forceinline__ u32 nm_chr_end(const u32 *chr_of_bin, const u32 *chr_off, u32 bin) { return chr_off[chr_of_bin[bin] + 1]; }
 
+template <int SC>
+__device__ __forceinline__ bool nm_in_scope(const u32 *chr_of_bin, const u32 *chr_off, u32 a, u32 b) {
+    return SC == NM_GENOME || ((b < nm_chr_end(chr_of_bin, chr_off, a)) == (SC == NM_INTRA));
+}
+
 // err bit 0: bin1 > bin2, bit 1: a bin past the end, bit 2: not sorted by (bin1, bin2)
+template <int SC>
 __global__ void __launch_bounds__(NM_T) k_nm_classify(const u32 *b1, const u32 *b2, u64 nnz, u32 nb, const u32 *chr_of_bin, const u32 *chr_off,
                                                      u32 *row_start, u32 *up_end, u64 *keys, u32 *err, unsigned long long *n_low) {
     u32 e = 0, low = 0;
@@ -65,11 +84,12 @@ __global__ void __launch_bounds__(NM_T) k_nm_classify(const u32 *b1, const u32 *
         if (b >= nb) { e |= 2u; bad = true; }
         if (i && (b1[i - 1] > a || (b1[i - 1] == a && b2[i - 1] >= b))) e |= 4u;
         if (bad) { keys[i] = nb; continue; }
-        const bool intra = b < nm_chr_end(chr_of_bin, chr_off, a);
-        // a row's intra entries are a prefix of its run in the COO (columns ascend, the chromosome ends at chr_end)
-        if (intra && (i == 0 || b1[i - 1] != a)) row_start[a] = (u32)i;
-        if (intra && (i + 1 == nnz || b1[i + 1] != a || b2[i + 1] >= nm_chr_end(chr_of_bin, chr_off, a))) up_end[a] = (u32)(i + 1);
-        const bool mirror = intra && a != b;
+        const bool in = nm_in_scope<SC>(chr_of_bin, chr_off, a, b);
+        // a row's entries in the scope are one piece of its run in the COO (columns ascend, the chromosome ends at chr_end):
+        // INTRA a prefix, INTER a suffix, GENOME the whole run
+        if (in && (i == 0 || b1[i - 1] != a || (SC == NM_INTER && b2[i - 1] < nm_chr_end(chr_of_bin, chr_off, a)))) row_start[a] = (u32)i;
+        if (in && (i + 1 == nnz || b1[i + 1] != a || (SC == NM_INTRA && b2[i + 1] >= nm_chr_end(chr_of_bin, chr_off, a)))) up_end[a] = (u32)(i + 1);
+        const bool mirror = in && a != b;
         keys[i] = mirror ? (u64)b : (u64)nb;                    // everything else sorts behind the mirrored entries
         low += mirror;
     }
@@ -122,11 +142,12 @@ __global__ void __launch_bounds__(NP_T) k_nm_row_ptr(u32 nb, const u32 *row_star
     }
 }
 
+template <int SC>
 __global__ void __launch_bounds__(NM_T) k_nm_fill_upper(const u32 *b1, const u32 *b2, const u32 *cnt, u64 nnz, const u32 *chr_of_bin, const u32 *chr_off,
                                                        const u64 *row_ptr, const u32 *row_start, const u32 *low_start, const u32 *low_end, uint2 *ents) {
     for (u64 i = (u64)blockIdx.x * NM_T + threadIdx.x; i < nnz; i += (u64)gridDim.x * NM_T) {
         const u32 a = b1[i], b = b2[i];
-        if (b >= nm_chr_end(chr_of_bin, chr_off, a)) continue;
+        if (!nm_in_scope<SC>(chr_of_bin, chr_off, a, b)) continue;
         ents[row_ptr[a] + (low_end[a] - low_start[a]) + (i - row_start[a])] = make_uint2(b, cnt[i]);
     }
 }
@@ -145,12 +166,12 @@ __global__ void __launch_bounds__(NM_T) k_nm_fill_lower(const RadixPlan *plan, c
 }
 
 // ---------------------------------------------------------------- product
-__global__ void __launch_bounds__(NM_T) k_nm_spmv(const u64 *row_ptr, const uint2 *ents, u32 nb, const u32 *chr_of_bin, const NormCmd *cmd,
+__global__ void __launch_bounds__(NM_T) k_nm_spmv(const u64 *row_ptr, const uint2 *ents, u32 nb, const u32 *seg_of_bin, const NormCmd *cmd,
                                                  const double *u, double *y) {
     const int lane = threadIdx.x & 31;
     const u64 warps = (u64)gridDim.x * (NM_T / 32);
     for (u64 r = (u64)blockIdx.x * (NM_T / 32) + (threadIdx.x >> 5); r < nb; r += warps) {
-        if (cmd[chr_of_bin[r]].op == OP_IDLE) continue;
+        if (cmd[seg_of_bin[r]].op == OP_IDLE) continue;
         const u64 beg = row_ptr[r], end = row_ptr[r + 1];
         double acc = 0.0;
         u64 k = beg + lane;
@@ -169,9 +190,9 @@ __global__ void __launch_bounds__(NM_T) k_nm_spmv(const u64 *row_ptr, const uint
 }
 
 // ---------------------------------------------------------------- per-row commands before a product
-__global__ void __launch_bounds__(NM_T) k_nm_pre(u32 nb, const u32 *chr_of_bin, const NormCmd *cmd, NormVecs V, const double *nvec) {
+__global__ void __launch_bounds__(NM_T) k_nm_pre(u32 nb, const u32 *seg_of_bin, const NormCmd *cmd, NormVecs V, const double *nvec) {
     for (u64 r = (u64)blockIdx.x * NM_T + threadIdx.x; r < nb; r += (u64)gridDim.x * NM_T) {
-        const NormCmd c = cmd[chr_of_bin[r]];
+        const NormCmd c = cmd[seg_of_bin[r]];
         const bool kp = V.kept[r];
         switch (c.op) {
         case OP_ONES: V.u[r] = 1.0; break;
@@ -190,6 +211,8 @@ __global__ void __launch_bounds__(NM_T) k_nm_pre(u32 nb, const u32 *chr_of_bin, 
 
 // ---------------------------------------------------------------- per-chromosome updates and reductions after a product
 // Every thread walks a fixed stride of the chromosome's rows in order, then a fixed tree: the same bits on every run.
+// NW: warps in the CTA (k_nm_post 32, k_nm_gpost NM_T / 32).
+template <int NW = NM_RT / 32>
 __device__ __forceinline__ double nm_bsum(double v, double *sh) {
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
 #pragma unroll
@@ -197,7 +220,7 @@ __device__ __forceinline__ double nm_bsum(double v, double *sh) {
     if (lane == 0) sh[wid] = v;
     __syncthreads();
     if (wid == 0) {
-        double t = sh[lane];
+        double t = lane < NW ? sh[lane] : 0.0;
 #pragma unroll
         for (int d = 16; d; d >>= 1) t += __shfl_xor_sync(0xffffffffu, t, d);
         if (lane == 0) sh[32] = t;
@@ -207,7 +230,7 @@ __device__ __forceinline__ double nm_bsum(double v, double *sh) {
     __syncthreads();
     return r;
 }
-template <bool MAX>
+template <bool MAX, int NW = NM_RT / 32>
 __device__ __forceinline__ double nm_bext(double v, double *sh) {
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
 #pragma unroll
@@ -215,7 +238,7 @@ __device__ __forceinline__ double nm_bext(double v, double *sh) {
     if (lane == 0) sh[wid] = v;
     __syncthreads();
     if (wid == 0) {
-        double t = sh[lane];
+        double t = lane < NW ? sh[lane] : (MAX ? -INFINITY : INFINITY);
 #pragma unroll
         for (int d = 16; d; d >>= 1) { const double o = __shfl_xor_sync(0xffffffffu, t, d); t = MAX ? fmax(t, o) : fmin(t, o); }
         if (lane == 0) sh[32] = t;
@@ -290,30 +313,147 @@ __global__ void __launch_bounds__(NM_RT) k_nm_post(const u32 *chr_off, const Nor
     if (threadIdx.x == 0) res[c] = out;
 }
 
-// kind 0: VC (row sums), 1: VC_SQRT, 2: KR (1 / x on kept rows of balanced chromosomes, NaN elsewhere)
-__global__ void __launch_bounds__(NM_T) k_nm_finish(int kind, u32 nb, const u32 *chr_of_bin, const u8 *kr_ok, NormVecs V, double *out) {
+// ---------------------------------------------------------------- the same for the one segment of GENOME / INTER
+// One CTA per segment would stream every vector of 617 669 rows (hg38 at 5 kb) through one SM.  The rows are cut into slices
+// of NM_GS; a CTA walks slices blockIdx.x, + gridDim.x, ... and writes one NormPart per slice and phase.  A CG step's dependent
+// reductions are three launches: phase 0 the product's update (w) with p·w and rk·Z, phase 1 alpha and the box test's extrema,
+// phase 2 the update and the new rk·Z.  In phases 1 and 2 every CTA recomputes the totals of the earlier phases from their
+// partials (nm_gtot: in slice order, then a fixed tree), so every CTA takes the same decision and the bits depend on the slice
+// width only, not on the grid.  The other ops need phase 0 only.  The final partials (pf) and phase 2's scalars (res) go to the
+// host in one copy; nm_gres sums them there in slice order.
+__device__ __forceinline__ double nm_gsum(const NormPart *p, u32 ns, int f, double *sh) {
+    double s = 0.0;
+    for (u32 i = threadIdx.x; i < ns; i += NM_T) s += (&p[i].a)[f];
+    return nm_bsum<NM_T / 32>(s, sh);
+}
+template <bool MAX>
+__device__ __forceinline__ double nm_gext(const NormPart *p, u32 ns, int f, double *sh) {
+    double s = MAX ? -INFINITY : INFINITY;
+    for (u32 i = threadIdx.x; i < ns; i += NM_T) s = MAX ? fmax(s, (&p[i].a)[f]) : fmin(s, (&p[i].a)[f]);
+    return nm_bext<MAX, NM_T / 32>(s, sh);
+}
+
+// part: [phase 0: ns][phase 1: ns][final: ns][NormRes]
+__global__ void __launch_bounds__(NM_T) k_nm_gpost(int phase, u32 nb, const NormCmd *cmd, NormVecs V, NormPart *part) {
+    __shared__ double sh[33];
+    const NormCmd cm = cmd[0];
+    if (cm.op == OP_IDLE) return;
+    const u32 ns = (nb + NM_GS - 1) / NM_GS;
+    NormPart *p0 = part, *p1 = part + ns, *pf = part + 2 * (size_t)ns;
+    NormRes *res = (NormRes *)(pf + ns);
+    const bool cg = cm.op == OP_CG_FIRST || cm.op == OP_CG_NEXT;
+    double rho = 0.0, alpha = 0.0, gamma = 0.0;
+    bool brk = false;
+    if (phase > 0) {
+        const double pw = nm_gsum(p0, ns, 0, sh), rz = nm_gsum(p0, ns, 1, sh);
+        rho = cm.op == OP_CG_FIRST ? rz : cm.rho; alpha = rho / pw;
+        if (!isfinite(alpha)) {
+            if (phase == 2 && blockIdx.x == 0 && threadIdx.x == 0) *res = NormRes{rho, 0.0, alpha, ST_FAIL, 0};
+            return;
+        }
+    }
+    if (phase == 2) {
+        const double ymin = nm_gext<false>(p1, ns, 0, sh), ymax = nm_gext<true>(p1, ns, 1, sh);
+        const double glo = nm_gext<false>(p1, ns, 2, sh), ghi = nm_gext<false>(p1, ns, 3, sh);
+        brk = ymin <= KR_DELTA || ymax >= KR_DELTA_HI;            // the step leaves the box: stop at its edge, end the inner loop
+        gamma = ymin <= KR_DELTA ? glo : ghi;
+        if (blockIdx.x == 0 && threadIdx.x == 0) *res = NormRes{rho, 0.0, alpha, brk ? ST_CG_BREAK : ST_CG_CONT, 0};
+    }
+    for (u32 sl = blockIdx.x; sl < ns; sl += gridDim.x) {
+        const u32 r0 = sl * NM_GS, r1 = min(nb, r0 + NM_GS);
+        NormPart o = {0.0, 0.0, 0.0, 0.0};
+        if (phase == 0 && cm.op == OP_ONES) {                          // row sums: raw total and rows kept by KR
+            double s = 0.0, k = 0.0;
+            for (u32 r = r0 + threadIdx.x; r < r1; r += NM_T) { const double a = V.au[r]; s += a; k += a > 0.0; V.rs[r] = a; V.kept[r] = a > 0.0; }
+            o.a = nm_bsum<NM_T / 32>(s, sh); o.b = nm_bsum<NM_T / 32>(k, sh);
+        } else if (phase == 0 && cm.op == OP_SUMF) {
+            double s = 0.0;
+            for (u32 r = r0 + threadIdx.x; r < r1; r += NM_T) s += V.u[r] * V.au[r];
+            o.a = nm_bsum<NM_T / 32>(s, sh);
+        } else if (phase == 0 && !cg) {                                 // OP_KR_INIT / OP_KR_OUTER: v = x (A x), rk = 1 - v
+            double s = 0.0, xmin = INFINITY; int bad = 0;
+            for (u32 r = r0 + threadIdx.x; r < r1; r += NM_T) {
+                if (!V.kept[r]) continue;
+                const double x = V.x[r], v = x * V.au[r], rk = 1.0 - v;
+                V.v[r] = v; V.rk[r] = rk;
+                s += rk * rk; xmin = fmin(xmin, x); bad |= !isfinite(x) || !isfinite(v);
+            }
+            o.a = nm_bsum<NM_T / 32>(s, sh); o.b = nm_bext<false, NM_T / 32>(xmin, sh); o.c = nm_bsum<NM_T / 32>((double)bad, sh);
+        } else if (phase == 0) {                                        // a CG step on the product A (x p): w, p·w, rk·Z
+            double pw = 0.0, rz = 0.0;
+            for (u32 r = r0 + threadIdx.x; r < r1; r += NM_T) {
+                if (!V.kept[r]) continue;
+                const double p = V.p[r], w = V.x[r] * V.au[r] + V.v[r] * p;
+                V.w[r] = w; pw += p * w; rz += V.rk[r] * V.z[r];
+            }
+            o.a = nm_bsum<NM_T / 32>(pw, sh); o.b = nm_bsum<NM_T / 32>(rz, sh);
+        } else if (phase == 1) {                                        // the box test's extrema
+            double ymin = INFINITY, ymax = -INFINITY, glo = INFINITY, ghi = INFINITY;
+            for (u32 r = r0 + threadIdx.x; r < r1; r += NM_T) {
+                if (!V.kept[r]) continue;
+                const double y = V.y[r], ap = alpha * V.p[r], yn = y + ap;
+                ymin = fmin(ymin, yn); ymax = fmax(ymax, yn);
+                if (ap < 0.0) glo = fmin(glo, (KR_DELTA - y) / ap);
+                if (yn > KR_DELTA_HI) ghi = fmin(ghi, (KR_DELTA_HI - y) / ap);
+            }
+            o.a = nm_bext<false, NM_T / 32>(ymin, sh); o.b = nm_bext<true, NM_T / 32>(ymax, sh);
+            o.c = nm_bext<false, NM_T / 32>(glo, sh); o.d = nm_bext<false, NM_T / 32>(ghi, sh);
+        } else if (brk) {
+            for (u32 r = r0 + threadIdx.x; r < r1; r += NM_T) if (V.kept[r]) V.y[r] = V.y[r] + gamma * (alpha * V.p[r]);
+        } else {                                                        // the update and the new rk·Z
+            double s = 0.0;
+            for (u32 r = r0 + threadIdx.x; r < r1; r += NM_T) {
+                if (!V.kept[r]) continue;
+                const double rk = V.rk[r] - alpha * V.w[r], z = rk / V.v[r];
+                V.y[r] = V.y[r] + alpha * V.p[r]; V.rk[r] = rk; V.z[r] = z; s += rk * z;
+            }
+            o.a = nm_bsum<NM_T / 32>(s, sh);
+        }
+        if (threadIdx.x == 0) (phase == 0 && cg ? p0 : phase == 1 ? p1 : pf)[sl] = o;
+    }
+}
+
+// the host side of k_nm_gpost: segment 0's NormRes from the final partials, summed in slice order
+static void nm_gres(int op, const NormPart *pf, u32 ns, NormRes *out) {
+    if (op == OP_CG_FIRST || op == OP_CG_NEXT) {
+        *out = *(const NormRes *)(pf + ns);
+        if (out->flag == ST_CG_CONT) { double s = 0.0; for (u32 i = 0; i < ns; ++i) s += pf[i].a; out->b = s; }
+        return;
+    }
+    NormRes r = {0.0, op == OP_ONES ? 0.0 : INFINITY, 0.0, 0, 0};
+    for (u32 i = 0; i < ns; ++i) {
+        r.a += pf[i].a;
+        if (op == OP_ONES) r.b += pf[i].b;
+        else { r.b = std::min(r.b, pf[i].b); r.flag |= pf[i].c > 0.0; }
+    }
+    *out = r;
+}
+
+// kind 0: VC (row sums), 1: VC_SQRT, 2: KR (1 / x on kept rows of balanced segments, NaN elsewhere)
+__global__ void __launch_bounds__(NM_T) k_nm_finish(int kind, u32 nb, const u32 *seg_of_bin, const u8 *kr_ok, NormVecs V, double *out) {
     for (u64 r = (u64)blockIdx.x * NM_T + threadIdx.x; r < nb; r += (u64)gridDim.x * NM_T) {
         const double s = V.rs[r];
         if (kind == 0) out[r] = s;
         else if (kind == 1) out[r] = sqrt(s);
-        else out[r] = (kr_ok[chr_of_bin[r]] && V.kept[r]) ? 1.0 / V.x[r] : (double)NAN;
+        else out[r] = (kr_ok[seg_of_bin[r]] && V.kept[r]) ? 1.0 / V.x[r] : (double)NAN;
     }
 }
 
-__global__ void __launch_bounds__(NM_T) k_nm_scale(u32 nb, const u32 *chr_of_bin, const double *f, double *n) {
-    for (u64 r = (u64)blockIdx.x * NM_T + threadIdx.x; r < nb; r += (u64)gridDim.x * NM_T) n[r] *= f[chr_of_bin[r]];
+__global__ void __launch_bounds__(NM_T) k_nm_scale(u32 nb, const u32 *seg_of_bin, const double *f, double *n) {
+    for (u64 r = (u64)blockIdx.x * NM_T + threadIdx.x; r < nb; r += (u64)gridDim.x * NM_T) n[r] *= f[seg_of_bin[r]];
 }
 
 // ---------------------------------------------------------------- host side
 struct mk_norm {
-    int device = 0, sms = 148, n_chrom = 0;
-    u32 res = 0, nb = 0;
+    int device = 0, sms = 148, n_chrom = 0, scope = NM_INTRA;   // scope: the current call's
+    u32 res = 0, nb = 0, ns = 0;                                 // ns: slices of a GENOME / INTER segment
     size_t max_nnz = 0;
     std::vector<u32> chr_off;                               // n_chrom + 1 bin offsets
     DevBuf d_chr_of_bin, d_chr_off, d_row_ptr, d_runs /* row_start | up_end | low_start | low_end */, d_ents;
     DevBuf d_keys[2], d_vals[2], d_desc, d_small /* err, n_low, ticket */, d_vecs, d_kept, d_cmd, d_res, d_f, d_krok;
+    DevBuf d_seg0 /* nb zeros: every bin in segment 0 */, d_gpart /* k_nm_gpost's partials and result */;
     RadixWs rws;
-    PinBuf h_cmd, h_res, h_f;
+    PinBuf h_cmd, h_res, h_f, h_gpart;
     u64 launches = 0;
     bool timing = false;
     double ms[8] = {0}; u64 count[8] = {0};
@@ -327,6 +467,8 @@ struct mk_norm {
         return V;
     }
     int grid(u64 n, int per) const { return (int)std::max<u64>(1, std::min<u64>((n + per - 1) / per, (u64)sms * 16)); }
+    int n_seg() const { return scope == NM_INTRA ? n_chrom : 1; }
+    const u32 *seg_of_bin() const { return scope == NM_INTRA ? d_chr_of_bin.as<u32>() : d_seg0.as<u32>(); }
 };
 
 extern "C" int mk_norm_create(int device, const uint32_t *chrom_len, int n_chrom, uint32_t res, size_t max_nnz, mk_norm **out) {
@@ -340,6 +482,7 @@ extern "C" int mk_norm_create(int device, const uint32_t *chrom_len, int n_chrom
     for (int c = 0; c < n_chrom; ++c) { nb += chrom_len[c] / res + 1; if (nb >= (1ull << 31)) { mk_set_error("mk_norm_create: more than 2^31 bins"); return MK_ERR_CAPACITY; } off[c + 1] = (u32)nb; }
     mk_norm *h = new mk_norm();
     h->device = device; h->sms = mk_sm_count(device); h->n_chrom = n_chrom; h->res = res; h->nb = (u32)nb; h->max_nnz = max_nnz; h->chr_off = off;
+    h->ns = (u32)((nb + NM_GS - 1) / NM_GS);
     std::vector<u32> cob(nb);
     for (int c = 0; c < n_chrom; ++c) for (u32 r = off[c]; r < off[c + 1]; ++r) cob[r] = (u32)c;
     const size_t m = std::max<size_t>(max_nnz, 1);
@@ -349,11 +492,13 @@ extern "C" int mk_norm_create(int device, const uint32_t *chrom_len, int n_chrom
     A(h->d_ents, 2 * m * 8); A(h->d_keys[0], m * 8); A(h->d_keys[1], m * 8); A(h->d_vals[0], m * 4); A(h->d_vals[1], m * 4);
     A(h->d_desc, ((nb + NP_T * NP_ITEMS - 1) / (NP_T * NP_ITEMS) + 2) * 8); A(h->d_small, 64);
     A(h->d_vecs, 10 * nb * 8); A(h->d_kept, nb); A(h->d_cmd, n_chrom * sizeof(NormCmd)); A(h->d_res, n_chrom * sizeof(NormRes));
-    A(h->d_f, n_chrom * 8); A(h->d_krok, n_chrom);
+    A(h->d_f, n_chrom * 8); A(h->d_krok, n_chrom); A(h->d_seg0, nb * 4); A(h->d_gpart, (3 * (size_t)h->ns + 1) * sizeof(NormPart));
     if (rc == MK_OK) rc = h->rws.alloc(m);
     if (rc == MK_OK) rc = h->h_cmd.alloc(n_chrom * sizeof(NormCmd));
     if (rc == MK_OK) rc = h->h_res.alloc(n_chrom * sizeof(NormRes));
     if (rc == MK_OK) rc = h->h_f.alloc(n_chrom * 8);
+    if (rc == MK_OK) rc = h->h_gpart.alloc(((size_t)h->ns + 1) * sizeof(NormPart));
+    if (rc == MK_OK && cudaMemset(h->d_seg0.p, 0, nb * 4) != cudaSuccess) { mk_set_error("mk_norm_create: cudaMemset"); rc = MK_ERR_CUDA; }
     if (rc == MK_OK && (cudaMemcpy(h->d_chr_of_bin.p, cob.data(), nb * 4, cudaMemcpyHostToDevice) != cudaSuccess ||
                         cudaMemcpy(h->d_chr_off.p, off.data(), (n_chrom + 1) * 4, cudaMemcpyHostToDevice) != cudaSuccess)) { mk_set_error("mk_norm_create: table upload failed"); rc = MK_ERR_CUDA; }
     for (int k = 0; k < 4 && rc == MK_OK; ++k) if (cudaEventCreate(&h->ev[k]) != cudaSuccess) { mk_set_error("mk_norm_create: cudaEventCreate"); rc = MK_ERR_CUDA; }
@@ -378,8 +523,8 @@ extern "C" int mk_norm_kernel_times(mk_norm *h, double *ms, uint64_t *count) {
 
 static double nm_elapsed(cudaEvent_t a, cudaEvent_t b) { float t = 0; cudaEventElapsedTime(&t, a, b); return t; }
 
-// symmetric CSR of the intra-chromosomal entries
-static int nm_build(mk_norm *h, const u32 *b1, const u32 *b2, const u32 *cnt, u64 nnz, cudaStream_t s) {
+// symmetric CSR of the entries in h->scope
+static int nm_build(mk_norm *h, const char *who, const u32 *b1, const u32 *b2, const u32 *cnt, u64 nnz, cudaStream_t s) {
     const u32 nb = h->nb;
     u32 *runs = h->d_runs.as<u32>();
     u32 *row_start = runs, *up_end = runs + nb, *low_start = runs + 2 * (size_t)nb, *low_end = runs + 3 * (size_t)nb;
@@ -392,15 +537,16 @@ static int nm_build(mk_norm *h, const u32 *b1, const u32 *b2, const u32 *cnt, u6
     MK_CUDA(cudaMemsetAsync(h->d_small.p, 0, 64, s));
     MK_CUDA(cudaMemsetAsync(h->d_kept.p, 0, nb, s));
     if (nnz) {
-        k_nm_classify<<<h->grid(nnz, NM_T), NM_T, 0, s>>>(b1, b2, nnz, nb, cob, coff, row_start, up_end, h->d_keys[0].as<u64>(), err, n_low);
+        auto classify = h->scope == NM_GENOME ? k_nm_classify<NM_GENOME> : h->scope == NM_INTER ? k_nm_classify<NM_INTER> : k_nm_classify<NM_INTRA>;
+        classify<<<h->grid(nnz, NM_T), NM_T, 0, s>>>(b1, b2, nnz, nb, cob, coff, row_start, up_end, h->d_keys[0].as<u64>(), err, n_low);
         h->launches += 1;
         u32 e = 0;
         MK_CUDA(cudaMemcpyAsync(&e, err, 4, cudaMemcpyDeviceToHost, s));
         MK_CUDA(cudaStreamSynchronize(s));
         MK_CUDA(cudaGetLastError());
-        if (e & 1u) { mk_set_error("mk_norm_device: an entry with bin1 > bin2 (the COO must be an upper triangle)"); return MK_ERR_ARG; }
-        if (e & 2u) { mk_set_error("mk_norm_device: a bin at or beyond the %u bins of resolution %u", nb, h->res); return MK_ERR_ARG; }
-        if (e & 4u) { mk_set_error("mk_norm_device: the COO is not sorted by (bin1, bin2)"); return MK_ERR_ARG; }
+        if (e & 1u) { mk_set_error("%s: an entry with bin1 > bin2 (the COO must be an upper triangle)", who); return MK_ERR_ARG; }
+        if (e & 2u) { mk_set_error("%s: a bin at or beyond the %u bins of resolution %u", who, nb, h->res); return MK_ERR_ARG; }
+        if (e & 4u) { mk_set_error("%s: the COO is not sorted by (bin1, bin2)", who); return MK_ERR_ARG; }
         RadixSchedule sch; sch.n_pass = 0;
         for (u64 v = nb; v; v >>= 8) { sch.byte_of[sch.n_pass] = sch.n_pass; ++sch.n_pass; }   // keys <= nb
         KV64::Bufs kb; kb.k[0] = h->d_keys[0].as<u64>(); kb.k[1] = h->d_keys[1].as<u64>(); kb.v[0] = h->d_vals[0].as<u32>(); kb.v[1] = h->d_vals[1].as<u32>();
@@ -414,7 +560,8 @@ static int nm_build(mk_norm *h, const u32 *b1, const u32 *b2, const u32 *cnt, u6
     k_nm_row_ptr<<<(int)std::min<u64>((u64)h->sms * 8, n_tiles), NP_T, 0, s>>>(nb, row_start, up_end, low_start, low_end, h->d_row_ptr.as<u64>(), h->d_desc.as<u64>(), ticket);
     h->launches += 1;
     if (nnz) {
-        k_nm_fill_upper<<<h->grid(nnz, NM_T), NM_T, 0, s>>>(b1, b2, cnt, nnz, cob, coff, h->d_row_ptr.as<u64>(), row_start, low_start, low_end, h->d_ents.as<uint2>());
+        auto fill_upper = h->scope == NM_GENOME ? k_nm_fill_upper<NM_GENOME> : h->scope == NM_INTER ? k_nm_fill_upper<NM_INTER> : k_nm_fill_upper<NM_INTRA>;
+        fill_upper<<<h->grid(nnz, NM_T), NM_T, 0, s>>>(b1, b2, cnt, nnz, cob, coff, h->d_row_ptr.as<u64>(), row_start, low_start, low_end, h->d_ents.as<uint2>());
         k_nm_fill_lower<<<h->grid(nnz, NM_T), NM_T, 0, s>>>(h->rws.plan.as<RadixPlan>(), h->d_keys[0].as<u64>(), h->d_keys[1].as<u64>(), h->d_vals[0].as<u32>(),
                                                              h->d_vals[1].as<u32>(), n_low, b1, cnt, h->d_row_ptr.as<u64>(), low_start, h->d_ents.as<uint2>());
         h->launches += 2;
@@ -428,24 +575,33 @@ static int nm_build(mk_norm *h, const u32 *b1, const u32 *b2, const u32 *cnt, u6
     return MK_OK;
 }
 
-// One step for every chromosome: commands up, pre -> product -> post, results down.  nvec: the vector of OP_SUMF.
+// One step for every segment: commands up, pre -> product -> post, results down.  nvec: the vector of OP_SUMF.
 // Timing slots: in_kr ? (1 product, 2 pre + post) : (4 product, 5 pre + post).
 static int nm_step(mk_norm *h, const double *nvec, bool in_kr, cudaStream_t s) {
     const NormVecs V = h->vecs();
-    const u32 *cob = h->d_chr_of_bin.as<u32>();
+    const u32 *seg = h->seg_of_bin();
     const NormCmd *cmd = h->d_cmd.as<NormCmd>();
-    MK_CUDA(cudaMemcpyAsync(h->d_cmd.p, h->h_cmd.p, h->n_chrom * sizeof(NormCmd), cudaMemcpyHostToDevice, s));
+    const int op0 = h->h_cmd.as<NormCmd>()[0].op;
+    MK_CUDA(cudaMemcpyAsync(h->d_cmd.p, h->h_cmd.p, h->n_seg() * sizeof(NormCmd), cudaMemcpyHostToDevice, s));
     if (h->timing) MK_CUDA(cudaEventRecord(h->ev[0], s));
-    k_nm_pre<<<h->grid(h->nb, NM_T), NM_T, 0, s>>>(h->nb, cob, cmd, V, nvec);
+    k_nm_pre<<<h->grid(h->nb, NM_T), NM_T, 0, s>>>(h->nb, seg, cmd, V, nvec);
     if (h->timing) MK_CUDA(cudaEventRecord(h->ev[1], s));
-    k_nm_spmv<<<h->grid(h->nb, NM_T / 32), NM_T, 0, s>>>(h->d_row_ptr.as<u64>(), h->d_ents.as<uint2>(), h->nb, cob, cmd, V.u, V.au);
+    k_nm_spmv<<<h->grid(h->nb, NM_T / 32), NM_T, 0, s>>>(h->d_row_ptr.as<u64>(), h->d_ents.as<uint2>(), h->nb, seg, cmd, V.u, V.au);
     if (h->timing) MK_CUDA(cudaEventRecord(h->ev[2], s));
-    k_nm_post<<<h->n_chrom, NM_RT, 0, s>>>(h->d_chr_off.as<u32>(), cmd, V, h->d_res.as<NormRes>());
+    if (h->scope == NM_INTRA) {
+        k_nm_post<<<h->n_chrom, NM_RT, 0, s>>>(h->d_chr_off.as<u32>(), cmd, V, h->d_res.as<NormRes>());
+        h->launches += 3;
+    } else {
+        const int phases = op0 == OP_CG_FIRST || op0 == OP_CG_NEXT ? 3 : 1;
+        for (int ph = 0; ph < phases; ++ph) k_nm_gpost<<<h->grid(h->ns, 1), NM_T, 0, s>>>(ph, h->nb, cmd, V, h->d_gpart.as<NormPart>());
+        h->launches += 2 + phases;
+    }
     if (h->timing) MK_CUDA(cudaEventRecord(h->ev[3], s));
-    h->launches += 3;
-    MK_CUDA(cudaMemcpyAsync(h->h_res.p, h->d_res.p, h->n_chrom * sizeof(NormRes), cudaMemcpyDeviceToHost, s));
+    if (h->scope == NM_INTRA) MK_CUDA(cudaMemcpyAsync(h->h_res.p, h->d_res.p, h->n_chrom * sizeof(NormRes), cudaMemcpyDeviceToHost, s));
+    else MK_CUDA(cudaMemcpyAsync(h->h_gpart.p, h->d_gpart.as<NormPart>() + 2 * (size_t)h->ns, ((size_t)h->ns + 1) * sizeof(NormPart), cudaMemcpyDeviceToHost, s));
     MK_CUDA(cudaStreamSynchronize(s));
     MK_CUDA(cudaGetLastError());
+    if (h->scope != NM_INTRA && op0 != OP_IDLE) nm_gres(op0, h->h_gpart.as<NormPart>(), h->ns, h->h_res.as<NormRes>());
     if (h->timing) {
         const int a = in_kr ? 1 : 4;
         h->ms[a] += nm_elapsed(h->ev[1], h->ev[2]); h->count[a] += 1;
@@ -460,9 +616,9 @@ struct KrState {                 // bnewt's scalars of one chromosome
     bool done = false, failed = false;
 };
 
-// Knight-Ruiz for every chromosome with kept rows, in lockstep; kr_ok[c] = 1 for the balanced ones
+// Knight-Ruiz for every segment with kept rows, in lockstep; kr_ok[c] = 1 for the balanced ones
 static int nm_kr(mk_norm *h, const std::vector<double> &kept_rows, std::vector<u8> &kr_ok, mk_norm_stats *st, cudaStream_t s) {
-    const int nc = h->n_chrom;
+    const int nc = h->n_seg();
     const double rt = KR_TOL * KR_TOL, stop_tol = 0.5 * KR_TOL;
     std::vector<KrState> k(nc);
     int active = 0;
@@ -525,19 +681,15 @@ static int nm_kr(mk_norm *h, const std::vector<double> &kept_rows, std::vector<u
     return MK_OK;
 }
 
-extern "C" int mk_norm_device(mk_norm *h, const uint32_t *d_bin1, const uint32_t *d_bin2, const uint32_t *d_cnt, size_t nnz, int types,
-                              double *d_vc, double *d_vc_sqrt, double *d_kr, uint8_t *chrom_status, mk_norm_stats *stats, void *stream) {
-    if (!h || (nnz && (!d_bin1 || !d_bin2 || !d_cnt)) || (types & ~(MK_NORM_VC | MK_NORM_VC_SQRT | MK_NORM_KR)) ||
-        ((types & MK_NORM_VC) && !d_vc) || ((types & MK_NORM_VC_SQRT) && !d_vc_sqrt) || ((types & MK_NORM_KR) && !d_kr)) {
-        mk_set_error("mk_norm_device: bad argument"); return MK_ERR_ARG;
-    }
-    if (nnz > h->max_nnz) { mk_set_error("mk_norm_device: %zu entries, capacity %zu", nnz, h->max_nnz); return MK_ERR_CAPACITY; }
+// One call in h->scope: CSR, row sums, KR, the requested vectors with their sum factors.  status: n_seg() values.
+static int nm_run(mk_norm *h, const char *who, const u32 *d_bin1, const u32 *d_bin2, const u32 *d_cnt, size_t nnz, int types,
+                  double *d_vc, double *d_vc_sqrt, double *d_kr, uint8_t *status, mk_norm_stats *stats, cudaStream_t s) {
+    if (nnz > h->max_nnz) { mk_set_error("%s: %zu entries, capacity %zu", who, nnz, h->max_nnz); return MK_ERR_CAPACITY; }
     MK_CUDA(cudaSetDevice(h->device));
-    cudaStream_t s = (cudaStream_t)stream;
-    const int nc = h->n_chrom;
+    const int nc = h->n_seg();
     const u32 nb = h->nb;
     mk_norm_stats st; st.kr_outer_max = 0; st.kr_matvecs = 0; st.kr_failed = 0; st.kr_residual_max = 0.0;
-    MK_TRY(nm_build(h, d_bin1, d_bin2, d_cnt, nnz, s));
+    MK_TRY(nm_build(h, who, d_bin1, d_bin2, d_cnt, nnz, s));
     // row sums: VC, the raw totals of the sum factors, the rows KR keeps
     NormCmd *cmd = h->h_cmd.as<NormCmd>();
     const NormRes *res = h->h_res.as<NormRes>();
@@ -549,13 +701,13 @@ extern "C" int mk_norm_device(mk_norm *h, const uint32_t *d_bin1, const uint32_t
     if (types & MK_NORM_KR) MK_TRY(nm_kr(h, kept_rows, kr_ok, &st, s));
     MK_CUDA(cudaMemcpyAsync(h->d_krok.p, kr_ok.data(), nc, cudaMemcpyHostToDevice, s));
     const NormVecs V = h->vecs();
-    const u32 *cob = h->d_chr_of_bin.as<u32>();
+    const u32 *seg = h->seg_of_bin();
     const int kinds[3] = {MK_NORM_VC, MK_NORM_VC_SQRT, MK_NORM_KR};
     double *outs[3] = {d_vc, d_vc_sqrt, d_kr};
     for (int t = 0; t < 3; ++t) {
         if (!(types & kinds[t])) continue;
         if (h->timing) MK_CUDA(cudaEventRecord(h->ev[0], s));
-        k_nm_finish<<<h->grid(nb, NM_T), NM_T, 0, s>>>(t, nb, cob, h->d_krok.as<u8>(), V, outs[t]);
+        k_nm_finish<<<h->grid(nb, NM_T), NM_T, 0, s>>>(t, nb, seg, h->d_krok.as<u8>(), V, outs[t]);
         if (h->timing) MK_CUDA(cudaEventRecord(h->ev[1], s));
         h->launches += 1;
         if (h->timing) { MK_CUDA(cudaEventSynchronize(h->ev[1])); h->ms[5] += nm_elapsed(h->ev[0], h->ev[1]); h->count[5] += 1; }
@@ -565,12 +717,33 @@ extern "C" int mk_norm_device(mk_norm *h, const uint32_t *d_bin1, const uint32_t
         double *f = h->h_f.as<double>();
         for (int c = 0; c < nc; ++c) f[c] = cmd[c].op == OP_SUMF ? std::sqrt(res[c].a / raw[c]) : 1.0;
         MK_CUDA(cudaMemcpyAsync(h->d_f.p, f, nc * 8, cudaMemcpyHostToDevice, s));
-        k_nm_scale<<<h->grid(nb, NM_T), NM_T, 0, s>>>(nb, cob, h->d_f.as<double>(), outs[t]);
+        k_nm_scale<<<h->grid(nb, NM_T), NM_T, 0, s>>>(nb, seg, h->d_f.as<double>(), outs[t]);
         h->launches += 1;
     }
     MK_CUDA(cudaStreamSynchronize(s));
     MK_CUDA(cudaGetLastError());
-    if (chrom_status) for (int c = 0; c < nc; ++c) chrom_status[c] = raw[c] <= 0 ? 1 : ((types & MK_NORM_KR) && !kr_ok[c]) ? 2 : 0;
+    if (status) for (int c = 0; c < nc; ++c) status[c] = raw[c] <= 0 ? 1 : ((types & MK_NORM_KR) && !kr_ok[c]) ? 2 : 0;
     if (stats) *stats = st;
     return MK_OK;
+}
+
+extern "C" int mk_norm_device(mk_norm *h, const uint32_t *d_bin1, const uint32_t *d_bin2, const uint32_t *d_cnt, size_t nnz, int types,
+                              double *d_vc, double *d_vc_sqrt, double *d_kr, uint8_t *chrom_status, mk_norm_stats *stats, void *stream) {
+    if (!h || (nnz && (!d_bin1 || !d_bin2 || !d_cnt)) || (types & ~(MK_NORM_VC | MK_NORM_VC_SQRT | MK_NORM_KR)) ||
+        ((types & MK_NORM_VC) && !d_vc) || ((types & MK_NORM_VC_SQRT) && !d_vc_sqrt) || ((types & MK_NORM_KR) && !d_kr)) {
+        mk_set_error("mk_norm_device: bad argument"); return MK_ERR_ARG;
+    }
+    h->scope = NM_INTRA;
+    return nm_run(h, "mk_norm_device", d_bin1, d_bin2, d_cnt, nnz, types, d_vc, d_vc_sqrt, d_kr, chrom_status, stats, (cudaStream_t)stream);
+}
+
+extern "C" int mk_norm_genome_device(mk_norm *h, const uint32_t *d_bin1, const uint32_t *d_bin2, const uint32_t *d_cnt, size_t nnz, int scope,
+                                     int types, double *d_vc, double *d_kr, uint8_t *status, mk_norm_stats *stats, void *stream) {
+    // no VC_SQRT: juicer has no genome-wide or inter-chromosomal form of it
+    if (!h || (nnz && (!d_bin1 || !d_bin2 || !d_cnt)) || (scope != MK_NORM_SCOPE_GW && scope != MK_NORM_SCOPE_INTER) ||
+        (types & ~(MK_NORM_VC | MK_NORM_KR)) || ((types & MK_NORM_VC) && !d_vc) || ((types & MK_NORM_KR) && !d_kr)) {
+        mk_set_error("mk_norm_genome_device: bad argument"); return MK_ERR_ARG;
+    }
+    h->scope = scope;
+    return nm_run(h, "mk_norm_genome_device", d_bin1, d_bin2, d_cnt, nnz, types, d_vc, nullptr, d_kr, status, stats, (cudaStream_t)stream);
 }

@@ -1,11 +1,13 @@
-"""Matrix balancing on the GPU (csrc/norm.cu): time, products and bytes per product of VC, VC_SQRT and KR at the nine default
-resolutions (microcket:98), on seeded synthetic pairs over hg38 (power-law distance decay p(d) ~ 1/d, a trans fraction) binned on
-the GPU; plus an independent scipy `bnewt` on the 100 kb matrices of the largest size as the CPU reference point.
+"""Matrix balancing on the GPU (csrc/norm.cu): time, products and bytes per product of VC, VC_SQRT and KR (per chromosome) and of
+GW_VC / GW_KR (whole-genome matrix) and INTER_VC / INTER_KR (inter-chromosomal entries) at the nine default resolutions
+(microcket:98), on seeded synthetic pairs over hg38 (power-law distance decay p(d) ~ 1/d, a trans fraction) binned on the GPU;
+plus an independent scipy `bnewt` on the 100 kb matrices of the largest size (every chromosome's, and the genome-wide one) as
+the CPU reference points.
 
   python tools/norm_bench.py --out <record.json> [--pairs 20000000,250000000]
 
-Bytes per product are algorithmic: 8 B per stored entry (u32 column + u32 count; both halves of the symmetric intra matrix, the
-diagonal once) + 8 B per row pointer + 8 B per row of y.  The input vector u (8 B per bin, 4.9 MB at 5 kb) is a gather that
+Bytes per product are algorithmic: 8 B per stored entry (u32 column + u32 count; both halves of the symmetric matrix of the
+scope, the diagonal once: 2 nnz - diagonal) + 8 B per row pointer + 8 B per row of y.  The input vector u (8 B per bin, 4.9 MB at 5 kb) is a gather that
 stays in L2 and is not counted.  The rate is compared with the HBM peak bench.py uses (MEASURED_PEAKS.json `hbm_gbs`, else
 bench.py's fallback; the record names which).
 The full products are the row sums and the sum factors (every row); KR's products skip the rows of chromosomes that are done.
@@ -55,12 +57,12 @@ def synth_pairs(torch, n, seed, trans=0.2):
     return rec
 
 
-def matrix_shape(torch, b1, b2, nnz, res):
+def matrix_shape(torch, b1, b2, nnz, res, scope="INTRA"):
     off = torch.tensor(np.cumsum([l // res + 1 for l in HG38_LEN]), dtype=torch.int64, device="cuda")
     x, y = b1[:nnz].long(), b2[:nnz].long()
     ch1, ch2 = torch.bucketize(x, off, right=True), torch.bucketize(y, off, right=True)
-    intra = ch1 == ch2
-    stored = 2 * int(intra.sum()) - int((intra & (x == y)).sum())
+    m = {"INTRA": ch1 == ch2, "GW": torch.ones_like(x, dtype=torch.bool), "INTER": ch1 != ch2}[scope]
+    stored = 2 * int(m.sum()) - int((m & (x == y)).sum())
     return stored, int(off[-1])
 
 
@@ -76,6 +78,41 @@ def cpu_kr_100kb(b1, b2, ct):
         kept = np.asarray(A.sum(axis=1)).ravel() > 0
         ok += bnewt(A[kept][:, kept]) is not None
     return (time.perf_counter() - t0) * 1e3, ok
+
+
+def cpu_gw_kr_100kb(b1, b2, ct):
+    """the same bnewt on the 100 kb genome-wide matrix"""
+    from test_gpu_norm import bnewt, sym
+    nb = sum(l // 100000 + 1 for l in HG38_LEN)
+    t0 = time.perf_counter()
+    A = sym(nb, b1.astype(np.int64), b2.astype(np.int64), ct.astype(np.float64))
+    kept = np.asarray(A.sum(axis=1)).ravel() > 0
+    ok = bnewt(A[kept][:, kept]) is not None
+    return (time.perf_counter() - t0) * 1e3, ok
+
+
+def timed(torch, nm, call, bytes_full):
+    """one warmed-up call with the kernel timers on -> the record of one type"""
+    call()
+    nm.enable_timing(True)
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    status, st = call()
+    torch.cuda.synchronize()
+    wall = (time.perf_counter() - t0) * 1e3
+    kt = nm.kernel_times()
+    nm.enable_timing(False)
+    full_ms, full_n = kt["product"]
+    kr_ms, kr_n = kt["kr_product"]
+    t = {"total_ms": wall, "products": full_n + kr_n, "build_ms": kt["build"][0],
+         "ms_per_full_product": full_ms / full_n, "gbs_full_product": bytes_full / (full_ms / full_n) / 1e6}
+    if kr_n:
+        kv_ms, _ = kt["kr_vector"]
+        kw_ms, steps = kt["kr_wall"]
+        t.update({"kr_steps": steps, "kr_outer_max": st.kr_outer_max, "kr_failed": st.kr_failed, "kr_residual_max": st.kr_residual_max,
+                  "ms_per_kr_product": kr_ms / kr_n, "kr_vector_kernels_ms": kv_ms, "kr_vector_ms_per_step": kv_ms / steps,
+                  "kr_loop_wall_ms": kw_ms, "kr_host_round_trip_share": (kw_ms - kr_ms - kv_ms) / kw_ms if kw_ms else 0.0})
+    return t, status
 
 
 def main():
@@ -105,35 +142,35 @@ def main():
             out = torch.empty(rows, dtype=torch.float64, device="cuda")
             for typ in ("VC", "VC_SQRT", "KR"):
                 kw = {"d_" + typ.lower(): out.data_ptr()}
-                nm.run(b1.data_ptr(), b2.data_ptr(), ct.data_ptr(), nnz, (typ,), **kw)            # warm-up
-                nm.enable_timing(True)
-                torch.cuda.synchronize()
-                t0 = time.perf_counter()
-                status, st = nm.run(b1.data_ptr(), b2.data_ptr(), ct.data_ptr(), nnz, (typ,), **kw)
-                torch.cuda.synchronize()
-                wall = (time.perf_counter() - t0) * 1e3
-                kt = nm.kernel_times()
-                nm.enable_timing(False)
-                full_ms, full_n = kt["product"]
-                kr_ms, kr_n = kt["kr_product"]
-                t = {"total_ms": wall, "products": full_n + kr_n, "build_ms": kt["build"][0],
-                     "ms_per_full_product": full_ms / full_n, "gbs_full_product": bytes_full / (full_ms / full_n) / 1e6}
+                t, status = timed(torch, nm, lambda: nm.run(b1.data_ptr(), b2.data_ptr(), ct.data_ptr(), nnz, (typ,), **kw), bytes_full)
                 t["share_of_hbm_peak"] = t["gbs_full_product"] / peak
                 if typ == "KR":
-                    kv_ms, _ = kt["kr_vector"]
-                    kw_ms, steps = kt["kr_wall"]
-                    t.update({"kr_steps": steps, "kr_outer_max": st.kr_outer_max, "kr_failed": st.kr_failed, "kr_residual_max": st.kr_residual_max,
-                              "ms_per_kr_product": kr_ms / max(kr_n, 1), "kr_vector_kernels_ms": kv_ms, "kr_loop_wall_ms": kw_ms,
-                              "kr_host_round_trip_share": (kw_ms - kr_ms - kv_ms) / kw_ms if kw_ms else 0.0,
-                              "failed_chromosomes": [i for i, s in enumerate(status) if s == 2]})
+                    t["failed_chromosomes"] = [i for i, s in enumerate(status) if s == 2]
                 row["types"][typ] = t
                 print(json.dumps({"pairs": n, "res": res, "type": typ, **{k: v for k, v in t.items() if k != "failed_chromosomes"}}), flush=True)
+            for scope in ("GW", "INTER"):
+                sstored, _ = matrix_shape(torch, b1, b2, nnz, res, scope)
+                sbytes = 8 * sstored + 16 * rows
+                row[scope] = {"stored_entries": sstored, "bytes_per_product": sbytes, "types": {}}
+                for typ in ("VC", "KR"):
+                    kw = {"d_" + typ.lower(): out.data_ptr()}
+                    t, status = timed(torch, nm, lambda: nm.run_genome(b1.data_ptr(), b2.data_ptr(), ct.data_ptr(), nnz, scope, (typ,), **kw), sbytes)
+                    t["share_of_hbm_peak"] = t["gbs_full_product"] / peak
+                    t["status"] = status
+                    if typ == "KR" and t.get("kr_steps"):
+                        t["gbs_kr_product"] = sbytes / t["ms_per_kr_product"] / 1e6
+                        t["kr_vector_over_product"] = t["kr_vector_ms_per_step"] / t["ms_per_kr_product"]
+                    row[scope]["types"][typ] = t
+                    print(json.dumps({"pairs": n, "res": res, "type": f"{scope}_{typ}", **t}), flush=True)
             nm.close()
             if res == 100000 and n == max(int(s) for s in a.pairs.split(",")):
                 host = [x[:nnz].cpu().numpy().astype(np.uint32) for x in (b1, b2, ct)]
                 ms, ok = cpu_kr_100kb(*host)
+                gms, gok = cpu_gw_kr_100kb(*host)
                 cpu_ref = {"pairs": n, "res": 100000, "scipy_bnewt_ms": ms, "chromosomes_balanced": ok,
-                           "gpu_kr_total_ms": row["types"]["KR"]["total_ms"], "cpu": os.cpu_count()}
+                           "gpu_kr_total_ms": row["types"]["KR"]["total_ms"],
+                           "scipy_gw_bnewt_ms": gms, "gw_balanced": gok, "gpu_gw_kr_total_ms": row["GW"]["types"]["KR"]["total_ms"],
+                           "cpu": os.cpu_count()}
                 print(json.dumps(cpu_ref), flush=True)
             size["resolutions"].append(row)
         rec["sizes"].append(size)
