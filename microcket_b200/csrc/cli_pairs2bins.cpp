@@ -32,92 +32,77 @@ using namespace std;
 
 #define CHECK(call) do { if ((call) != MK_OK) { cerr << "Error: " << mk_last_error() << "\n"; return 20; } } while (0)
 
+// -n: the normalisation types, in the order their vectors go into the container.  scope 0: per chromosome (mk_norm_device),
+// else the MK_NORM_SCOPE_* of mk_norm_genome_device; bit: the type's MK_NORM_* bit in that call.
+static const struct { const char *name; int scope, bit; } NORMS[] = {
+    {"VC", 0, MK_NORM_VC}, {"VC_SQRT", 0, MK_NORM_VC_SQRT}, {"KR", 0, MK_NORM_KR},
+    {"GW_VC", MK_NORM_SCOPE_GW, MK_NORM_VC}, {"GW_KR", MK_NORM_SCOPE_GW, MK_NORM_KR},
+    {"INTER_VC", MK_NORM_SCOPE_INTER, MK_NORM_VC}, {"INTER_KR", MK_NORM_SCOPE_INTER, MK_NORM_KR}};
+static const int N_NORMS = sizeof NORMS / sizeof NORMS[0];
+
 static hic::Writer *g_hic = NULL;                                         // -H: every resolution's arrays also go into the container
-static int g_norm_types = 0, g_dev = 0;                                   // -n: MK_NORM_* bits of the per-chromosome vectors
-static int g_scope_types[2] = {0, 0};                                     // -n: MK_NORM_VC / MK_NORM_KR bits of GW_*, INTER_*
+static int g_norms = 0, g_dev = 0;                                        // -n: bit i requests NORMS[i]
 static vector<uint32_t> g_len; static vector<string> g_names;
 
-// the per-chromosome vectors (mk_norm_device)
-static int balance_intra(mk_norm *nm, uint32_t res, uint64_t nb, const void *d_b1, const void *d_b2, const void *d_ct, size_t nnz,
-                         vector<vector<double>> &vals, vector<hic::NormInput> &norms) {
-    static const char *names[3] = {"VC", "VC_SQRT", "KR"};
-    void *d_out[3] = {NULL, NULL, NULL};
-    for (int t = 0; t < 3; ++t) if (g_norm_types & (1 << t)) CHECK(mk_dev_alloc(g_dev, nb * 8 + 8, &d_out[t]));
-    vector<uint8_t> status(g_len.size(), 0); mk_norm_stats st;
-    CHECK(mk_norm_device(nm, (const uint32_t *)d_b1, (const uint32_t *)d_b2, (const uint32_t *)d_ct, nnz, g_norm_types,
-                         (double *)d_out[0], (double *)d_out[1], (double *)d_out[2], status.data(), &st, NULL));
-    for (int t = 0; t < 3; ++t) {
-        if (!d_out[t]) continue;
-        vals[t].resize(nb);
-        CHECK(mk_copy_to_host(vals[t].data(), d_out[t], nb * 8));
-        mk_dev_free(d_out[t]);
-        hic::NormInput q; q.type = names[t]; q.values = vals[t].data();
-        for (size_t c = 0; c < g_len.size(); ++c) q.stored.push_back(status[c] == 0 || (status[c] == 2 && t < 2));
-        norms.push_back(q);
-    }
-    if (g_norm_types & MK_NORM_KR) {
-        string failed;
-        for (size_t c = 0; c < g_len.size(); ++c) if (status[c] == 2) failed += (failed.empty() ? "" : ", ") + g_names[c];
-        cerr << "INFO: KR at " << res << " bp: " << st.kr_matvecs << " steps, " << st.kr_failed << " chromosome(s) failed"
-             << (failed.empty() ? "" : ": " + failed) << ".\n";
-    }
-    return 0;
-}
-
-// GW_* (k = 0) or INTER_* (k = 1) vectors (mk_norm_genome_device).  A chromosome's slice is stored when the matrix has entries,
-// the type did not fail, and one of the chromosome's rows has a valid norm, i.e. a nonzero row sum in that matrix.
-static int balance_genome(mk_norm *nm, int k, uint32_t res, uint64_t nb, const void *d_b1, const void *d_b2, const void *d_ct, size_t nnz,
-                          vector<vector<double>> &vals, vector<hic::NormInput> &norms) {
-    static const char *names[2][2] = {{"GW_VC", "GW_KR"}, {"INTER_VC", "INTER_KR"}};
-    const int types = g_scope_types[k];
-    void *d_out[2] = {NULL, NULL};
-    for (int t = 0; t < 2; ++t) if (types & (t ? MK_NORM_KR : MK_NORM_VC)) CHECK(mk_dev_alloc(g_dev, nb * 8 + 8, &d_out[t]));
-    uint8_t status = 0; mk_norm_stats st;
-    CHECK(mk_norm_genome_device(nm, (const uint32_t *)d_b1, (const uint32_t *)d_b2, (const uint32_t *)d_ct, nnz,
-                                k ? MK_NORM_SCOPE_INTER : MK_NORM_SCOPE_GW, types, (double *)d_out[0], (double *)d_out[1], &status, &st, NULL));
-    for (int t = 0; t < 2; ++t) {
-        if (!d_out[t]) continue;
-        vector<double> &v = vals[3 + 2 * k + t];
-        v.resize(nb);
-        CHECK(mk_copy_to_host(v.data(), d_out[t], nb * 8));
-        mk_dev_free(d_out[t]);
-        hic::NormInput q; q.type = names[k][t]; q.values = v.data();
-        const bool ok = status == 0 || (status == 2 && t == 0);
-        for (size_t c = 0, o = 0; c < g_len.size(); ++c) {
-            const size_t e = o + g_len[c] / res + 1;
-            bool any = false;
-            for (size_t r = o; r < e && ok && !any; ++r) any = isfinite(v[r]) && v[r] > 0;
-            q.stored.push_back(any);
-            o = e;
-        }
-        norms.push_back(q);
-    }
-    if (types & MK_NORM_KR)
-        cerr << "INFO: " << names[k][1] << " at " << res << " bp: " << st.kr_matvecs << " steps, "
-             << (status == 0 ? "the matrix balanced" : status == 1 ? "the matrix has no entries" : "the matrix did not balance") << ".\n";
-    return 0;
-}
-
-// -n: the resolution's normalisation vectors from its device COO, copied to the host for the writer
+// -n: the resolution's normalisation vectors from its device COO, copied to the host for the writer; one library call per scope.
+// A chromosome's slice is stored when it holds a finite value > 0: a type that failed or a matrix without entries leaves NaN or 0.
 static int balance(uint32_t res, const void *d_b1, const void *d_b2, const void *d_ct, size_t nnz, vector<vector<double>> &vals, vector<hic::NormInput> &norms) {
     uint64_t nb = 0; CHECK(mk_hist_cells(g_len.data(), (int)g_len.size(), res, &nb, NULL));
     mk_norm *nm = NULL;
     CHECK(mk_norm_create(g_dev, g_len.data(), (int)g_len.size(), res, nnz, &nm));
-    vals.assign(7, vector<double>());                                     // VC, VC_SQRT, KR, GW_VC, GW_KR, INTER_VC, INTER_KR
-    int rc = g_norm_types ? balance_intra(nm, res, nb, d_b1, d_b2, d_ct, nnz, vals, norms) : 0;
-    for (int k = 0; k < 2 && !rc; ++k) if (g_scope_types[k]) rc = balance_genome(nm, k, res, nb, d_b1, d_b2, d_ct, nnz, vals, norms);
+    vals.assign(N_NORMS, vector<double>());
+    const uint32_t *b1 = (const uint32_t *)d_b1, *b2 = (const uint32_t *)d_b2, *ct = (const uint32_t *)d_ct;
+    for (int scope : {0, MK_NORM_SCOPE_GW, MK_NORM_SCOPE_INTER}) {
+        int types = 0;
+        void *d_out[N_NORMS] = {};
+        double *arg[MK_NORM_KR + 1] = {};                                 // the call's output arguments, by MK_NORM_* bit
+        const char *kr = NULL;                                            // the KR type's name, when requested
+        for (int i = 0; i < N_NORMS; ++i) {
+            if (!(g_norms >> i & 1) || NORMS[i].scope != scope) continue;
+            CHECK(mk_dev_alloc(g_dev, nb * 8 + 8, &d_out[i]));
+            types |= NORMS[i].bit; arg[NORMS[i].bit] = (double *)d_out[i];
+            if (NORMS[i].bit == MK_NORM_KR) kr = NORMS[i].name;
+        }
+        if (!types) continue;
+        vector<uint8_t> status(scope ? 1 : g_len.size(), 0); mk_norm_stats st;
+        CHECK(scope ? mk_norm_genome_device(nm, b1, b2, ct, nnz, scope, types, arg[MK_NORM_VC], arg[MK_NORM_KR], status.data(), &st, NULL)
+                    : mk_norm_device(nm, b1, b2, ct, nnz, types, arg[MK_NORM_VC], arg[MK_NORM_VC_SQRT], arg[MK_NORM_KR], status.data(), &st, NULL));
+        for (int i = 0; i < N_NORMS; ++i) {
+            if (!d_out[i]) continue;
+            vector<double> &v = vals[i];
+            v.resize(nb);
+            CHECK(mk_copy_to_host(v.data(), d_out[i], nb * 8));
+            mk_dev_free(d_out[i]);
+            hic::NormInput q; q.type = NORMS[i].name; q.values = v.data();
+            for (size_t c = 0, o = 0; c < g_len.size(); ++c) {
+                const size_t e = o + g_len[c] / res + 1;
+                bool any = false;
+                for (size_t r = o; r < e && !any; ++r) any = isfinite(v[r]) && v[r] > 0;
+                q.stored.push_back(any);
+                o = e;
+            }
+            norms.push_back(q);
+        }
+        if (!kr) continue;
+        cerr << "INFO: " << kr << " at " << res << " bp: " << st.kr_matvecs << " steps, ";
+        if (scope) cerr << (status[0] == 0 ? "the matrix balanced" : status[0] == 1 ? "the matrix has no entries" : "the matrix did not balance") << ".\n";
+        else {
+            string failed;
+            for (size_t c = 0; c < g_len.size(); ++c) if (status[c] == 2) failed += (failed.empty() ? "" : ", ") + g_names[c];
+            cerr << st.kr_failed << " chromosome(s) failed" << (failed.empty() ? "" : ": " + failed) << ".\n";
+        }
+    }
     mk_norm_destroy(nm);
-    return rc;
+    return 0;
 }
 
 static int write_coo(const string &prefix, uint32_t res, const void *d_b1, const void *d_b2, const void *d_ct, size_t nnz) {
     const string path = prefix + "." + to_string(res) + ".coo";
     vector<vector<double>> vals; vector<hic::NormInput> norms;           // before the copy: the device arrays are reused afterwards
-    const bool norm = g_norm_types || g_scope_types[0] || g_scope_types[1];
-    if (norm) if (int rc = balance(res, d_b1, d_b2, d_ct, nnz, vals, norms)) return rc;
+    if (g_norms) if (int rc = balance(res, d_b1, d_b2, d_ct, nnz, vals, norms)) return rc;
     vector<uint32_t> b1(nnz + 1), b2(nnz + 1), ct(nnz + 1);
     if (nnz) { CHECK(mk_copy_to_host(b1.data(), d_b1, nnz * 4)); CHECK(mk_copy_to_host(b2.data(), d_b2, nnz * 4)); CHECK(mk_copy_to_host(ct.data(), d_ct, nnz * 4)); }
-    if (g_hic) { string err; if (g_hic->add(res, b1.data(), b2.data(), ct.data(), nnz, &err, norm ? &norms : NULL)) { cerr << "Error: " << err << "\n"; return 10; } }
+    if (g_hic) { string err; if (g_hic->add(res, b1.data(), b2.data(), ct.data(), nnz, &err, g_norms ? &norms : NULL)) { cerr << "Error: " << err << "\n"; return 10; } }
     FILE *fo = fopen(path.c_str(), "w");
     if (!fo) { cerr << "Error: cannot write " << path << "\n"; return 10; }
     static char big[1 << 22];
@@ -142,14 +127,13 @@ int main(int argc, char *argv[]) {
     if (!normlist.empty()) {
         stringstream ss(normlist); string t;
         while (getline(ss, t, ',')) {
-            if (t == "VC") g_norm_types |= MK_NORM_VC;
-            else if (t == "VC_SQRT") g_norm_types |= MK_NORM_VC_SQRT;
-            else if (t == "KR") g_norm_types |= MK_NORM_KR;
-            else if (t == "GW_VC") g_scope_types[0] |= MK_NORM_VC;
-            else if (t == "GW_KR") g_scope_types[0] |= MK_NORM_KR;
-            else if (t == "INTER_VC") g_scope_types[1] |= MK_NORM_VC;
-            else if (t == "INTER_KR") g_scope_types[1] |= MK_NORM_KR;
-            else { cerr << "Error: unknown normalisation '" << t << "' (VC, VC_SQRT, KR, GW_VC, GW_KR, INTER_VC, INTER_KR)\n"; return 2; }
+            int i = 0;
+            while (i < N_NORMS && t != NORMS[i].name) ++i;
+            if (i < N_NORMS) { g_norms |= 1 << i; continue; }
+            cerr << "Error: unknown normalisation '" << t << "' (";
+            for (i = 0; i < N_NORMS; ++i) cerr << (i ? ", " : "") << NORMS[i].name;
+            cerr << ")\n";
+            return 2;
         }
     }
     if (argc - a < 3 || reslist.empty() || (!normlist.empty() && hic_path.empty())) {

@@ -23,8 +23,9 @@
 //   k_nm_spmv         y = A u: one warp per row, every lane sums a fixed stride of the row in order, then a fixed
 //                     butterfly: no floating-point atomics, so the vectors are bitwise reproducible from run to run
 //   k_nm_pre          per row, the vector that goes into the next product, from its chromosome's command
-//   k_nm_post         one CTA per chromosome: the vector updates and segmented reductions after a product (INTRA)
-//   k_nm_gpost        the same work for the one segment of GENOME / INTER, over fixed slices of NM_GS rows in 1 or 3 phases
+//   k_nm_post         the vector updates and reductions after a product, one CTA per chromosome (INTRA), in one launch
+//   k_nm_gpost        the same for the one segment of GENOME / INTER, over fixed slices of NM_GS rows, in 1 or 3 launches;
+//                     both run the same per-row phases (nm_row_sums ... nm_cg_update) and scalar decisions (nm_alpha ...)
 //   k_nm_finish       1 / x (KR) or sqrt (VC_SQRT) into the output vectors; k_nm_scale: the sum factors
 //
 // KR runs for all segments in lockstep: every step is k_nm_pre -> k_nm_spmv -> k_nm_post (k_nm_gpost), and the per-segment
@@ -59,7 +60,7 @@ enum { NM_INTRA = 0, NM_GENOME = MK_NORM_SCOPE_GW, NM_INTER = MK_NORM_SCOPE_INTE
 
 struct NormCmd { int op, pad; double beta, rho; };             // host -> device, one per chromosome and step
 struct NormRes { double a, b, c; int flag, pad; };             // device -> host
-struct NormPart { double a, b, c, d; };                         // one slice's partials of one k_nm_gpost phase
+struct NormPart { double a, b, c, d; };                         // a phase's totals over one CTA's rows (in k_nm_gpost: one slice's)
 static_assert(sizeof(NormRes) == sizeof(NormPart), "k_nm_gpost's result sits behind its final partials, copied in one piece");
 
 struct NormVecs { double *x, *v, *rk, *y, *z, *p, *w, *u, *au, *rs; u8 *kept; };   // rs: row sums (au is every product's output)
@@ -209,38 +210,26 @@ __global__ void __launch_bounds__(NM_T) k_nm_pre(u32 nb, const u32 *seg_of_bin, 
     }
 }
 
-// ---------------------------------------------------------------- per-chromosome updates and reductions after a product
-// Every thread walks a fixed stride of the chromosome's rows in order, then a fixed tree: the same bits on every run.
-// NW: warps in the CTA (k_nm_post 32, k_nm_gpost NM_T / 32).
-template <int NW = NM_RT / 32>
-__device__ __forceinline__ double nm_bsum(double v, double *sh) {
+// ---------------------------------------------------------------- updates and reductions after a product
+// A phase walks rows [r0, r1) with a stride of NT from threadIdx.x, in order, updates V, and reduces its per-thread partials
+// over the CTA's NT threads with a fixed tree (nm_bred): the same bits on every run.  It returns the CTA's totals, several of
+// them as a NormPart.
+enum { RED_SUM = 0, RED_MIN, RED_MAX };
+template <int OP> __device__ __forceinline__ double nm_op(double a, double b) { return OP == RED_SUM ? a + b : OP == RED_MIN ? fmin(a, b) : fmax(a, b); }
+template <int OP> __device__ __forceinline__ double nm_pad() { return OP == RED_SUM ? 0.0 : OP == RED_MIN ? INFINITY : -INFINITY; }
+
+// NW <= 32 warps: each warp's butterfly, then one over the warps' results in warp 0.  sh: 33 doubles
+template <int OP, int NW>
+__device__ __forceinline__ double nm_bred(double v, double *sh) {
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
 #pragma unroll
-    for (int d = 16; d; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
+    for (int d = 16; d; d >>= 1) v = nm_op<OP>(v, __shfl_xor_sync(0xffffffffu, v, d));
     if (lane == 0) sh[wid] = v;
     __syncthreads();
     if (wid == 0) {
-        double t = lane < NW ? sh[lane] : 0.0;
+        double t = lane < NW ? sh[lane] : nm_pad<OP>();
 #pragma unroll
-        for (int d = 16; d; d >>= 1) t += __shfl_xor_sync(0xffffffffu, t, d);
-        if (lane == 0) sh[32] = t;
-    }
-    __syncthreads();
-    const double r = sh[32];
-    __syncthreads();
-    return r;
-}
-template <bool MAX, int NW = NM_RT / 32>
-__device__ __forceinline__ double nm_bext(double v, double *sh) {
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-#pragma unroll
-    for (int d = 16; d; d >>= 1) { const double o = __shfl_xor_sync(0xffffffffu, v, d); v = MAX ? fmax(v, o) : fmin(v, o); }
-    if (lane == 0) sh[wid] = v;
-    __syncthreads();
-    if (wid == 0) {
-        double t = lane < NW ? sh[lane] : (MAX ? -INFINITY : INFINITY);
-#pragma unroll
-        for (int d = 16; d; d >>= 1) { const double o = __shfl_xor_sync(0xffffffffu, t, d); t = MAX ? fmax(t, o) : fmin(t, o); }
+        for (int d = 16; d; d >>= 1) t = nm_op<OP>(t, __shfl_xor_sync(0xffffffffu, t, d));
         if (lane == 0) sh[32] = t;
     }
     __syncthreads();
@@ -249,6 +238,91 @@ __device__ __forceinline__ double nm_bext(double v, double *sh) {
     return r;
 }
 
+// row sums (OP_ONES) -> {raw total, rows kept by KR}
+template <int NT>
+__device__ __forceinline__ NormPart nm_row_sums(const NormVecs &V, u32 r0, u32 r1, double *sh) {
+    double s = 0.0, k = 0.0;
+    for (u32 r = r0 + threadIdx.x; r < r1; r += NT) { const double a = V.au[r]; s += a; k += a > 0.0; V.rs[r] = a; V.kept[r] = a > 0.0; }
+    return NormPart{nm_bred<RED_SUM, NT / 32>(s, sh), nm_bred<RED_SUM, NT / 32>(k, sh), 0.0, 0.0};
+}
+
+// the sum factor's u·(A u) (OP_SUMF)
+template <int NT>
+__device__ __forceinline__ double nm_sumf(const NormVecs &V, u32 r0, u32 r1, double *sh) {
+    double s = 0.0;
+    for (u32 r = r0 + threadIdx.x; r < r1; r += NT) s += V.u[r] * V.au[r];
+    return nm_bred<RED_SUM, NT / 32>(s, sh);
+}
+
+// after A x (OP_KR_INIT / OP_KR_OUTER): v = x (A x), rk = 1 - v -> {rk·rk, min x, > 0 when an x or v is not finite}
+template <int NT>
+__device__ __forceinline__ NormPart nm_outer(const NormVecs &V, u32 r0, u32 r1, double *sh) {
+    double s = 0.0, xmin = INFINITY; int bad = 0;
+    for (u32 r = r0 + threadIdx.x; r < r1; r += NT) {
+        if (!V.kept[r]) continue;
+        const double x = V.x[r], v = x * V.au[r], rk = 1.0 - v;
+        V.v[r] = v; V.rk[r] = rk;
+        s += rk * rk; xmin = fmin(xmin, x); bad |= !isfinite(x) || !isfinite(v);
+    }
+    return NormPart{nm_bred<RED_SUM, NT / 32>(s, sh), nm_bred<RED_MIN, NT / 32>(xmin, sh), nm_bred<RED_SUM, NT / 32>((double)bad, sh), 0.0};
+}
+
+// a CG step's product A (x p): w -> {p·w, rk·Z}
+template <int NT>
+__device__ __forceinline__ NormPart nm_cg_product(const NormVecs &V, u32 r0, u32 r1, double *sh) {
+    double pw = 0.0, rz = 0.0;
+    for (u32 r = r0 + threadIdx.x; r < r1; r += NT) {
+        if (!V.kept[r]) continue;
+        const double p = V.p[r], w = V.x[r] * V.au[r] + V.v[r] * p;
+        V.w[r] = w; pw += p * w; rz += V.rk[r] * V.z[r];
+    }
+    return NormPart{nm_bred<RED_SUM, NT / 32>(pw, sh), nm_bred<RED_SUM, NT / 32>(rz, sh), 0.0, 0.0};
+}
+
+// the box test of y + alpha p -> {min, max, step to the lower edge, step to the upper edge}
+template <int NT>
+__device__ __forceinline__ NormPart nm_box(const NormVecs &V, u32 r0, u32 r1, double alpha, double *sh) {
+    double ymin = INFINITY, ymax = -INFINITY, glo = INFINITY, ghi = INFINITY;
+    for (u32 r = r0 + threadIdx.x; r < r1; r += NT) {
+        if (!V.kept[r]) continue;
+        const double y = V.y[r], ap = alpha * V.p[r], yn = y + ap;
+        ymin = fmin(ymin, yn); ymax = fmax(ymax, yn);
+        if (ap < 0.0) glo = fmin(glo, (KR_DELTA - y) / ap);
+        if (yn > KR_DELTA_HI) ghi = fmin(ghi, (KR_DELTA_HI - y) / ap);
+    }
+    return NormPart{nm_bred<RED_MIN, NT / 32>(ymin, sh), nm_bred<RED_MAX, NT / 32>(ymax, sh), nm_bred<RED_MIN, NT / 32>(glo, sh),
+                    nm_bred<RED_MIN, NT / 32>(ghi, sh)};
+}
+
+// the step that leaves the box stops at its edge
+template <int NT>
+__device__ __forceinline__ void nm_edge(const NormVecs &V, u32 r0, u32 r1, double gamma, double alpha) {
+    for (u32 r = r0 + threadIdx.x; r < r1; r += NT) if (V.kept[r]) V.y[r] = V.y[r] + gamma * (alpha * V.p[r]);
+}
+
+// the step inside the box: y, rk, Z -> the new rk·Z
+template <int NT>
+__device__ __forceinline__ double nm_cg_update(const NormVecs &V, u32 r0, u32 r1, double alpha, double *sh) {
+    double s = 0.0;
+    for (u32 r = r0 + threadIdx.x; r < r1; r += NT) {
+        if (!V.kept[r]) continue;
+        const double rk = V.rk[r] - alpha * V.w[r], z = rk / V.v[r];
+        V.y[r] = V.y[r] + alpha * V.p[r]; V.rk[r] = rk; V.z[r] = z; s += rk * z;
+    }
+    return nm_bred<RED_SUM, NT / 32>(s, sh);
+}
+
+// A CG step's scalars from nm_cg_product's totals: rho is the step's rk·Z at OP_CG_FIRST, else the last update's.
+// false: alpha is not finite, the segment fails.
+__device__ __forceinline__ bool nm_alpha(const NormCmd &cm, const NormPart &pr, double &rho, double &alpha) {
+    rho = cm.op == OP_CG_FIRST ? pr.b : cm.rho; alpha = rho / pr.a;
+    return isfinite(alpha);
+}
+// from nm_box's totals: the step leaves the box (stop at its edge, end the inner loop), and the edge's gamma
+__device__ __forceinline__ bool nm_leaves_box(double ymin, double ymax) { return ymin <= KR_DELTA || ymax >= KR_DELTA_HI; }
+__device__ __forceinline__ double nm_gamma(double ymin, double glo, double ghi) { return ymin <= KR_DELTA ? glo : ghi; }
+
+// one CTA per chromosome, every phase of the step in one launch
 __global__ void __launch_bounds__(NM_RT) k_nm_post(const u32 *chr_off, const NormCmd *cmd, NormVecs V, NormRes *res) {
     __shared__ double sh[33];
     const int c = blockIdx.x;
@@ -256,81 +330,41 @@ __global__ void __launch_bounds__(NM_RT) k_nm_post(const u32 *chr_off, const Nor
     if (cm.op == OP_IDLE) return;
     const u32 r0 = chr_off[c], r1 = chr_off[c + 1];
     NormRes out = {0.0, 0.0, 0.0, 0, 0};
-    if (cm.op == OP_ONES) {                                           // row sums: raw total and rows kept by KR
-        double s = 0.0, k = 0.0;
-        for (u32 r = r0 + threadIdx.x; r < r1; r += NM_RT) { const double a = V.au[r]; s += a; k += a > 0.0; V.rs[r] = a; V.kept[r] = a > 0.0; }
-        out.a = nm_bsum(s, sh); out.b = nm_bsum(k, sh);
+    if (cm.op == OP_ONES) {
+        const NormPart t = nm_row_sums<NM_RT>(V, r0, r1, sh);
+        out.a = t.a; out.b = t.b;
     } else if (cm.op == OP_SUMF) {
-        double s = 0.0;
-        for (u32 r = r0 + threadIdx.x; r < r1; r += NM_RT) s += V.u[r] * V.au[r];
-        out.a = nm_bsum(s, sh);
-    } else if (cm.op == OP_KR_INIT || cm.op == OP_KR_OUTER) {         // v = x (A x), rk = 1 - v
-        double s = 0.0, xmin = INFINITY; int bad = 0;
-        for (u32 r = r0 + threadIdx.x; r < r1; r += NM_RT) {
-            if (!V.kept[r]) continue;
-            const double x = V.x[r], v = x * V.au[r], rk = 1.0 - v;
-            V.v[r] = v; V.rk[r] = rk;
-            s += rk * rk; xmin = fmin(xmin, x); bad |= !isfinite(x) || !isfinite(v);
-        }
-        out.a = nm_bsum(s, sh); out.b = nm_bext<false>(xmin, sh); out.flag = nm_bsum((double)bad, sh) > 0.0;
-    } else {                                                          // one CG step on the product A (x p)
-        double pw = 0.0, rz = 0.0;
-        for (u32 r = r0 + threadIdx.x; r < r1; r += NM_RT) {
-            if (!V.kept[r]) continue;
-            const double p = V.p[r], w = V.x[r] * V.au[r] + V.v[r] * p;
-            V.w[r] = w; pw += p * w; rz += V.rk[r] * V.z[r];
-        }
-        pw = nm_bsum(pw, sh); rz = nm_bsum(rz, sh);
-        const double rho = cm.op == OP_CG_FIRST ? rz : cm.rho, alpha = rho / pw;
+        out.a = nm_sumf<NM_RT>(V, r0, r1, sh);
+    } else if (cm.op == OP_KR_INIT || cm.op == OP_KR_OUTER) {
+        const NormPart t = nm_outer<NM_RT>(V, r0, r1, sh);
+        out.a = t.a; out.b = t.b; out.flag = t.c > 0.0;
+    } else {
+        double rho, alpha;
+        const bool ok = nm_alpha(cm, nm_cg_product<NM_RT>(V, r0, r1, sh), rho, alpha);
         out.a = rho; out.c = alpha;
-        if (!isfinite(alpha)) out.flag = ST_FAIL;
+        if (!ok) out.flag = ST_FAIL;
         else {
-            double ymin = INFINITY, ymax = -INFINITY, glo = INFINITY, ghi = INFINITY;
-            for (u32 r = r0 + threadIdx.x; r < r1; r += NM_RT) {
-                if (!V.kept[r]) continue;
-                const double y = V.y[r], ap = alpha * V.p[r], yn = y + ap;
-                ymin = fmin(ymin, yn); ymax = fmax(ymax, yn);
-                if (ap < 0.0) glo = fmin(glo, (KR_DELTA - y) / ap);
-                if (yn > KR_DELTA_HI) ghi = fmin(ghi, (KR_DELTA_HI - y) / ap);
-            }
-            ymin = nm_bext<false>(ymin, sh); ymax = nm_bext<true>(ymax, sh); glo = nm_bext<false>(glo, sh); ghi = nm_bext<false>(ghi, sh);
-            if (ymin <= KR_DELTA || ymax >= KR_DELTA_HI) {            // the step leaves the box: stop at its edge, end the inner loop
-                const double gamma = ymin <= KR_DELTA ? glo : ghi;
-                for (u32 r = r0 + threadIdx.x; r < r1; r += NM_RT) if (V.kept[r]) V.y[r] = V.y[r] + gamma * (alpha * V.p[r]);
-                out.flag = ST_CG_BREAK;
-            } else {
-                double s = 0.0;
-                for (u32 r = r0 + threadIdx.x; r < r1; r += NM_RT) {
-                    if (!V.kept[r]) continue;
-                    const double rk = V.rk[r] - alpha * V.w[r], z = rk / V.v[r];
-                    V.y[r] = V.y[r] + alpha * V.p[r]; V.rk[r] = rk; V.z[r] = z; s += rk * z;
-                }
-                out.b = nm_bsum(s, sh);
-                out.flag = ST_CG_CONT;
-            }
+            const NormPart box = nm_box<NM_RT>(V, r0, r1, alpha, sh);
+            if (nm_leaves_box(box.a, box.b)) { nm_edge<NM_RT>(V, r0, r1, nm_gamma(box.a, box.c, box.d), alpha); out.flag = ST_CG_BREAK; }
+            else { out.b = nm_cg_update<NM_RT>(V, r0, r1, alpha, sh); out.flag = ST_CG_CONT; }
         }
     }
     if (threadIdx.x == 0) res[c] = out;
 }
 
-// ---------------------------------------------------------------- the same for the one segment of GENOME / INTER
+// ---------------------------------------------------------------- the same phases for the one segment of GENOME / INTER
 // One CTA per segment would stream every vector of 617 669 rows (hg38 at 5 kb) through one SM.  The rows are cut into slices
-// of NM_GS; a CTA walks slices blockIdx.x, + gridDim.x, ... and writes one NormPart per slice and phase.  A CG step's dependent
-// reductions are three launches: phase 0 the product's update (w) with p·w and rk·Z, phase 1 alpha and the box test's extrema,
-// phase 2 the update and the new rk·Z.  In phases 1 and 2 every CTA recomputes the totals of the earlier phases from their
-// partials (nm_gtot: in slice order, then a fixed tree), so every CTA takes the same decision and the bits depend on the slice
-// width only, not on the grid.  The other ops need phase 0 only.  The final partials (pf) and phase 2's scalars (res) go to the
-// host in one copy; nm_gres sums them there in slice order.
-__device__ __forceinline__ double nm_gsum(const NormPart *p, u32 ns, int f, double *sh) {
-    double s = 0.0;
-    for (u32 i = threadIdx.x; i < ns; i += NM_T) s += (&p[i].a)[f];
-    return nm_bsum<NM_T / 32>(s, sh);
-}
-template <bool MAX>
-__device__ __forceinline__ double nm_gext(const NormPart *p, u32 ns, int f, double *sh) {
-    double s = MAX ? -INFINITY : INFINITY;
-    for (u32 i = threadIdx.x; i < ns; i += NM_T) s = MAX ? fmax(s, (&p[i].a)[f]) : fmin(s, (&p[i].a)[f]);
-    return nm_bext<MAX, NM_T / 32>(s, sh);
+// of NM_GS; a CTA runs the phase on slices blockIdx.x, + gridDim.x, ... and writes one NormPart per slice.  A CG step's
+// dependent reductions are three launches: phase 0 nm_cg_product, phase 1 nm_box, phase 2 nm_edge or nm_cg_update.  In
+// phases 1 and 2 every CTA recomputes the totals of the earlier phases from their partials (nm_gred: in slice order, then a
+// fixed tree), so every CTA takes the same decision and the bits depend on the slice width only, not on the grid.  The other
+// ops need phase 0 only.  The final partials (pf) and phase 2's scalars (res) go to the host in one copy; nm_gres sums them
+// there in slice order.
+template <int OP>
+__device__ __forceinline__ double nm_gred(const NormPart *p, u32 ns, int f, double *sh) {
+    double s = nm_pad<OP>();
+    for (u32 i = threadIdx.x; i < ns; i += NM_T) s = nm_op<OP>(s, (&p[i].a)[f]);
+    return nm_bred<OP, NM_T / 32>(s, sh);
 }
 
 // part: [phase 0: ns][phase 1: ns][final: ns][NormRes]
@@ -345,70 +379,29 @@ __global__ void __launch_bounds__(NM_T) k_nm_gpost(int phase, u32 nb, const Norm
     double rho = 0.0, alpha = 0.0, gamma = 0.0;
     bool brk = false;
     if (phase > 0) {
-        const double pw = nm_gsum(p0, ns, 0, sh), rz = nm_gsum(p0, ns, 1, sh);
-        rho = cm.op == OP_CG_FIRST ? rz : cm.rho; alpha = rho / pw;
-        if (!isfinite(alpha)) {
+        const NormPart pr = {nm_gred<RED_SUM>(p0, ns, 0, sh), nm_gred<RED_SUM>(p0, ns, 1, sh), 0.0, 0.0};
+        if (!nm_alpha(cm, pr, rho, alpha)) {
             if (phase == 2 && blockIdx.x == 0 && threadIdx.x == 0) *res = NormRes{rho, 0.0, alpha, ST_FAIL, 0};
             return;
         }
     }
     if (phase == 2) {
-        const double ymin = nm_gext<false>(p1, ns, 0, sh), ymax = nm_gext<true>(p1, ns, 1, sh);
-        const double glo = nm_gext<false>(p1, ns, 2, sh), ghi = nm_gext<false>(p1, ns, 3, sh);
-        brk = ymin <= KR_DELTA || ymax >= KR_DELTA_HI;            // the step leaves the box: stop at its edge, end the inner loop
-        gamma = ymin <= KR_DELTA ? glo : ghi;
+        const NormPart box = {nm_gred<RED_MIN>(p1, ns, 0, sh), nm_gred<RED_MAX>(p1, ns, 1, sh), nm_gred<RED_MIN>(p1, ns, 2, sh),
+                              nm_gred<RED_MIN>(p1, ns, 3, sh)};
+        brk = nm_leaves_box(box.a, box.b);
+        gamma = nm_gamma(box.a, box.c, box.d);
         if (blockIdx.x == 0 && threadIdx.x == 0) *res = NormRes{rho, 0.0, alpha, brk ? ST_CG_BREAK : ST_CG_CONT, 0};
     }
     for (u32 sl = blockIdx.x; sl < ns; sl += gridDim.x) {
         const u32 r0 = sl * NM_GS, r1 = min(nb, r0 + NM_GS);
         NormPart o = {0.0, 0.0, 0.0, 0.0};
-        if (phase == 0 && cm.op == OP_ONES) {                          // row sums: raw total and rows kept by KR
-            double s = 0.0, k = 0.0;
-            for (u32 r = r0 + threadIdx.x; r < r1; r += NM_T) { const double a = V.au[r]; s += a; k += a > 0.0; V.rs[r] = a; V.kept[r] = a > 0.0; }
-            o.a = nm_bsum<NM_T / 32>(s, sh); o.b = nm_bsum<NM_T / 32>(k, sh);
-        } else if (phase == 0 && cm.op == OP_SUMF) {
-            double s = 0.0;
-            for (u32 r = r0 + threadIdx.x; r < r1; r += NM_T) s += V.u[r] * V.au[r];
-            o.a = nm_bsum<NM_T / 32>(s, sh);
-        } else if (phase == 0 && !cg) {                                 // OP_KR_INIT / OP_KR_OUTER: v = x (A x), rk = 1 - v
-            double s = 0.0, xmin = INFINITY; int bad = 0;
-            for (u32 r = r0 + threadIdx.x; r < r1; r += NM_T) {
-                if (!V.kept[r]) continue;
-                const double x = V.x[r], v = x * V.au[r], rk = 1.0 - v;
-                V.v[r] = v; V.rk[r] = rk;
-                s += rk * rk; xmin = fmin(xmin, x); bad |= !isfinite(x) || !isfinite(v);
-            }
-            o.a = nm_bsum<NM_T / 32>(s, sh); o.b = nm_bext<false, NM_T / 32>(xmin, sh); o.c = nm_bsum<NM_T / 32>((double)bad, sh);
-        } else if (phase == 0) {                                        // a CG step on the product A (x p): w, p·w, rk·Z
-            double pw = 0.0, rz = 0.0;
-            for (u32 r = r0 + threadIdx.x; r < r1; r += NM_T) {
-                if (!V.kept[r]) continue;
-                const double p = V.p[r], w = V.x[r] * V.au[r] + V.v[r] * p;
-                V.w[r] = w; pw += p * w; rz += V.rk[r] * V.z[r];
-            }
-            o.a = nm_bsum<NM_T / 32>(pw, sh); o.b = nm_bsum<NM_T / 32>(rz, sh);
-        } else if (phase == 1) {                                        // the box test's extrema
-            double ymin = INFINITY, ymax = -INFINITY, glo = INFINITY, ghi = INFINITY;
-            for (u32 r = r0 + threadIdx.x; r < r1; r += NM_T) {
-                if (!V.kept[r]) continue;
-                const double y = V.y[r], ap = alpha * V.p[r], yn = y + ap;
-                ymin = fmin(ymin, yn); ymax = fmax(ymax, yn);
-                if (ap < 0.0) glo = fmin(glo, (KR_DELTA - y) / ap);
-                if (yn > KR_DELTA_HI) ghi = fmin(ghi, (KR_DELTA_HI - y) / ap);
-            }
-            o.a = nm_bext<false, NM_T / 32>(ymin, sh); o.b = nm_bext<true, NM_T / 32>(ymax, sh);
-            o.c = nm_bext<false, NM_T / 32>(glo, sh); o.d = nm_bext<false, NM_T / 32>(ghi, sh);
-        } else if (brk) {
-            for (u32 r = r0 + threadIdx.x; r < r1; r += NM_T) if (V.kept[r]) V.y[r] = V.y[r] + gamma * (alpha * V.p[r]);
-        } else {                                                        // the update and the new rk·Z
-            double s = 0.0;
-            for (u32 r = r0 + threadIdx.x; r < r1; r += NM_T) {
-                if (!V.kept[r]) continue;
-                const double rk = V.rk[r] - alpha * V.w[r], z = rk / V.v[r];
-                V.y[r] = V.y[r] + alpha * V.p[r]; V.rk[r] = rk; V.z[r] = z; s += rk * z;
-            }
-            o.a = nm_bsum<NM_T / 32>(s, sh);
-        }
+        if (phase == 0 && cm.op == OP_ONES) o = nm_row_sums<NM_T>(V, r0, r1, sh);
+        else if (phase == 0 && cm.op == OP_SUMF) o.a = nm_sumf<NM_T>(V, r0, r1, sh);
+        else if (phase == 0 && !cg) o = nm_outer<NM_T>(V, r0, r1, sh);
+        else if (phase == 0) o = nm_cg_product<NM_T>(V, r0, r1, sh);
+        else if (phase == 1) o = nm_box<NM_T>(V, r0, r1, alpha, sh);
+        else if (brk) nm_edge<NM_T>(V, r0, r1, gamma, alpha);
+        else o.a = nm_cg_update<NM_T>(V, r0, r1, alpha, sh);
         if (threadIdx.x == 0) (phase == 0 && cg ? p0 : phase == 1 ? p1 : pf)[sl] = o;
     }
 }
