@@ -318,6 +318,40 @@ uint64_t mk_norm_launch_count(mk_norm *);
 int  mk_norm_enable_timing(mk_norm *, int on);
 int  mk_norm_kernel_times(mk_norm *, double *ms, uint64_t *count);
 
+/* ------------------------------------------------------------------ BGZF inflate (bgzipped .pairs, BAM) */
+/* BGZF (SAMv1 §4.1) is a chain of gzip members, each an independent raw-deflate stream of at most 64 KiB of output whose
+ * header gives its compressed size (BSIZE) and whose trailer gives its CRC-32 and output size (ISIZE): mk_bgzf_scan finds
+ * the members on the host, mk_bgzf_inflate_device inflates them side by side in HBM (one warp per member). */
+typedef struct {
+    uint64_t in_off;    /* the member's first byte in the compressed buffer */
+    uint64_t out_off;   /* where its output goes in the output buffer: the running sum of ISIZE */
+    uint32_t in_len;    /* BSIZE + 1: header, deflate data and trailer */
+    uint32_t isize;     /* output bytes (<= 65536) */
+} mk_bgzf_member;
+/* Walks the member headers at the start of buf (host memory): one entry per WHOLE member, at most cap of them.  Stops at the
+ * first incomplete member (or the end of buf, or cap); *n_bytes = bytes the whole members take (may be NULL), *n_out = sum of
+ * their ISIZE (may be NULL).  A member that is not BGZF (1f 8b 08 with FLG.FEXTRA, a BC subfield with SLEN 2 among any others,
+ * BSIZE covering header and trailer, ISIZE <= 65536) is refused with MK_ERR_INPUT and a message naming its byte offset;
+ * plain gzip (no BC subfield) is refused so. */
+int  mk_bgzf_scan(const void *buf, size_t n, mk_bgzf_member *members, size_t cap, size_t *n_members, size_t *n_bytes, uint64_t *n_out);
+/* A reusable device object for calls of up to max_members members (member table and error word; no allocation per call). */
+typedef struct mk_bgzf mk_bgzf;
+int  mk_bgzf_create(int device, size_t max_members, mk_bgzf **);
+void mk_bgzf_destroy(mk_bgzf *);
+/* Inflates members[0..n) (host array, as mk_bgzf_scan returns them) of the compressed bytes at d_in (device) to
+ * d_out + out_off (device); checks every member's CRC-32 and ISIZE on the device, and returns when the output is complete.
+ * Any input bytes are safe: no read outside a member's in_len bytes, no write outside [out_off, out_off + isize).
+ * Damaged members (bad block type, code set or symbol, a distance before the member's start, output past or short of
+ * ISIZE, a stream that does not end right before the trailer, a CRC or ISIZE mismatch) give MK_ERR_INPUT naming the first
+ * failing member in file order and the reason.  Refused before any launch (MK_ERR_ARG): out_cap below the sum of ISIZE,
+ * a member whose output leaves [0, out_cap) or whose sizes break the format's limits; n > max_members (MK_ERR_CAPACITY).
+ * Byte-identical to zlib on every member zlib accepts; no floating point, no atomics on the output. */
+int  mk_bgzf_inflate_device(mk_bgzf *, const void *d_in, const mk_bgzf_member *members, size_t n, void *d_out, size_t out_cap, void *stream);
+/* What the last successful call wrote, for text consumers: the number of '\n' bytes, and the offset from d_out of the last
+ * one (-1 when there is none). */
+int  mk_bgzf_text_stats(mk_bgzf *, uint64_t *newlines, int64_t *last_newline);
+uint64_t mk_bgzf_launch_count(mk_bgzf *);
+
 /* ------------------------------------------------------------------ multi-GPU exchange over NVLink peer memory */
 /* One object per rank (one process per GPU, or several ranks in one process).  Owner bucketing and the all-to-all are ONE
  * kernel: owner = mix(chr1, chr2, pos1 / res) mod world (mk_pairs_owner); every rank writes its pairs straight into the

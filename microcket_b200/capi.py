@@ -62,6 +62,10 @@ NORM_TYPES = {"VC": 1, "VC_SQRT": 2, "KR": 4}
 NORM_SCOPES = {"GW": 1, "INTER": 2}
 
 
+class BgzfMember(C.Structure):
+    _fields_ = [("in_off", C.c_uint64), ("out_off", C.c_uint64), ("in_len", C.c_uint32), ("isize", C.c_uint32)]
+
+
 class DedupCfg(C.Structure):
     _fields_ = [("hskip1", C.c_int), ("klen1", C.c_int), ("hskip2", C.c_int), ("klen2", C.c_int), ("device", C.c_int),
                 ("window_bytes", C.c_size_t), ("async_pull", C.c_int)]
@@ -158,7 +162,10 @@ class Lib:
                            ("mk_norm_device", [vp, vp, vp, vp, sz, i, vp, vp, vp, P(C.c_uint8), P(NormStats), vp]),
                            ("mk_norm_genome_device", [vp, vp, vp, vp, sz, i, i, vp, vp, P(C.c_uint8), P(NormStats), vp]),
                            ("mk_norm_launch_count", [vp]), ("mk_norm_enable_timing", [vp, i]),
-                           ("mk_norm_kernel_times", [vp, P(C.c_double), P(u64)])):
+                           ("mk_norm_kernel_times", [vp, P(C.c_double), P(u64)]),
+                           ("mk_bgzf_scan", [vp, sz, P(BgzfMember), sz, P(sz), P(sz), P(u64)]), ("mk_bgzf_create", [i, sz, P(vp)]),
+                           ("mk_bgzf_destroy", [vp]), ("mk_bgzf_inflate_device", [vp, vp, P(BgzfMember), sz, vp, sz, vp]),
+                           ("mk_bgzf_text_stats", [vp, P(u64), P(C.c_int64)]), ("mk_bgzf_launch_count", [vp])):
             if hasattr(L, name):
                 getattr(L, name).argtypes = args
         if hasattr(L, "mk_pairs_owner"):
@@ -168,7 +175,7 @@ class Lib:
             L.mk_pairs_launch_count.restype = u64
         if hasattr(L, "mk_pairs_dropped"):
             L.mk_pairs_dropped.restype = u64
-        for name in ("mk_hist_dropped", "mk_hist_launch_count", "mk_xchg_launch_count", "mk_norm_launch_count"):
+        for name in ("mk_hist_dropped", "mk_hist_launch_count", "mk_xchg_launch_count", "mk_norm_launch_count", "mk_bgzf_launch_count"):
             if hasattr(L, name):
                 getattr(L, name).restype = u64
 
@@ -626,6 +633,68 @@ class Norm:
             self.close()
         except Exception:
             pass
+
+
+def bgzf_scan(data, cap=None):
+    """BGZF member walk over host bytes (mk_bgzf_scan) -> (members: BgzfMember array, bytes the whole members take, output bytes)"""
+    cap = len(data) // 20 + 1 if cap is None else cap
+    arr = (BgzfMember * max(cap, 1))()
+    n, nb, no = C.c_size_t(), C.c_size_t(), C.c_uint64()
+    L = lib()
+    L.check(L.L.mk_bgzf_scan(data, len(data), arr, cap, C.byref(n), C.byref(nb), C.byref(no)))
+    return (BgzfMember * n.value).from_buffer_copy(arr) if n.value else (BgzfMember * 0)(), nb.value, no.value
+
+
+class Bgzf:
+    """Inflate of BGZF members in HBM (csrc/bgzf.cu): one reusable object for calls of up to max_members members."""
+
+    def __init__(self, max_members, device=0):
+        self.lib = lib()
+        self.lib.require_gpu()
+        self.h = C.c_void_p()
+        self.lib.check(self.lib.L.mk_bgzf_create(device, max_members, C.byref(self.h)))
+
+    def inflate(self, d_in, members, d_out, out_cap, stream=0):
+        """members (BgzfMember array or list, e.g. from bgzf_scan) of the compressed bytes at device pointer d_in -> d_out"""
+        if not isinstance(members, C.Array):
+            members = (BgzfMember * len(members))(*members)
+        self.lib.check(self.lib.L.mk_bgzf_inflate_device(self.h, d_in, members, len(members), d_out, out_cap, stream))
+
+    def text_stats(self):
+        """-> (newline bytes the last call wrote, offset of the last one from d_out or -1)"""
+        nl, last = C.c_uint64(), C.c_int64()
+        self.lib.check(self.lib.L.mk_bgzf_text_stats(self.h, C.byref(nl), C.byref(last)))
+        return nl.value, last.value
+
+    def launches(self):
+        return self.lib.L.mk_bgzf_launch_count(self.h)
+
+    def close(self):
+        if self.h:
+            self.lib.L.mk_bgzf_destroy(self.h)
+            self.h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def bgzf_decompress(data, device=0):
+    """bytes of whole BGZF members -> their inflated bytes, through the GPU (torch tensors in and out)"""
+    import torch
+    mem, nb, n_out = bgzf_scan(data)
+    if nb != len(data):
+        raise MkError(f"BGZF input: {len(data) - nb} bytes after the last whole member (a truncated member)")
+    d_in = torch.frombuffer(bytearray(data) or bytearray(1), dtype=torch.uint8).to(f"cuda:{device}")
+    d_out = torch.empty(max(n_out, 1), dtype=torch.uint8, device=f"cuda:{device}")
+    bz = Bgzf(max(len(mem), 1), device)
+    try:
+        bz.inflate(d_in.data_ptr(), mem, d_out.data_ptr(), n_out)
+    finally:
+        bz.close()
+    return d_out[:n_out].cpu().numpy().tobytes()
 
 
 class Xchg:

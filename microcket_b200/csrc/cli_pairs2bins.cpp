@@ -1,12 +1,14 @@
 // cli_pairs2bins.cpp — contact binning of a .pairs file on the GPU (new tool; stands where the driver calls
 // `java -jar juicer_tools.jar pre -r <res,...> <sid>.final.pairs <sid>.hic <genome>.info`, microcket:525-529).
-//   pairs2bins [-d] [-b] [-H <out.hic>] [-g <genomeId>] -r <res[,res...]> <in.pairs|-> <out.prefix> <genome.info>
+//   pairs2bins [-d] [-b] [-H <out.hic>] [-g <genomeId>] -r <res[,res...]> <in.pairs|in.pairs.gz|-> <out.prefix> <genome.info>
 // Writes <out.prefix>.<res>.coo with `bin1<TAB>bin2<TAB>count` (upper triangle, sorted), bins numbered in .info order with
 // bin = offset[chr] + pos / res.  -d removes coordinate duplicates first (first occurrence wins).
 // -b also writes <out.prefix>.<res>.bins.bed (`chrom<TAB>start<TAB>end`, one line per bin id): the pair of files is what
 // `cooler load -f coo <bins.bed> <coo> out.cool` takes, i.e. the hand-over point to the .cool branch of the driver
 // (microcket:531-551) without `cooler cload pairs` re-reading and re-binning the pairs.
-// The file is streamed in 256 MiB chunks from pinned memory and PARSED ON THE GPU (mk_pairs_parse_text_device); resolutions
+// The file is streamed in 256 MiB chunks from pinned memory and PARSED ON THE GPU (mk_pairs_parse_text_device).  A bgzipped
+// file or stream (BGZF, the 4DN .pairs.gz) is INFLATED ON THE GPU into the same chunks (mk_bgzf_*, bgzf.cu); gzip that is not
+// BGZF is refused (one deflate stream cannot be split: `zcat x.pairs.gz | pairs2bins ... -` reads it).  Resolutions
 // whose upper triangle fits MICROCKET_DENSE_MB (default 4096) all come from one pass of the dense histogram (mk_hist_*), the
 // finer ones from the sort path.
 // -H <out.hic> also packs every resolution's counts into one `.hic` (version 8) container, i.e. the file the driver's
@@ -20,6 +22,7 @@
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
+#include <algorithm>
 #include <cstring>
 #include <fstream>
 #include <iostream>
@@ -112,6 +115,126 @@ static int write_coo(const string &prefix, uint32_t res, const void *d_b1, const
     return 0;
 }
 
+// the pair array holds at least `need` pairs: grown by doubling, with a device-to-device copy of the n there
+static int reserve(void **d_pairs, size_t *cap, size_t n, size_t need) {
+    if (need <= *cap) return 0;
+    size_t ncap = *cap; while (ncap < need) ncap *= 2;
+    void *bigger = NULL;
+    CHECK(mk_dev_alloc(g_dev, ncap * sizeof(mk_pair), &bigger));
+    if (n) CHECK(mk_copy_device(bigger, *d_pairs, n * sizeof(mk_pair)));
+    mk_dev_free(*d_pairs); *d_pairs = bigger; *cap = ncap;
+    return 0;
+}
+
+// Plain text: read in CHUNK-byte pieces into pinned memory, cut at the last '\n', parsed on the GPU.  pre: bytes already
+// taken from the stream to look for a gzip member (at most two, when the first is 0x1f).
+static int read_text(FILE *fp, const char *pre, size_t npre, const vector<const char *> &cnames, size_t CHUNK, void **d_pairs_out, size_t *n_out, size_t *skipped_out) {
+    const int dev = g_dev;
+    size_t cap = 1u << 22;                                               // pairs capacity, grown as the file goes by
+    void *d_pairs = NULL, *d_text = NULL; char *h_text = NULL;
+    CHECK(mk_dev_alloc(dev, cap * sizeof(mk_pair), &d_pairs));
+    CHECK(mk_dev_alloc(dev, CHUNK + 64, &d_text));
+    CHECK(mk_host_alloc(CHUNK + 64, (void **)&h_text));
+    mk_pairs_ws *pws = NULL;                                             // parser workspace (sized per chunk: a line is >= 14 bytes)
+    const size_t chunk_lines = CHUNK / 14 + 16;
+    CHECK(mk_pairs_ws_create(dev, chunk_lines, &pws));
+    size_t n = 0, have = npre, skipped = 0;
+    memcpy(h_text, pre, npre);
+    while (true) {
+        const size_t got = fread(h_text + have, 1, CHUNK - have, fp);
+        const bool eof = got == 0;
+        size_t tot = have + got;
+        if (tot == 0) break;
+        size_t cut = tot;
+        if (!eof) { while (cut > 0 && h_text[cut - 1] != '\n') --cut; if (cut == 0) { if (tot == CHUNK) { cerr << "Error: a line longer than " << CHUNK << " bytes\n"; return 10; } have = tot; continue; } }
+        else if (h_text[tot - 1] != '\n') { h_text[tot++] = '\n'; cut = tot; }   // last line without a newline
+        size_t lines_max = 0; for (size_t i = 0; i < cut; ++i) lines_max += h_text[i] == '\n';
+        if (int rc = reserve(&d_pairs, &cap, n, n + lines_max)) return rc;
+        CHECK(mk_copy_to_device(d_text, h_text, cut));
+        size_t nl = 0, ns = 0;
+        CHECK(mk_pairs_parse_text_device(pws, (const char *)d_text, cut, cnames.data(), (int)cnames.size(), (mk_pair *)d_pairs + n, cap - n, &nl, &ns, NULL));
+        n += nl; skipped += ns;
+        have = tot - cut;
+        if (have) memmove(h_text, h_text + cut, have);
+        if (eof) break;
+    }
+    mk_pairs_ws_destroy(pws); mk_dev_free(d_text); mk_host_free(h_text);
+    *d_pairs_out = d_pairs; *n_out = n; *skipped_out = skipped;
+    return 0;
+}
+
+// BGZF (bgzip's .pairs.gz; concatenated files and EOF members anywhere): whole members are read into pinned memory, copied to
+// the device and inflated there (mk_bgzf_inflate_device) right behind the partial line carried from the previous chunk, as
+// many as keep the text within CHUNK.  The text up to its last '\n' is parsed like a plain chunk, and the rest moves to the
+// front of the other text buffer.  The host never sees the text: the inflate's newline count bounds the parser's output.
+// The leading 1f 8b are already taken from the stream.  A damaged or truncated member, or gzip that is not BGZF, exits 10.
+static int bgzf_fail(const char *name, uint64_t at, const char *why) {
+    cerr << "Error: " << name << ": BGZF input, compressed bytes from " << at << " on: " << why;
+    if (strstr(why, "not BGZF")) cerr << "; a single gzip stream cannot be inflated in parallel: decompress it first, `zcat " << name << " | pairs2bins ... -`";
+    cerr << "\n";
+    return 10;
+}
+static int read_bgzf(FILE *fp, const char *name, const vector<const char *> &cnames, size_t CHUNK, void **d_pairs_out, size_t *n_out, size_t *skipped_out) {
+    const size_t CIN = max<size_t>(CHUNK, 1 << 20), TEXT = CHUNK + 65536 + 64, MAXM = 65536;   // CIN holds any whole member
+    size_t cap = 1u << 22;
+    void *d_pairs = NULL, *d_text[2] = {NULL, NULL}, *d_in = NULL; uint8_t *h_in = NULL;
+    CHECK(mk_dev_alloc(g_dev, cap * sizeof(mk_pair), &d_pairs));
+    CHECK(mk_dev_alloc(g_dev, TEXT, &d_text[0])); CHECK(mk_dev_alloc(g_dev, TEXT, &d_text[1]));
+    CHECK(mk_dev_alloc(g_dev, CIN, &d_in));
+    CHECK(mk_host_alloc(CIN, (void **)&h_in));
+    mk_pairs_ws *pws = NULL;
+    CHECK(mk_pairs_ws_create(g_dev, CHUNK / 14 + 16, &pws));
+    mk_bgzf *bz = NULL;
+    CHECK(mk_bgzf_create(g_dev, MAXM, &bz));
+    vector<mk_bgzf_member> mem(MAXM);
+    h_in[0] = 0x1f; h_in[1] = 0x8b;
+    size_t have = 2, carry = 0, n = 0, skipped = 0; uint64_t at = 0;   // at: file offset of h_in[0]
+    bool in_eof = false; int cur = 0;
+    while (true) {
+        if (!in_eof) { const size_t got = fread(h_in + have, 1, CIN - have, fp); in_eof = got < CIN - have; have += got; }
+        size_t nm = 0, nb = 0;
+        if (mk_bgzf_scan(h_in, have, mem.data(), MAXM, &nm, &nb, NULL) != MK_OK) return bgzf_fail(name, at, mk_last_error());
+        if (nm == 0 && have) return bgzf_fail(name, at, "a truncated member at the end of the input");
+        if (nm && carry >= CHUNK) { cerr << "Error: a line longer than " << CHUNK << " bytes\n"; return 10; }
+        size_t k = 0, out = 0;                                          // the first member always fits: TEXT has 64 KiB to spare
+        while (k < nm && (k == 0 || carry + out + mem[k].isize <= CHUNK)) out += mem[k++].isize;
+        const size_t cb = k ? mem[k - 1].in_off + mem[k - 1].in_len : 0;
+        uint64_t nl = 0; int64_t last = -1;
+        if (k) {
+            CHECK(mk_copy_to_device(d_in, h_in, cb));
+            const int rc = mk_bgzf_inflate_device(bz, d_in, mem.data(), k, (char *)d_text[cur] + carry, TEXT - carry, NULL);
+            if (rc == MK_ERR_INPUT) return bgzf_fail(name, at, mk_last_error());
+            CHECK(rc);
+            CHECK(mk_bgzf_text_stats(bz, &nl, &last));
+        }
+        at += cb; have -= cb;
+        if (have) memmove(h_in, h_in + cb, have);
+        const bool end = in_eof && have == 0;
+        size_t tot = carry + out, cut = last >= 0 ? carry + (size_t)last + 1 : 0;
+        if (end && tot > cut) {                                         // last line without a newline
+            CHECK(mk_copy_to_device((char *)d_text[cur] + tot, "\n", 1));
+            cut = ++tot; ++nl;
+        }
+        if (cut == 0) {
+            if (tot >= CHUNK) { cerr << "Error: a line longer than " << CHUNK << " bytes\n"; return 10; }
+            carry = tot;
+            if (end) break;
+            continue;
+        }
+        if (int rc = reserve(&d_pairs, &cap, n, n + nl)) return rc;
+        size_t lines = 0, ns = 0;
+        CHECK(mk_pairs_parse_text_device(pws, (const char *)d_text[cur], cut, cnames.data(), (int)cnames.size(), (mk_pair *)d_pairs + n, cap - n, &lines, &ns, NULL));
+        n += lines; skipped += ns;
+        carry = tot - cut;                                              // the partial line moves to the other buffer's front
+        if (carry) CHECK(mk_copy_device(d_text[cur ^ 1], (char *)d_text[cur] + cut, carry));
+        cur ^= 1;
+        if (end) break;
+    }
+    mk_bgzf_destroy(bz); mk_pairs_ws_destroy(pws); mk_dev_free(d_text[0]); mk_dev_free(d_text[1]); mk_dev_free(d_in); mk_host_free(h_in);
+    *d_pairs_out = d_pairs; *n_out = n; *skipped_out = skipped;
+    return 0;
+}
+
 int main(int argc, char *argv[]) {
     bool dedup = false, bins_bed = false; string reslist, hic_path, genome, normlist;
     int a = 1;
@@ -137,7 +260,8 @@ int main(int argc, char *argv[]) {
         }
     }
     if (argc - a < 3 || reslist.empty() || (!normlist.empty() && hic_path.empty())) {
-        cerr << "\nUsage: " << argv[0] << " [-d] [-b] [-H <out.hic> [-n VC,VC_SQRT,KR,GW_VC,GW_KR,INTER_VC,INTER_KR]] [-g <genomeId>] -r <res[,res...]> <in.pairs|-> <out.prefix> <genome.info>\n\n";
+        cerr << "\nUsage: " << argv[0] << " [-d] [-b] [-H <out.hic> [-n VC,VC_SQRT,KR,GW_VC,GW_KR,INTER_VC,INTER_KR]] [-g <genomeId>] -r <res[,res...]> <in.pairs|in.pairs.gz|-> <out.prefix> <genome.info>\n"
+                "  the input may be plain text or bgzipped (BGZF: bgzip, the 4DN .pairs.gz), from a file or from stdin\n\n";
         return 2;
     }
     vector<uint32_t> res;
@@ -173,43 +297,17 @@ int main(int argc, char *argv[]) {
     g_dev = dev; g_len = chr_len; g_names = names;
     if (mk_device_count() < 1) { cerr << "Error: no CUDA device: microcket_b200 has no CPU fallback\n"; return 20; }
 
-    // ---- stream the text to the GPU and parse it there
+    // ---- stream the text to the GPU and parse it there; a file that starts with a gzip member (1f 8b) is read as BGZF
+    size_t n = 0, skipped = 0; void *d_pairs = NULL;
+    const int c0 = getc(fp), c1 = c0 == 0x1f ? getc(fp) : EOF;
     const size_t CHUNK = (size_t)(getenv("MICROCKET_CHUNK_MB") ? atol(getenv("MICROCKET_CHUNK_MB")) : 256) << 20;
-    size_t cap = 1u << 22;                                               // pairs capacity, grown as the file goes by
-    void *d_pairs = NULL, *d_text = NULL; char *h_text = NULL;
-    CHECK(mk_dev_alloc(dev, cap * sizeof(mk_pair), &d_pairs));
-    CHECK(mk_dev_alloc(dev, CHUNK + 64, &d_text));
-    CHECK(mk_host_alloc(CHUNK + 64, (void **)&h_text));
-    mk_pairs_ws *pws = NULL;                                             // parser workspace (sized per chunk: a line is >= 14 bytes)
-    const size_t chunk_lines = CHUNK / 14 + 16;
-    CHECK(mk_pairs_ws_create(dev, chunk_lines, &pws));
-    size_t n = 0, have = 0, skipped = 0;
-    while (true) {
-        const size_t got = fread(h_text + have, 1, CHUNK - have, fp);
-        const bool eof = got == 0;
-        size_t tot = have + got;
-        if (tot == 0) break;
-        size_t cut = tot;
-        if (!eof) { while (cut > 0 && h_text[cut - 1] != '\n') --cut; if (cut == 0) { if (tot == CHUNK) { cerr << "Error: a line longer than " << CHUNK << " bytes\n"; return 10; } have = tot; continue; } }
-        else if (h_text[tot - 1] != '\n') { h_text[tot++] = '\n'; cut = tot; }   // last line without a newline
-        size_t lines_max = 0; for (size_t i = 0; i < cut; ++i) lines_max += h_text[i] == '\n';
-        if (n + lines_max > cap) {                                       // grow the pair array (device-to-device copy of what is there)
-            size_t ncap = cap; while (ncap < n + lines_max) ncap *= 2;
-            void *bigger = NULL;
-            CHECK(mk_dev_alloc(dev, ncap * sizeof(mk_pair), &bigger));
-            if (n) CHECK(mk_copy_device(bigger, d_pairs, n * sizeof(mk_pair)));
-            mk_dev_free(d_pairs); d_pairs = bigger; cap = ncap;
-        }
-        CHECK(mk_copy_to_device(d_text, h_text, cut));
-        size_t nl = 0, ns = 0;
-        CHECK(mk_pairs_parse_text_device(pws, (const char *)d_text, cut, cnames.data(), (int)cnames.size(), (mk_pair *)d_pairs + n, cap - n, &nl, &ns, NULL));
-        n += nl; skipped += ns;
-        have = tot - cut;
-        if (have) memmove(h_text, h_text + cut, have);
-        if (eof) break;
+    if (c0 == 0x1f && c1 == 0x8b) { if (int rc = read_bgzf(fp, argv[a], cnames, CHUNK, &d_pairs, &n, &skipped)) return rc; }
+    else {
+        const char pre[2] = {(char)c0, (char)c1};
+        if (c0 != 0x1f && c0 != EOF) ungetc(c0, fp);
+        if (int rc = read_text(fp, pre, c0 != 0x1f ? 0 : c1 == EOF ? 1 : 2, cnames, CHUNK, &d_pairs, &n, &skipped)) return rc;
     }
     if (fp != stdin) fclose(fp);
-    mk_pairs_ws_destroy(pws); mk_dev_free(d_text); mk_host_free(h_text);
 
     // ---- bins
     mk_pairs_ws *ws = NULL;
