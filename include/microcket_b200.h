@@ -352,6 +352,29 @@ int  mk_bgzf_inflate_device(mk_bgzf *, const void *d_in, const mk_bgzf_member *m
 int  mk_bgzf_text_stats(mk_bgzf *, uint64_t *newlines, int64_t *last_newline);
 uint64_t mk_bgzf_launch_count(mk_bgzf *);
 
+/* ------------------------------------------------------------------ BGZF deflate (bgzip, .pairs.gz output) */
+/* The other direction: input bytes in HBM -> BGZF members in HBM, one CTA per member.  Member k holds input bytes
+ * [k * 65280, min(n, (k + 1) * 65280)), the cut bgzip makes, and bgzip's header bytes (XLEN 6, one BC subfield).  Levels 1-9
+ * (and -1, the default) all write the same bytes: a greedy parse with one match candidate per position and per-member
+ * Huffman codes, the smallest of a stored, fixed or dynamic block.  Level 0 writes stored members only.  The bytes depend
+ * only on the input and on "level 0 or not": not on the card, the grid, the stream, the input address, or on where a
+ * caller cuts its input into calls, as long as the cuts fall on multiples of 65280.  They are this project's own (not
+ * htslib's bgzip bytes); zlib, gzip, htslib and mk_bgzf_inflate_device read them back. */
+/* Worst-case output bytes for n input bytes (every member stored: n + 31 per member); no EOF member. */
+size_t mk_bgzf_deflate_bound(size_t n);
+/* A reusable device object for calls of up to max_bytes input bytes (staging, member sizes, scratch; no allocation per call). */
+typedef struct mk_bgzf_enc mk_bgzf_enc;
+int  mk_bgzf_enc_create(int device, size_t max_bytes, mk_bgzf_enc **);
+void mk_bgzf_enc_destroy(mk_bgzf_enc *);
+/* Compresses n bytes at d_in (device) into members written back to back at d_out (device); returns when they are complete.
+ * *out_len: their bytes; *n_members: their number; members (host, may be NULL): the table mk_bgzf_scan returns on the output.
+ * No EOF member is written: the caller appends it (28 bytes, 1f 8b 08 04 00 00 00 00 00 ff 06 00 42 43 02 00 1b 00 03 00 then
+ * eight zeros).  Refused before any launch: a null object, pointer or count pointer, level outside -1..9, out_cap below
+ * mk_bgzf_deflate_bound(n), a members table smaller than the member count (MK_ERR_ARG); n > max_bytes (MK_ERR_CAPACITY). */
+int  mk_bgzf_deflate_device(mk_bgzf_enc *, const void *d_in, size_t n, int level, void *d_out, size_t out_cap, size_t *out_len,
+                            mk_bgzf_member *members, size_t members_cap, size_t *n_members, void *stream);
+uint64_t mk_bgzf_enc_launch_count(mk_bgzf_enc *);
+
 /* ------------------------------------------------------------------ multi-GPU exchange over NVLink peer memory */
 /* One object per rank (one process per GPU, or several ranks in one process).  Owner bucketing and the all-to-all are ONE
  * kernel: owner = mix(chr1, chr2, pos1 / res) mod world (mk_pairs_owner); every rank writes its pairs straight into the

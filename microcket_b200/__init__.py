@@ -7,6 +7,6 @@ every compute call raises if the CUDA library or a GPU is missing.
 """
 from .capi import (MkError, Lib, lib, build, S2PConfig, Sam2Pairs, Krmdup, PairsWorkspace, synth_host,  # noqa: F401
                    synth_device, synth_opts, SynthOpts, chrom_ranks, Hist, Norm, NormStats, NORM_TYPES, NORM_SCOPES, Xchg, LIB_PATH, PAIR_DTYPE,
-                   Bgzf, BgzfMember, bgzf_scan, bgzf_decompress)
+                   Bgzf, BgzfMember, bgzf_scan, bgzf_decompress, BgzfDeflate, bgzf_compress, bgzf_deflate_bound, BGZF_EOF)
 
-__all__ = ["MkError", "Lib", "lib", "build", "S2PConfig", "Sam2Pairs", "Krmdup", "PairsWorkspace", "synth_host", "synth_device", "synth_opts", "SynthOpts", "chrom_ranks", "Hist", "Norm", "NormStats", "NORM_TYPES", "NORM_SCOPES", "Xchg", "LIB_PATH", "PAIR_DTYPE", "Bgzf", "BgzfMember", "bgzf_scan", "bgzf_decompress"]
+__all__ = ["MkError", "Lib", "lib", "build", "S2PConfig", "Sam2Pairs", "Krmdup", "PairsWorkspace", "synth_host", "synth_device", "synth_opts", "SynthOpts", "chrom_ranks", "Hist", "Norm", "NormStats", "NORM_TYPES", "NORM_SCOPES", "Xchg", "LIB_PATH", "PAIR_DTYPE", "Bgzf", "BgzfMember", "bgzf_scan", "bgzf_decompress", "BgzfDeflate", "bgzf_compress", "bgzf_deflate_bound", "BGZF_EOF"]

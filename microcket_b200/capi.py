@@ -165,7 +165,10 @@ class Lib:
                            ("mk_norm_kernel_times", [vp, P(C.c_double), P(u64)]),
                            ("mk_bgzf_scan", [vp, sz, P(BgzfMember), sz, P(sz), P(sz), P(u64)]), ("mk_bgzf_create", [i, sz, P(vp)]),
                            ("mk_bgzf_destroy", [vp]), ("mk_bgzf_inflate_device", [vp, vp, P(BgzfMember), sz, vp, sz, vp]),
-                           ("mk_bgzf_text_stats", [vp, P(u64), P(C.c_int64)]), ("mk_bgzf_launch_count", [vp])):
+                           ("mk_bgzf_text_stats", [vp, P(u64), P(C.c_int64)]), ("mk_bgzf_launch_count", [vp]),
+                           ("mk_bgzf_deflate_bound", [sz]), ("mk_bgzf_enc_create", [i, sz, P(vp)]), ("mk_bgzf_enc_destroy", [vp]),
+                           ("mk_bgzf_deflate_device", [vp, vp, sz, i, vp, sz, P(sz), P(BgzfMember), sz, P(sz), vp]),
+                           ("mk_bgzf_enc_launch_count", [vp])):
             if hasattr(L, name):
                 getattr(L, name).argtypes = args
         if hasattr(L, "mk_pairs_owner"):
@@ -175,9 +178,12 @@ class Lib:
             L.mk_pairs_launch_count.restype = u64
         if hasattr(L, "mk_pairs_dropped"):
             L.mk_pairs_dropped.restype = u64
-        for name in ("mk_hist_dropped", "mk_hist_launch_count", "mk_xchg_launch_count", "mk_norm_launch_count", "mk_bgzf_launch_count"):
+        for name in ("mk_hist_dropped", "mk_hist_launch_count", "mk_xchg_launch_count", "mk_norm_launch_count", "mk_bgzf_launch_count",
+                     "mk_bgzf_enc_launch_count"):
             if hasattr(L, name):
                 getattr(L, name).restype = u64
+        if hasattr(L, "mk_bgzf_deflate_bound"):
+            L.mk_bgzf_deflate_bound.restype = sz
 
     def check(self, rc):
         if rc != 0:
@@ -695,6 +701,61 @@ def bgzf_decompress(data, device=0):
     finally:
         bz.close()
     return d_out[:n_out].cpu().numpy().tobytes()
+
+
+BGZF_EOF = bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000")   # bgzip's end-of-file member
+
+
+def bgzf_deflate_bound(n):
+    """worst-case bytes of the members mk_bgzf_deflate_device writes for n input bytes (no EOF member)"""
+    return lib().L.mk_bgzf_deflate_bound(n)
+
+
+class BgzfDeflate:
+    """BGZF members written in HBM (csrc/bgzf_deflate.cu): one reusable object for calls of up to max_bytes input bytes."""
+
+    def __init__(self, max_bytes, device=0):
+        self.lib = lib()
+        self.lib.require_gpu()
+        self.h = C.c_void_p()
+        self.lib.check(self.lib.L.mk_bgzf_enc_create(device, max_bytes, C.byref(self.h)))
+
+    def deflate(self, d_in, n, d_out, out_cap, level=-1, stream=0):
+        """n bytes at device pointer d_in -> members back to back at d_out; -> (bytes written, BgzfMember table of the output)"""
+        nm = -(-n // 65280)
+        arr = (BgzfMember * max(nm, 1))()
+        out_len, got = C.c_size_t(), C.c_size_t()
+        self.lib.check(self.lib.L.mk_bgzf_deflate_device(self.h, d_in, n, level, d_out, out_cap, C.byref(out_len), arr, nm,
+                                                         C.byref(got), stream))
+        return out_len.value, (BgzfMember * got.value).from_buffer_copy(arr) if got.value else (BgzfMember * 0)()
+
+    def launches(self):
+        return self.lib.L.mk_bgzf_enc_launch_count(self.h)
+
+    def close(self):
+        if self.h:
+            self.lib.L.mk_bgzf_enc_destroy(self.h)
+            self.h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def bgzf_compress(data, level=-1, eof=True, device=0):
+    """bytes -> BGZF bytes compressed on the GPU (bgzip's member cut), with bgzip's EOF member unless eof=False"""
+    import torch
+    d_in = torch.frombuffer(bytearray(data) or bytearray(1), dtype=torch.uint8).to(f"cuda:{device}")
+    cap = bgzf_deflate_bound(len(data))
+    d_out = torch.empty(max(cap, 1), dtype=torch.uint8, device=f"cuda:{device}")
+    bd = BgzfDeflate(max(len(data), 1), device)
+    try:
+        n, _ = bd.deflate(d_in.data_ptr(), len(data), d_out.data_ptr(), cap, level)
+    finally:
+        bd.close()
+    return d_out[:n].cpu().numpy().tobytes() + (BGZF_EOF if eof else b"")
 
 
 class Xchg:
