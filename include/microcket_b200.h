@@ -375,6 +375,47 @@ int  mk_bgzf_deflate_device(mk_bgzf_enc *, const void *d_in, size_t n, int level
                             mk_bgzf_member *members, size_t members_cap, size_t *n_members, void *stream);
 uint64_t mk_bgzf_enc_launch_count(mk_bgzf_enc *);
 
+/* ------------------------------------------------------------------ coordinate-sorted BAM (sam2bam, valid.bam) */
+/* SAM text in HBM -> BAM records (SAMv1 §4.2) -> coordinate order -> the .bai index (SAMv1 §5.2).  One object holds the
+ * reference dictionary (the @SQ SN / LN pairs, in order) and the workspace; compression is mk_bgzf_deflate_device.
+ * Records are those of tests/bam_writer.encode_records, except that a flag-4 record with a CIGAR has bin = reg2bin(pos, pos+1).
+ * Offsets: a record array is a device pointer d_rec to record 0 and d_off[0..n] (n + 1 values, any base): record i is at
+ * d_rec + d_off[i] - d_off[0] and has d_off[i + 1] - d_off[i] bytes.  Text chunks stay below 4 GiB, sorts below 2^30 records. */
+typedef struct mk_bam mk_bam;
+int  mk_bam_create(int device, const char *const *ref_names, const uint32_t *ref_len, int n_refs, size_t max_text, size_t max_records, mk_bam **);
+void mk_bam_destroy(mk_bam *);
+/* Step 1 of the encode: the line index of n bytes of SAM records at d_text (whole lines, the last one ending with '\n', no
+ * header lines) and every line's record size.  *n_lines, *rec_bytes: the records and their bytes.  A refused line gives
+ * MK_ERR_INPUT with *bad_line (0-based, within the call) and *bad_code (the lowest bad line, whatever the thread order):
+ * 1 fewer than 11 fields, 2 QNAME, 3 FLAG, 4 RNAME not in the dictionary, 5 POS, 6 MAPQ, 7 CIGAR, 8 more than 65535 CIGAR
+ * ops, 9 RNEXT, 10 PNEXT, 11 TLEN, 12 QUAL, 13 a malformed tag, 14 an unknown tag type, 15 an unknown B subtype,
+ * 16 an integer out of range, 17 a float, 18 RNAME set with POS 0, 19 a header line. */
+int  mk_bam_encode_size_device(mk_bam *, const char *d_text, size_t n, size_t *n_lines, size_t *rec_bytes, uint64_t *bad_line, int *bad_code,
+                               void *stream);
+/* Step 2: the records of the last step 1 written at d_out + base (d_out + out_cap is the end of the buffer), and
+ * d_off[0..n_lines] = base + their offsets.  d_text must be unchanged since step 1.  Float values off the exact fast path are
+ * converted on the host with strtof inside the call (*n_patched lines, may be NULL). */
+int  mk_bam_encode_write_device(mk_bam *, uint8_t *d_out, uint64_t base, size_t out_cap, uint64_t *d_off, size_t *n_patched, void *stream);
+/* Stable sort of n records by (tid with -1 last, pos + 1, flag & 16); *total_bytes: their bytes.  The records must stay in place
+ * until the last gather of this order. */
+int  mk_bam_sort_device(mk_bam *, const uint8_t *d_rec, const uint64_t *d_off, size_t n, size_t *total_bytes, void *stream);
+/* Sorted records [i0, i1) back to back at d_out: i1 is the largest index whose records take at most max_bytes (at least one
+ * record).  *d_out_off (may be NULL): device offsets of those records (i1 - i0 + 1 values, base: the first), for
+ * mk_bam_index_add_device. */
+int  mk_bam_gather_device(mk_bam *, size_t i0, size_t max_bytes, uint8_t *d_out, size_t out_cap, size_t *i1, size_t *bytes,
+                          const uint64_t **d_out_off, void *stream);
+/* The index: records are added in file order with their offset in the uncompressed record stream (u_base of each call =
+ * the bytes added before); mk_bam_bai lays out the .bai from the member table of the compressed record stream:
+ * coff[k] = the file offset of member k, k = 0 .. n_members (the last: where the EOF member starts).  *bai is owned by the
+ * object until its next call; the index then starts over (as after mk_bam_index_reset). */
+int  mk_bam_index_reset(mk_bam *);
+int  mk_bam_index_add_device(mk_bam *, const uint8_t *d_rec, const uint64_t *d_off, size_t n, uint64_t u_base, void *stream);
+int  mk_bam_bai(mk_bam *, const uint64_t *coff, size_t n_coff, const uint8_t **bai, size_t *len);
+uint64_t mk_bam_launch_count(mk_bam *);
+/* The default run size of sam2bam for text chunks of `chunk` bytes: (free device memory - 8 chunks - 512 MiB) / 2.2 (the run's
+ * bytes plus the per-record workspace of an object with max_records = bytes / 64); 0 when that is negative. */
+int  mk_bam_sort_budget(int device, size_t chunk, size_t *bytes);
+
 /* ------------------------------------------------------------------ multi-GPU exchange over NVLink peer memory */
 /* One object per rank (one process per GPU, or several ranks in one process).  Owner bucketing and the all-to-all are ONE
  * kernel: owner = mix(chr1, chr2, pos1 / res) mod world (mk_pairs_owner); every rank writes its pairs straight into the

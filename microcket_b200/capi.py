@@ -168,7 +168,15 @@ class Lib:
                            ("mk_bgzf_text_stats", [vp, P(u64), P(C.c_int64)]), ("mk_bgzf_launch_count", [vp]),
                            ("mk_bgzf_deflate_bound", [sz]), ("mk_bgzf_enc_create", [i, sz, P(vp)]), ("mk_bgzf_enc_destroy", [vp]),
                            ("mk_bgzf_deflate_device", [vp, vp, sz, i, vp, sz, P(sz), P(BgzfMember), sz, P(sz), vp]),
-                           ("mk_bgzf_enc_launch_count", [vp])):
+                           ("mk_bgzf_enc_launch_count", [vp]),
+                           ("mk_bam_create", [i, P(C.c_char_p), P(C.c_uint32), i, sz, sz, P(vp)]), ("mk_bam_destroy", [vp]),
+                           ("mk_bam_encode_size_device", [vp, vp, sz, P(sz), P(sz), P(u64), P(i), vp]),
+                           ("mk_bam_encode_write_device", [vp, vp, u64, sz, vp, P(sz), vp]),
+                           ("mk_bam_sort_device", [vp, vp, vp, sz, P(sz), vp]),
+                           ("mk_bam_gather_device", [vp, sz, sz, vp, sz, P(sz), P(sz), P(vp), vp]),
+                           ("mk_bam_index_reset", [vp]), ("mk_bam_index_add_device", [vp, vp, vp, sz, u64, vp]),
+                           ("mk_bam_bai", [vp, P(u64), sz, P(vp), P(sz)]), ("mk_bam_launch_count", [vp]),
+                           ("mk_bam_sort_budget", [i, sz, P(sz)])):
             if hasattr(L, name):
                 getattr(L, name).argtypes = args
         if hasattr(L, "mk_pairs_owner"):
@@ -179,7 +187,7 @@ class Lib:
         if hasattr(L, "mk_pairs_dropped"):
             L.mk_pairs_dropped.restype = u64
         for name in ("mk_hist_dropped", "mk_hist_launch_count", "mk_xchg_launch_count", "mk_norm_launch_count", "mk_bgzf_launch_count",
-                     "mk_bgzf_enc_launch_count"):
+                     "mk_bgzf_enc_launch_count", "mk_bam_launch_count"):
             if hasattr(L, name):
                 getattr(L, name).restype = u64
         if hasattr(L, "mk_bgzf_deflate_bound"):
@@ -756,6 +764,76 @@ def bgzf_compress(data, level=-1, eof=True, device=0):
     finally:
         bd.close()
     return d_out[:n].cpu().numpy().tobytes() + (BGZF_EOF if eof else b"")
+
+
+class BamInputError(MkError):
+    """a refused SAM line: .line (0-based within the call) and .code (bam_encode.h's BE_E* code)"""
+
+    def __init__(self, msg, line, code):
+        super().__init__(msg)
+        self.line, self.code = line, code
+
+
+class Bam:
+    """Coordinate-sorted BAM records and their .bai in HBM (csrc/bam_out.cu): one object per reference dictionary."""
+
+    def __init__(self, refs, max_text, max_records, device=0):
+        """refs: [(name, length)] in @SQ order; max_text: bytes of one encode call; max_records: records of one sort"""
+        self.lib = lib()
+        self.lib.require_gpu()
+        self.h = C.c_void_p()
+        names = (C.c_char_p * max(len(refs), 1))(*[n.encode() for n, _ in refs])
+        lens = (C.c_uint32 * max(len(refs), 1))(*[l for _, l in refs])
+        self.lib.check(self.lib.L.mk_bam_create(device, names, lens, len(refs), max_text, max_records, C.byref(self.h)))
+
+    def encode(self, d_text, n, d_out, out_cap, d_off, base=0, stream=0):
+        """n bytes of SAM lines at d_text -> records at d_out + base, d_off[0..n_records] = base + offsets -> (n_records, bytes)"""
+        nl, rb, bad, code = C.c_size_t(), C.c_size_t(), C.c_uint64(), C.c_int()
+        r = self.lib.L.mk_bam_encode_size_device(self.h, d_text, n, C.byref(nl), C.byref(rb), C.byref(bad), C.byref(code), stream)
+        if r == -6:
+            raise BamInputError(self.lib.L.mk_last_error().decode(errors="replace"), bad.value, code.value)
+        self.lib.check(r)
+        self.lib.check(self.lib.L.mk_bam_encode_write_device(self.h, d_out, base, out_cap, d_off, None, stream))
+        return nl.value, rb.value
+
+    def sort(self, d_rec, d_off, n, stream=0):
+        """stable coordinate sort of n records -> their bytes"""
+        tot = C.c_size_t()
+        self.lib.check(self.lib.L.mk_bam_sort_device(self.h, d_rec, d_off, n, C.byref(tot), stream))
+        return tot.value
+
+    def gather(self, i0, max_bytes, d_out, out_cap, stream=0):
+        """sorted records [i0, i1) to d_out -> (i1, bytes, device pointer of their offsets)"""
+        i1, nb, p = C.c_size_t(), C.c_size_t(), C.c_void_p()
+        self.lib.check(self.lib.L.mk_bam_gather_device(self.h, i0, max_bytes, d_out, out_cap, C.byref(i1), C.byref(nb), C.byref(p), stream))
+        return i1.value, nb.value, p.value
+
+    def index_reset(self):
+        self.lib.check(self.lib.L.mk_bam_index_reset(self.h))
+
+    def index_add(self, d_rec, d_off, n, u_base, stream=0):
+        self.lib.check(self.lib.L.mk_bam_index_add_device(self.h, d_rec, d_off, n, u_base, stream))
+
+    def bai(self, coff):
+        """the .bai bytes from the member table of the record stream (file offset of every member, then of the EOF member)"""
+        arr = (C.c_uint64 * max(len(coff), 1))(*coff)
+        p, n = C.c_void_p(), C.c_size_t()
+        self.lib.check(self.lib.L.mk_bam_bai(self.h, arr, len(coff), C.byref(p), C.byref(n)))
+        return C.string_at(p.value, n.value) if n.value else b""
+
+    def launches(self):
+        return self.lib.L.mk_bam_launch_count(self.h)
+
+    def close(self):
+        if self.h:
+            self.lib.L.mk_bam_destroy(self.h)
+            self.h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 class Xchg:

@@ -49,6 +49,13 @@ BG_FN void bgd_dist_sym(uint32_t dist, uint32_t &sym, uint32_t &ext, uint32_t &n
     else { nb = (uint32_t)bgd_log2(d) - 1; sym = 2 * nb + 2 + ((d >> nb) & 1); ext = d & ((1u << nb) - 1); }
 }
 BG_FN uint32_t bgd_fixed_len(int s) { return s < 144 ? 8 : s < 256 ? 9 : s < 280 ? 7 : 8; }
+// the fixed literal/length code of RFC 1951 §3.2.6, bit-reversed.  Not the canonical code of the 286 lengths above: the fixed
+// code also gives 8-bit codes to symbols 286 and 287, which shifts every 9-bit code (literals 144-255) by 4
+BG_FN uint32_t bgd_fixed_code(int s) {
+    uint32_t v = s < 144 ? 0x30 + s : s < 256 ? 0x190 + (s - 144) : s < 280 ? s - 256 : 0xc0 + (s - 280), r = 0;
+    for (uint32_t b = 0; b < bgd_fixed_len(s); ++b) { r = r << 1 | (v & 1); v >>= 1; }
+    return r;
+}
 
 // ---------------------------------------------------------------- the member's codes and block plan
 struct BgdPlan {
@@ -189,7 +196,9 @@ template <class T> BG_FN void bgd_plan(T &t, BgdPlan *p, uint32_t n) {
             for (int s = 0; s < BGD_NL; ++s) p->ll[s] = (uint8_t)bgd_fixed_len(s);
             for (int s = 0; s < BGD_ND; ++s) p->ld[s] = 5;
         } else { p->btype = 2; p->bits = dyn; p->hdr_bits = hdr; }
-        if (p->btype) { bgd_codes(p, p->ll, BGD_NL, p->cl); bgd_codes(p, p->ld, BGD_ND, p->cd); bgd_codes(p, p->lc, BGD_NC, p->cc); }
+        if (p->btype == 1) for (int s = 0; s < BGD_NL; ++s) p->cl[s] = (uint16_t)bgd_fixed_code(s);
+        if (p->btype == 2) bgd_codes(p, p->ll, BGD_NL, p->cl);
+        if (p->btype) { bgd_codes(p, p->ld, BGD_ND, p->cd); bgd_codes(p, p->lc, BGD_NC, p->cc); }
     }
     t.sync();
 }
