@@ -149,6 +149,31 @@ int  mk_s2p_run_device(mk_ctx *, const char *d_sam, size_t n, int is_last, mk_s2
  * mk_xchg_finish_device.  NULL detaches. */
 struct mk_xchg;
 int  mk_s2p_attach_xchg(mk_ctx *, struct mk_xchg *, uint32_t res);
+/* Multi-GPU SAM-space krmdup (cfg.rmdup): ONE first-occurrence decision over the whole stream, whose shards of whole read
+ * groups sit on the ranks in file order (shard r on rank r, every shard but the last followed by the next shard's first
+ * read group, as for cfg.sharded).  A read pair is kept iff no pair with its key (and identity space) comes earlier in
+ * (rank, line) order on any rank.  Concatenated in rank order, the ranks' pass-2 text and SAM passthrough are those of
+ * one cfg.rmdup context over the whole stream, and the ranks' logs add up to its logs.
+ *   pass 1  mk_s2p_rmdup_keys_device over the shard WITHOUT the appended group, any number of calls (as
+ *           mk_s2p_run_device: *consumed tells where the next call starts; is_last on the final one).  One 16-byte
+ *           record {key, rank | line} per read pair; discarded pairs never leave the GPU.  More than cfg.rmdup_capacity
+ *           read pairs in the shard: MK_ERR_CAPACITY.
+ *   send    mk_s2p_rmdup_send: the records go to their keys' owners through the exchange (returns at once).
+ *   decide  mk_s2p_rmdup_decide: waits for the keys this rank owns, sorts them by (key, rank, line), keeps the first of
+ *           each key and sends the others back to their ranks.  An owner sent 2^30 or more records, or more than the
+ *           exchange's capacity: MK_ERR_CAPACITY.
+ *   receive mk_s2p_rmdup_receive: waits for this rank's removed read pairs; the context is then settled.
+ *   pass 2  mk_s2p_run_device over the shard WITH the appended group: settled read pairs are removed before grouping;
+ *           lines past pass 1's are kept.  Pass 2 before receive: MK_ERR_STATE; text whose lines differ from pass 1's:
+ *           MK_ERR_INPUT on the is_last call.
+ * One host thread can drive all ranks of one process (send all, decide all, receive all); a rank in a process of its own
+ * calls the three steps in a row.  Every wait is the exchange's bounded one.  Steps out of order, or a context without
+ * cfg.rmdup: MK_ERR_STATE.  mk_s2p_push is refused in this mode; mk_s2p_rmdup_stats gives this rank's share of krmdup's
+ * log (its read pairs and discards, the keys it owns as Uniq / Dup); mk_s2p_reset leaves the mode. */
+int  mk_s2p_rmdup_keys_device(mk_ctx *, const char *d_sam, size_t n, int is_last, size_t *consumed, void *stream);
+int  mk_s2p_rmdup_send(mk_ctx *, struct mk_xchg *, void *stream);
+int  mk_s2p_rmdup_decide(mk_ctx *, struct mk_xchg *, void *stream);
+int  mk_s2p_rmdup_receive(mk_ctx *, struct mk_xchg *, void *stream);
 /* number of kernel launches issued by this context so far (for bench accounting) */
 uint64_t mk_launch_count(mk_ctx *);
 /* Optional per-kernel device timing with CUDA events on the launching stream (bench.py's roofline figure).

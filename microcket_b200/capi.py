@@ -123,6 +123,9 @@ class Lib:
         L.mk_s2p_run_device.argtypes = [vp, vp, sz, i, P(S2PDevIO), vp]
         L.mk_launch_count.argtypes = [vp]
         L.mk_s2p_attach_xchg.argtypes = [vp, vp, C.c_uint32]
+        L.mk_s2p_rmdup_keys_device.argtypes = [vp, vp, sz, i, P(sz), vp]
+        for name in ("mk_s2p_rmdup_send", "mk_s2p_rmdup_decide", "mk_s2p_rmdup_receive"):
+            getattr(L, name).argtypes = [vp, vp, vp]
         L.mk_launch_count.restype = u64
         L.mk_synth_host.argtypes = [u64, i, i, u64, u64, vp, sz, P(sz)]
         L.mk_synth_device.argtypes = [i, u64, i, i, u64, u64, vp, sz, P(sz), vp]
@@ -343,6 +346,24 @@ class Sam2Pairs:
     def attach_xchg(self, xchg, res):
         """every window's packed pairs leave for their owners on a side stream while the next window is parsed"""
         self.lib.check(self.lib.L.mk_s2p_attach_xchg(self.h, xchg.h if xchg is not None else None, res))
+
+    def rmdup_keys_device(self, d_ptr, n, is_last, stream=0):
+        """multi-rank krmdup, pass 1 over this rank's shard in HBM (cfg.rmdup) → bytes consumed (the next call starts there)"""
+        consumed = C.c_size_t()
+        self.lib.check(self.lib.L.mk_s2p_rmdup_keys_device(self.h, d_ptr, n, int(is_last), C.byref(consumed), stream))
+        return consumed.value
+
+    def rmdup_send(self, xchg, stream=0):
+        """the pass-1 key records leave for their owners (returns at once)"""
+        self.lib.check(self.lib.L.mk_s2p_rmdup_send(self.h, xchg.h, stream))
+
+    def rmdup_decide(self, xchg, stream=0):
+        """wait for the keys this rank owns, keep each key's first occurrence, send the others back"""
+        self.lib.check(self.lib.L.mk_s2p_rmdup_decide(self.h, xchg.h, stream))
+
+    def rmdup_receive(self, xchg, stream=0):
+        """wait for this rank's removed read pairs; run_device is then pass 2"""
+        self.lib.check(self.lib.L.mk_s2p_rmdup_receive(self.h, xchg.h, stream))
 
     def enable_timing(self, on=True):
         self.lib.check(self.lib.L.mk_s2p_enable_timing(self.h, int(on)))

@@ -7,11 +7,16 @@
 #include <vector>
 #include "ctx.h"
 #include "s2p_kernels.cuh"
+#include "radix_sort.cuh"
 
 struct mk_xchg;
 extern "C" int mk_xchg_begin(mk_xchg *);
 extern "C" int mk_xchg_scatter_part_device(mk_xchg *, const mk_pair *, const uint64_t *, uint32_t, void *);
 extern "C" int mk_xchg_end_device(mk_xchg *, void *);
+int xchg_scatter_records(mk_xchg *, const void *d_rec, u64 n, const unsigned long long *d_part, int owner, cudaStream_t);   // xchg.cu
+void xchg_world_rank(const mk_xchg *, int *world, int *rank);
+// multi-rank krmdup (mk_s2p_rmdup_*): off, pass 1 running, pass 1 done, keys sent, losers sent back, drop bits settled
+enum { RKP_OFF = 0, RKP_PASS1, RKP_KEYED, RKP_SENT, RKP_DECIDED, RKP_SETTLED };
 #define S2P_XPARTS 4096                            // windows of one mk_s2p_run_device call whose pairs can be scattered separately
 
 static const size_t S2P_CARRY = 8u << 20;          // room in front of every window for the previous window's last group
@@ -62,6 +67,11 @@ struct S2PCtx : mk_ctx {
     // overlapped multi-GPU scatter (mk_s2p_attach_xchg)
     mk_xchg *xchg = nullptr; u32 xchg_res = 0; cudaStream_t s_x = nullptr; DevBuf d_xparts; u32 x_slot = 0;
     std::vector<cudaEvent_t> x_events; size_t x_ev_used = 0;
+    // multi-rank krmdup: phase, pass 1's records (in d_rmtab[0], which this mode does not use as a table) and totals, the
+    // owner's sort buffers, the drop bits of pass 1's lines
+    int rk = RKP_OFF;
+    u64 rk_cap = 0, rk_lines = 0, rk_keys = 0, rk_disc = 0;
+    DevBuf d_rkcnt, d_rksort, d_rklose, d_rkdrop; RadixWs rk_rws;
     // optional per-kernel timing (bench.py roofline): events around every kernel of every window
     bool timing = false;
     std::vector<cudaEvent_t> ev_pool; size_t ev_used = 0;
@@ -117,7 +127,11 @@ static S2PParams make_params(S2PCtx *c, const char *buf, u64 *sc_list, u32 sc_ca
     p.mode = c->cfg.mode; p.min_mapq = c->cfg.min_mapq; p.ratio = c->cfg.min_mapped_ratio; p.lane = c->cfg.lane;
     p.write_sam = c->cfg.write_sam && out_sam; p.emit_text = c->cfg.emit_text && out_text; p.emit_packed = c->cfg.emit_packed && out_pairs;
     p.running_offsets = running;
-    p.xparts = (c->xchg && c->d_xparts.p) ? c->d_xparts.as<unsigned long long>() : nullptr;
+    p.xparts = (c->xchg && c->d_xparts.p && c->rk != RKP_PASS1) ? c->d_xparts.as<unsigned long long>() : nullptr;
+    if (c->rk != RKP_OFF) {
+        p.rk_rec = c->d_rmtab[0].as<uint4>(); p.rk_cap = c->rk_cap;
+        p.rk_drop = c->d_rkdrop.as<u32>(); p.rk_lines = c->rk_lines; p.rk_cnt = c->d_rkcnt.as<unsigned long long>();
+    }
     p.rm_on = c->cfg.rmdup ? 1 : 0;
     if (p.rm_on) {
         p.rm_hskip1 = c->cfg.hskip1; p.rm_klen1 = c->cfg.klen1; p.rm_hskip2 = c->cfg.hskip2; p.rm_klen2 = c->cfg.klen2;
@@ -149,7 +163,21 @@ static void launch_window(S2PCtx *c, const S2PParams &p, cudaStream_t s) {
     k_chunk_compact<<<(c->n_chunks_cap + 7) / 8, 256, 0, s>>>(p);
     k_scan_lines<4, 4><<<c->grid_scan4, S2P_SCAN_THREADS, 4 * 8192, s>>>(p, 1);
     mark(1);
-    if (p.rm_on) {                                       // SAM-space krmdup: duplicate / discarded read pairs lose LM_KEEP before grouping
+    if (c->rk == RKP_PASS1) {                            // multi-rank krmdup, pass 1: the key records of the window's runs, no output
+        k_parse<true><<<c->grid_parse, 256, PR_SMEM, s>>>(p);
+        mark(7);
+        k_rm_keys<<<c->grid_rm, 256, 0, s>>>(p);
+        mark(5);
+        k_win_end<<<1, 1, 0, s>>>(p, c->x_slot);
+        c->launches += 8;
+        return;
+    }
+    if (p.rm_on && c->rk == RKP_SETTLED) {               // pass 2: the settled drop bits in place of the key table
+        k_parse<false><<<c->grid_parse, 256, PR_SMEM, s>>>(p);
+        mark(7);
+        k_rm_apply<<<c->grid_gs, 256, 0, s>>>(p);
+        c->launches += 1;
+    } else if (p.rm_on) {                                // SAM-space krmdup: duplicate / discarded read pairs lose LM_KEEP before grouping
         k_parse<true><<<c->grid_parse, 256, PR_SMEM, s>>>(p);
         mark(7);
         k_rm_insert<<<c->grid_rm, 256, 0, s>>>(p);
@@ -481,6 +509,7 @@ static bool host_ptr_is_pinned(const void *p) {
 
 extern "C" int mk_s2p_push(mk_ctx *x, const char *bytes, size_t n, int is_last) {
     S2PCtx *c; MK_TRY(s2p_check(x, &c));
+    if (c->rk != RKP_OFF) { mk_set_error("mk_s2p_push on a context in the multi-rank krmdup mode (device-resident only)"); return MK_ERR_STATE; }
     if (c->finished_input) { mk_set_error("mk_s2p_push after the last chunk"); return MK_ERR_STATE; }
     if (c->use_device_path) { mk_set_error("mk_s2p_push on a context used with mk_s2p_run_device"); return MK_ERR_STATE; }
     const bool pinned = n >= (1u << 20) && host_ptr_is_pinned(bytes);
@@ -665,6 +694,13 @@ extern "C" int mk_s2p_rmdup_stats(mk_ctx *x, mk_dedup_stats *out) {
     if (!out) { mk_set_error("mk_s2p_rmdup_stats: null stats"); return MK_ERR_ARG; }
     if (!c->cfg.rmdup) { mk_set_error("mk_s2p_rmdup_stats: context created without cfg.rmdup"); return MK_ERR_STATE; }
     MK_CUDA(cudaStreamSynchronize(c->s_comp));
+    if (c->rk != RKP_OFF) {                          // this rank's share: its read pairs and discards, the keys it owns
+        unsigned long long h[RK_N];
+        MK_CUDA(cudaDeviceSynchronize());
+        MK_CUDA(cudaMemcpy(h, c->d_rkcnt.p, sizeof h, cudaMemcpyDeviceToHost));
+        out->uniq = (u32)h[RK_UNIQ]; out->dup = (u32)h[RK_DUP]; out->discard = (u32)c->rk_disc; out->pairs = c->rk_keys + c->rk_disc;
+        return MK_OK;
+    }
     WinState st;
     MK_CUDA(cudaMemcpy(&st, c->d_state.p, sizeof st, cudaMemcpyDeviceToHost));
     out->uniq = (u32)st.rm_uniq; out->discard = (u32)st.rm_discard; out->dup = (u32)(st.rm_total - st.rm_uniq - st.rm_discard);
@@ -672,17 +708,25 @@ extern "C" int mk_s2p_rmdup_stats(mk_ctx *x, mk_dedup_stats *out) {
     return MK_OK;
 }
 
-// Forget the stream (counters, carried group, pending output) but keep every allocation and the chromosome table:
-// the context can then process another input from the start.
-extern "C" int mk_s2p_reset(mk_ctx *x) {
-    S2PCtx *c; MK_TRY(s2p_check(x, &c));
+// a stream that starts over, with the chromosome table learnt so far
+static int s2p_state_clear(S2PCtx *c) {
     MK_CUDA(cudaDeviceSynchronize());
     WinState st;
     MK_CUDA(cudaMemcpy(&st, c->d_state.p, sizeof st, cudaMemcpyDeviceToHost));
     u32 n_chrom = st.n_chrom;
     memset(&st, 0, sizeof st); st.n_chrom = n_chrom; st.rm_allones[0] = st.rm_allones[1] = ~0ull;
     MK_CUDA(cudaMemcpy(c->d_state.p, &st, sizeof st, cudaMemcpyHostToDevice));
+    return MK_OK;
+}
+
+// Forget the stream (counters, carried group, pending output) but keep every allocation and the chromosome table:
+// the context can then process another input from the start.
+extern "C" int mk_s2p_reset(mk_ctx *x) {
+    S2PCtx *c; MK_TRY(s2p_check(x, &c));
+    MK_TRY(s2p_state_clear(c));
     for (int t = 0; t < 2; ++t) if (c->d_rmtab[t].p) MK_CUDA(cudaMemset(c->d_rmtab[t].p, 0xFF, c->rm_slots[t] * 16));
+    if (c->d_rkcnt.p) MK_CUDA(cudaMemset(c->d_rkcnt.p, 0, c->d_rkcnt.n));
+    c->rk = RKP_OFF; c->rk_lines = c->rk_keys = c->rk_disc = 0;
     for (auto &s : c->slot) { s.busy = false; s.free_pending = false; s.text_len = s.text_off = s.pairs_n = s.pairs_off = s.sam_len = s.sam_off = 0; }
     c->tail.clear(); c->windows = 0; c->prev_slot = -1; c->finished_input = false; c->use_device_path = false;
     c->q_text.clear(); c->q_sam.clear(); c->q_pairs.clear(); c->q_text_off = c->q_sam_off = c->q_pairs_off = 0;
@@ -717,26 +761,17 @@ extern "C" uint64_t mk_launch_count(mk_ctx *x) {
 }
 
 // ------------------------------------------------------------------------------------------------ device-resident run
-extern "C" int mk_s2p_run_device(mk_ctx *x, const char *d_sam, size_t n, int is_last, mk_s2p_dev_io *io, void *stream) {
-    S2PCtx *c; MK_TRY(s2p_check(x, &c));
-    if (!io) { mk_set_error("mk_s2p_run_device: null io"); return MK_ERR_ARG; }
-    if (((uintptr_t)d_sam & 15) != 0) { mk_set_error("mk_s2p_run_device: d_sam must be 16-byte aligned"); return MK_ERR_ARG; }
-    if (c->windows) { mk_set_error("mk_s2p_run_device on a context used with mk_s2p_push"); return MK_ERR_STATE; }
-    c->use_device_path = true;
-    if (!c->d_sclist.p) { c->sc_cap_dev = 16u << 20; MK_TRY(c->d_sclist.alloc((size_t)c->sc_cap_dev * 8)); }
-    cudaStream_t s = stream ? (cudaStream_t)stream : c->s_comp;
+// The windows of one device-resident call, enqueued ahead and topped up until the input is consumed (both passes of the
+// multi-rank krmdup and mk_s2p_run_device)
+static int s2p_device_loop(S2PCtx *c, S2PParams &p, size_t n, int is_last, cudaStream_t s, WinState &st) {
     WinState *dst = c->d_state.as<WinState>();
     k_set_stream<<<1, 1, 0, s>>>(dst, 0, n, is_last ? 1u : 0u);
     c->launches += 1;
-    S2PParams p = make_params(c, d_sam, c->d_sclist.as<u64>(), c->sc_cap_dev, io->d_pairs_text, io->pairs_text_cap, io->d_pairs, io->pairs_cap, io->d_sam_text, io->sam_text_cap, c->W, 1, (u64 *)io->d_line_off, io->line_off_cap, io->line_off_base);
     MK_TRY(upload_params(c, p, 2, s));
-    const bool xch = c->xchg && p.xparts && p.out_pairs;
-    if (xch) { MK_TRY(mk_xchg_begin(c->xchg)); c->x_ev_used = 0; }
     // running output offsets restart at 0 for every call
     MK_CUDA(cudaMemsetAsync((char *)dst + offsetof(WinState, out_text), 0, 3 * sizeof(u64), s));
     // every window consumes at least W - (largest read group) bytes; enqueue an upper bound and top up if needed
     size_t done = 0;
-    WinState st;
     int guard = 0;
     while (true) {
         size_t remaining = n - done;
@@ -757,13 +792,146 @@ extern "C" int mk_s2p_run_device(mk_ctx *x, const char *d_sam, size_t n, int is_
         if (!is_last && st.we == n) break;
         done = st.cursor;
     }
-    io->pairs_text_len = st.out_text; io->n_pairs = st.out_pairs; io->sam_text_len = st.out_sam; io->consumed = st.cursor;
     c->last_state = st;
+    return MK_OK;
+}
+
+extern "C" int mk_s2p_run_device(mk_ctx *x, const char *d_sam, size_t n, int is_last, mk_s2p_dev_io *io, void *stream) {
+    S2PCtx *c; MK_TRY(s2p_check(x, &c));
+    if (!io) { mk_set_error("mk_s2p_run_device: null io"); return MK_ERR_ARG; }
+    if (((uintptr_t)d_sam & 15) != 0) { mk_set_error("mk_s2p_run_device: d_sam must be 16-byte aligned"); return MK_ERR_ARG; }
+    if (c->windows) { mk_set_error("mk_s2p_run_device on a context used with mk_s2p_push"); return MK_ERR_STATE; }
+    if (c->rk != RKP_OFF && c->rk != RKP_SETTLED) { mk_set_error("mk_s2p_run_device: multi-rank krmdup pass 2 before mk_s2p_rmdup_receive"); return MK_ERR_STATE; }
+    c->use_device_path = true;
+    if (!c->d_sclist.p) { c->sc_cap_dev = 16u << 20; MK_TRY(c->d_sclist.alloc((size_t)c->sc_cap_dev * 8)); }
+    cudaStream_t s = stream ? (cudaStream_t)stream : c->s_comp;
+    S2PParams p = make_params(c, d_sam, c->d_sclist.as<u64>(), c->sc_cap_dev, io->d_pairs_text, io->pairs_text_cap, io->d_pairs, io->pairs_cap, io->d_sam_text, io->sam_text_cap, c->W, 1, (u64 *)io->d_line_off, io->line_off_cap, io->line_off_base);
+    const bool xch = c->xchg && p.xparts && p.out_pairs;
+    if (xch) { MK_TRY(mk_xchg_begin(c->xchg)); c->x_ev_used = 0; }
+    WinState st;
+    MK_TRY(s2p_device_loop(c, p, n, is_last, s, st));
+    io->pairs_text_len = st.out_text; io->n_pairs = st.out_pairs; io->sam_text_len = st.out_sam; io->consumed = st.cursor;
     if (xch) {                                              // every part is out: close the epoch on the side stream, and let `s` see it
         MK_TRY(mk_xchg_end_device(c->xchg, c->s_x));
         if (c->x_events.empty()) { cudaEvent_t e; cudaEventCreateWithFlags(&e, cudaEventDisableTiming); c->x_events.push_back(e); }
         MK_CUDA(cudaEventRecord(c->x_events[0], c->s_x));
         MK_CUDA(cudaStreamWaitEvent(s, c->x_events[0], 0));
     }
+    if (c->rk == RKP_SETTLED && is_last) {                  // pass 2 must have met every run head of pass 1, at the same lines
+        unsigned long long h[RK_N];
+        MK_CUDA(cudaMemcpy(h, c->d_rkcnt.p, sizeof h, cudaMemcpyDeviceToHost));
+        if (st.lines_done < c->rk_lines || h[RK_FP1] != h[RK_FP2]) {
+            mk_set_error("mk_s2p_run_device: pass 2 does not hold the %llu lines of pass 1 (the text differs)", (unsigned long long)c->rk_lines);
+            return MK_ERR_INPUT;
+        }
+    }
+    return MK_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ multi-rank krmdup
+extern "C" int mk_s2p_rmdup_keys_device(mk_ctx *x, const char *d_sam, size_t n, int is_last, size_t *consumed, void *stream) {
+    S2PCtx *c; MK_TRY(s2p_check(x, &c));
+    if (((uintptr_t)d_sam & 15) != 0) { mk_set_error("mk_s2p_rmdup_keys_device: d_sam must be 16-byte aligned"); return MK_ERR_ARG; }
+    if (!c->cfg.rmdup) { mk_set_error("mk_s2p_rmdup_keys_device: context created without cfg.rmdup"); return MK_ERR_STATE; }
+    if (c->windows || (c->rk == RKP_OFF && c->use_device_path)) { mk_set_error("mk_s2p_rmdup_keys_device on a context that has run: mk_s2p_reset first"); return MK_ERR_STATE; }
+    if (c->rk != RKP_OFF && c->rk != RKP_PASS1) { mk_set_error("mk_s2p_rmdup_keys_device: pass 1 is over"); return MK_ERR_STATE; }
+    if (c->rk == RKP_OFF) {
+        c->rk_cap = c->cfg.rmdup_capacity ? c->cfg.rmdup_capacity : (u64)1 << 24;   // d_rmtab[0] holds 2 x that many records
+        if (!c->d_rkcnt.p) MK_TRY(c->d_rkcnt.alloc(RK_N * sizeof(unsigned long long)));
+        MK_CUDA(cudaMemset(c->d_rkcnt.p, 0, c->d_rkcnt.n));
+        c->rk = RKP_PASS1;
+    }
+    c->use_device_path = true;
+    if (!c->d_sclist.p) { c->sc_cap_dev = 16u << 20; MK_TRY(c->d_sclist.alloc((size_t)c->sc_cap_dev * 8)); }
+    cudaStream_t s = stream ? (cudaStream_t)stream : c->s_comp;
+    S2PParams p = make_params(c, d_sam, c->d_sclist.as<u64>(), c->sc_cap_dev, nullptr, 0, nullptr, 0, nullptr, 0, c->W, 1);
+    WinState st;
+    MK_TRY(s2p_device_loop(c, p, n, is_last, s, st));
+    if (consumed) *consumed = st.cursor;
+    unsigned long long h[RK_N];
+    MK_CUDA(cudaMemcpy(h, c->d_rkcnt.p, sizeof h, cudaMemcpyDeviceToHost));
+    if (h[RK_KEYS] + h[RK_DISC] > c->rk_cap) {
+        mk_set_error("mk_s2p_rmdup_keys_device: more than cfg.rmdup_capacity = %llu read pairs in the shard", (unsigned long long)c->rk_cap);
+        return MK_ERR_CAPACITY;
+    }
+    if (is_last) {                                           // pass 2 starts a new stream over the same lines
+        c->rk_lines = st.lines_done; c->rk_keys = h[RK_KEYS]; c->rk_disc = h[RK_DISC];
+        MK_TRY(s2p_state_clear(c));
+        c->sc_full_rule = 0; c->sc_tail.clear(); c->sc_true = 0;
+        c->rk = RKP_KEYED;
+    }
+    return MK_OK;
+}
+
+static int rk_step(mk_ctx *x, mk_xchg *xc, int want, const char *what, S2PCtx **out) {
+    S2PCtx *c; MK_TRY(s2p_check(x, &c));
+    if (!xc) { mk_set_error("%s: null exchange", what); return MK_ERR_ARG; }
+    if (!c->cfg.rmdup) { mk_set_error("%s: context created without cfg.rmdup", what); return MK_ERR_STATE; }
+    if (c->rk != want) {
+        static const char *ph[] = {"before mk_s2p_rmdup_keys_device", "before the last pass-1 call", "before mk_s2p_rmdup_send",
+                                   "before mk_s2p_rmdup_decide", "before mk_s2p_rmdup_receive", "after mk_s2p_rmdup_receive"};
+        mk_set_error("%s called %s", what, ph[c->rk]);
+        return MK_ERR_STATE;
+    }
+    *out = c;
+    return MK_OK;
+}
+
+extern "C" int mk_s2p_rmdup_send(mk_ctx *x, mk_xchg *xc, void *stream) {
+    S2PCtx *c; MK_TRY(rk_step(x, xc, RKP_KEYED, "mk_s2p_rmdup_send", &c));
+    MK_TRY(xchg_scatter_records(xc, c->d_rmtab[0].p, c->rk_keys, nullptr, 1, (cudaStream_t)stream));
+    c->rk = RKP_SENT;
+    return MK_OK;
+}
+
+extern "C" int mk_s2p_rmdup_decide(mk_ctx *x, mk_xchg *xc, void *stream) {
+    S2PCtx *c; MK_TRY(rk_step(x, xc, RKP_SENT, "mk_s2p_rmdup_decide", &c));
+    cudaStream_t s = (cudaStream_t)stream;
+    mk_pair *d_recv = nullptr; size_t n = 0;
+    MK_TRY(mk_xchg_finish_device(xc, &d_recv, &n, s));                      // every rank's keys of this rank's share
+    if (n >= ((size_t)1 << 30)) { mk_set_error("mk_s2p_rmdup_decide: %zu key records for one owner (at most 2^30 - 1)", n); return MK_ERR_CAPACITY; }
+    if (c->d_rksort.n < n * 16) { MK_TRY(c->d_rksort.alloc(n * 16)); MK_TRY(c->d_rklose.alloc(n * 16)); }
+    if (!c->rk_rws.plan.p || c->rk_rws.max_n < n) MK_TRY(c->rk_rws.alloc(n));
+    // (tag, key, ord), LSD: ord's line and rank bytes, the key, the tag byte
+    RadixSchedule sch; sch.n_pass = 15;
+    for (int b = 0; b < 6; ++b) sch.byte_of[b] = 8 + b;
+    for (int b = 0; b < 8; ++b) sch.byte_of[6 + b] = b;
+    sch.byte_of[14] = 15;
+    Rec16::Bufs b; b.k[0] = (uint4 *)d_recv; b.k[1] = c->d_rksort.as<uint4>(); b.v[0] = b.v[1] = nullptr;
+    const int sms = mk_sm_count(c->cfg.device);
+    MK_TRY(radix_sort<Rec16>(b, n, sch, c->rk_rws, 0, sms, s, &c->launches));
+    unsigned long long *cnt = c->d_rkcnt.as<unsigned long long>();
+    const int grid = (int)std::max<u64>(1, std::min<u64>((n + 255) / 256, (u64)sms * 8));
+    k_rm_decide<<<grid, 256, 0, s>>>(b.k[0], b.k[1], &c->rk_rws.plan.as<RadixPlan>()->final_buf, n, c->d_rklose.as<uint4>(), cnt);
+    c->launches += 1;
+    MK_CUDA(cudaGetLastError());
+    MK_TRY(mk_xchg_begin(xc));                                                // the losers go back to their ranks
+    MK_TRY(xchg_scatter_records(xc, c->d_rklose.p, 0, cnt + RK_LOSE, 2, s));
+    MK_TRY(mk_xchg_end_device(xc, s));
+    c->rk = RKP_DECIDED;
+    return MK_OK;
+}
+
+extern "C" int mk_s2p_rmdup_receive(mk_ctx *x, mk_xchg *xc, void *stream) {
+    S2PCtx *c; MK_TRY(rk_step(x, xc, RKP_DECIDED, "mk_s2p_rmdup_receive", &c));
+    cudaStream_t s = (cudaStream_t)stream;
+    mk_pair *d_recv = nullptr; size_t n = 0;
+    MK_TRY(mk_xchg_finish_device(xc, &d_recv, &n, s));                      // this rank's losers, from every owner
+    int world = 1, rank = 0;
+    xchg_world_rank(xc, &world, &rank);
+    const size_t words = c->rk_lines / 32 + 1;
+    if (c->d_rkdrop.n < words * 4) MK_TRY(c->d_rkdrop.alloc(words * 4));
+    MK_CUDA(cudaMemsetAsync(c->d_rkdrop.p, 0, words * 4, s));
+    unsigned long long *cnt = c->d_rkcnt.as<unsigned long long>();
+    const int sms = mk_sm_count(c->cfg.device);
+    auto grid = [&](u64 m) { return (int)std::max<u64>(1, std::min<u64>((m + 255) / 256, (u64)sms * 8)); };
+    k_rm_settle<<<grid(c->rk_disc), 256, 0, s>>>(c->d_rmtab[0].as<uint4>() + (c->rk_cap - c->rk_disc), c->rk_disc, (u32)rank, 0, c->rk_lines, c->d_rkdrop.as<u32>(), cnt);
+    k_rm_settle<<<grid(n), 256, 0, s>>>((const uint4 *)d_recv, n, (u32)rank, 1, c->rk_lines, c->d_rkdrop.as<u32>(), cnt);
+    c->launches += 2;
+    unsigned long long bad = 0;
+    MK_CUDA(cudaMemcpyAsync(&bad, cnt + RK_BAD, 8, cudaMemcpyDeviceToHost, s));
+    MK_CUDA(cudaStreamSynchronize(s));
+    if (bad) { mk_set_error("mk_s2p_rmdup_receive: %llu returned records name another rank or a line past pass 1", bad); return MK_ERR_STATE; }
+    c->rk = RKP_SETTLED;
     return MK_OK;
 }

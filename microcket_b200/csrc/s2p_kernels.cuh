@@ -7,6 +7,8 @@
 //                  with more than 512 newlines in a chunk; also the FASTQ path's scan)
 //   k_parse        K2: one thread per line: first six fields, filter, CIGAR walk         (pairutil.h:63-126,155-161; unc2pairs.h:34-36)
 //   k_rm_insert    (cfg.rmdup only) krmdup's duplicate removal taken on the SAM: duplicate read pairs lose LM_KEEP    (src/preprocess/krmdup.cpp:103-212)
+//                  over several ranks (mk_s2p_rmdup_*): k_rm_keys in pass 1, k_rm_decide / k_rm_settle between the passes,
+//                  k_rm_apply in its place in pass 2
 //   k_group        K3: group heads among kept records + per-group resolution             (pairutil.h:163-173; flash2pairs.h; unc2pairs.h)
 //   k_emit_prefix / k_emit   K4: prefixes of the per-tile output sizes, .pairs text + packed records + line offsets   (unc2pairs.h:310-348)
 //   k_copy_sam     K5: SAM passthrough of the kept lines of emitted groups               (unc2pairs.h:351-356)
@@ -109,6 +111,11 @@ struct S2PParams {
     int rm_on, rm_hskip1, rm_klen1, rm_hskip2, rm_klen2;
     unsigned long long *rm_tab[2]; u64 rm_mask[2];
     u32 *rm_info;   // rm_info: K2's (flag | SEQ offset << 16) per line
+    // multi-rank krmdup (mk_s2p_rmdup_*): pass 1 writes {key, ord} records from the front of rk_rec and discarded run heads
+    // from its back; pass 2 reads the settled drop bits of the first rk_lines lines.  rk_cnt: RK_* counters
+    uint4 *rk_rec; u64 rk_cap;
+    const u32 *rk_drop; u64 rk_lines;
+    unsigned long long *rk_cnt;
     unsigned long long *xparts;   // optional: per launched window (end, count) of its packed pairs, for the overlapped multi-GPU scatter
     const S2PParams *self;    // device copy of this struct: what out-of-line callees are handed, so that the kernels' parameter block is never copied to local memory
 };
@@ -1149,6 +1156,25 @@ static __device__ __noinline__ void rm_line_keys_far(const S2PParams &p, u64 ws,
 // a smaller index -> this run is the duplicate.  No second pass over the table.  Uniq = keys ever claimed.
 // A run cut by the window end is decided in the next window; until then its lines do not count as kept, so that the group
 // before it stays the window's last (carried) group: it may yet turn out to be the stream's last one (pairutil.h:176).
+// The read pair of the run that starts at line i: its mates' key bits b1 / b2 and have = RL_M* | RL_OK* | RL_TAG.  Lines of
+// the CTA's round (i0 + t, t < 256) come from the staged s_*[t], later ones from global memory.  Returns the line after the run.
+static __device__ __forceinline__ u32 rm_run_combine(const S2PParams &p, u64 ws, u32 n, u32 i0, u32 i, u32 sl, u64 k1, u64 k2, const u8 *s_meta,
+                                                     const u8 *s_stat, const unsigned long long *s_k1, const unsigned long long *s_k2,
+                                                     u32 &have, u64 &b1, u64 &b2) {
+    have = 0; b1 = 0; b2 = 0;
+    u32 j = i;
+    while (true) {
+        if (sl & ~have & RL_M1) { b1 = k1; have |= RL_M1 | (sl & (RL_OK1 | RL_TAG)); }
+        if (sl & ~have & RL_M2) { b2 = k2; have |= RL_M2 | (sl & RL_OK2); }
+        ++j;
+        if (j >= n) break;
+        const u32 t = j - i0;
+        if (t < 256u) { if (!(s_meta[t] & LM_EQ)) break; sl = s_stat[t]; k1 = s_k1[t]; k2 = s_k2[t]; }
+        else { if (!(p.lmeta[j] & LM_EQ)) break; rm_line_keys_far(*p.self, ws, j, sl, k1, k2); }
+    }
+    return j;
+}
+
 static __global__ void __launch_bounds__(256) k_rm_insert(S2PParams p) {
     __shared__ unsigned long long s_k1[256], s_k2[256];
     __shared__ u8 s_stat[256], s_meta[256];
@@ -1166,17 +1192,8 @@ static __global__ void __launch_bounds__(256) k_rm_insert(S2PParams p) {
         s_meta[tid] = (u8)m_i; s_stat[tid] = (u8)sl; s_k1[tid] = k1; s_k2[tid] = k2;
         __syncthreads();
         if (i < n && !(m_i & LM_EQ) && !(sl & RL_HDR)) {
-            u32 have = 0; u64 b1 = 0, b2 = 0;
-            u32 j = i;
-            while (true) {
-                if (sl & ~have & RL_M1) { b1 = k1; have |= RL_M1 | (sl & (RL_OK1 | RL_TAG)); }
-                if (sl & ~have & RL_M2) { b2 = k2; have |= RL_M2 | (sl & RL_OK2); }
-                ++j;
-                if (j >= n) break;
-                const u32 t = j - i0;
-                if (t < 256u) { if (!(s_meta[t] & LM_EQ)) break; sl = s_stat[t]; k1 = s_k1[t]; k2 = s_k2[t]; }
-                else { if (!(p.lmeta[j] & LM_EQ)) break; rm_line_keys_far(*p.self, ws, j, sl, k1, k2); }
-            }
+            u32 have; u64 b1, b2;
+            const u32 j = rm_run_combine(p, ws, n, i0, i, sl, k1, k2, s_meta, s_stat, s_k1, s_k2, have, b1, b2);
             bool keep = false;
             if (j >= n && !final_win) ;                                  // undecided
             else if ((have & (RL_OK1 | RL_OK2)) == (RL_OK1 | RL_OK2)) {
@@ -1204,6 +1221,141 @@ static __global__ void __launch_bounds__(256) k_rm_insert(S2PParams p) {
         if (c_tot) atomicAdd(&st->rm_total, (unsigned long long)c_tot);
         if (c_uniq) atomicAdd(&st->rm_uniq, (unsigned long long)c_uniq);
         if (c_disc) atomicAdd(&st->rm_discard, (unsigned long long)c_disc);
+    }
+}
+
+// ---- the same rule over several ranks (mk_s2p_rmdup_*).  Shard line index = global line index of the single-GPU kernels.
+// A record is {key, ord}, ord = tag << 63 | rank << 40 | line of the run head: the smallest ord of a (tag, key) is the
+// first occurrence in (rank, line) order.  The rank is stamped by the exchange on the way to the key's owner.
+#define RK_KEYS 0      /* rk_cnt[]: records written from the front of rk_rec */
+#define RK_DISC 1      /* discarded run heads written from the back */
+#define RK_FP1 2       /* fingerprint of pass 1's run heads */
+#define RK_FP2 3       /* the same over pass 2's run heads below rk_lines */
+#define RK_UNIQ 4      /* owner: (tag, key) segments */
+#define RK_DUP 5       /* owner: records after a segment's first */
+#define RK_LOSE 6      /* owner: the losers' part (end, count) for the way back: 6, 7 */
+#define RK_BAD 8       /* receive: losers that name another rank or a line past pass 1 */
+#define RK_N 9
+#define RK_LINE_MASK ((1ull << 40) - 1)
+// what pass 2 must see again at a run head: its line index and the line's first bytes
+static __device__ __forceinline__ unsigned long long rk_fp(const S2PParams &p, u64 ws, u32 i, u64 me) {
+    const u64 a = ws + (i ? (u64)p.nl_pos[i - 1] + 1 : 0);
+    const u32 len = p.nl_pos[i] - (u32)(a - ws);
+    GlobalFetch gf; gf.buf = p.buf; gf.A = 0;
+    u64 x = fetch8(gf, a);
+    if (len < 8) x &= (1ull << (8 * len)) - 1;
+    return rm_hash(x ^ rm_hash(me + 1));
+}
+
+// Pass 1: one record per run head that the single-GPU kernel would settle (same staging, same run rule); a discarded run
+// (short mate, non-ACGT key base, no primary record for a mate) only leaves its line index, at the back.
+static __global__ void __launch_bounds__(256) k_rm_keys(S2PParams p) {
+    __shared__ unsigned long long s_k1[256], s_k2[256];
+    __shared__ u8 s_stat[256], s_meta[256];
+    WinState *st = p.st;
+    const u32 n = st->n_lines;
+    const u64 ws = st->ws, g0 = st->lines_done, counted = st->rm_counted;
+    const bool final_win = (st->we == st->total) && st->is_last;
+    const u32 tid = threadIdx.x, lane = tid & 31u;
+    unsigned long long fp = 0;
+    for (u32 i0 = blockIdx.x * 256u; i0 < n; i0 += gridDim.x * 256u) {
+        const u32 i = i0 + tid;
+        u32 m_i = 0, sl = 0; u64 k1 = 0, k2 = 0;
+        if (i < n) { m_i = p.lmeta[i]; rm_line_keys(p, ws, i, sl, k1, k2); }
+        __syncthreads();
+        s_meta[tid] = (u8)m_i; s_stat[tid] = (u8)sl; s_k1[tid] = k1; s_k2[tid] = k2;
+        __syncthreads();
+        bool is_key = false, is_disc = false;
+        uint4 rec = make_uint4(0, 0, 0, 0);
+        const u64 me = g0 + i;
+        if (i < n && !(m_i & LM_EQ) && !(sl & RL_HDR)) {
+            u32 have; u64 b1, b2;
+            const u32 j = rm_run_combine(p, ws, n, i0, i, sl, k1, k2, s_meta, s_stat, s_k1, s_k2, have, b1, b2);
+            if ((j < n || final_win) && me >= counted) {                // settled here, and not in an earlier window
+                const u64 ord = ((have & RL_TAG) ? 1ull << 63 : 0ull) | me;
+                if ((have & (RL_OK1 | RL_OK2)) == (RL_OK1 | RL_OK2)) {
+                    const u64 key = (b1 << (2 * p.rm_klen2)) | b2;
+                    rec = make_uint4((u32)key, (u32)(key >> 32), (u32)ord, (u32)(ord >> 32));
+                    is_key = true;
+                } else { rec = make_uint4(0, 0, (u32)me, (u32)(me >> 32)); is_disc = true; }
+                fp += rk_fp(p, ws, i, me);
+            }
+        }
+        // one reservation per warp and kind
+        const u32 bk = __ballot_sync(0xFFFFFFFFu, is_key), bd = __ballot_sync(0xFFFFFFFFu, is_disc);
+        unsigned long long base_k = 0, base_d = 0;
+        if (lane == 0 && bk) base_k = atomicAdd(&p.rk_cnt[RK_KEYS], (unsigned long long)__popc(bk));
+        if (lane == 0 && bd) base_d = atomicAdd(&p.rk_cnt[RK_DISC], (unsigned long long)__popc(bd));
+        base_k = __shfl_sync(0xFFFFFFFFu, base_k, 0); base_d = __shfl_sync(0xFFFFFFFFu, base_d, 0);
+        const u32 below = (1u << lane) - 1u;
+        if (is_key) { const u64 k = base_k + __popc(bk & below); if (k < p.rk_cap) p.rk_rec[k] = rec; }
+        if (is_disc) { const u64 d = base_d + __popc(bd & below); if (d < p.rk_cap) p.rk_rec[p.rk_cap - 1 - d] = rec; }
+    }
+    for (int o = 16; o; o >>= 1) fp += __shfl_xor_sync(0xFFFFFFFFu, fp, o);
+    if (lane == 0 && fp) atomicAdd(&p.rk_cnt[RK_FP1], fp);
+}
+
+// Pass 2, in place of k_rm_insert: a run loses LM_KEEP when its head's drop bit is set, or when the window end cuts it (it
+// is seen again in the next window, as in k_rm_insert).  Lines from rk_lines on belong to no settled run (the shard-boundary
+// group appended behind the shard) and are kept.
+static __global__ void __launch_bounds__(256) k_rm_apply(S2PParams p) {
+    const WinState *st = p.st;
+    const u32 n = st->n_lines;
+    const u64 ws = st->ws, g0 = st->lines_done, counted = st->rm_counted;
+    const bool final_win = (st->we == st->total) && st->is_last;
+    unsigned long long fp = 0;
+    for (u32 i = blockIdx.x * 256u + threadIdx.x; i < n; i += gridDim.x * 256u) {
+        if (p.lmeta[i] & LM_EQ) continue;
+        if (p.buf[ws + (i ? (u64)p.nl_pos[i - 1] + 1 : 0)] == '@') continue;   // a header line is no run (RL_HDR)
+        u32 j = i + 1;
+        while (j < n && (p.lmeta[j] & LM_EQ)) ++j;
+        const u64 me = g0 + i;
+        bool drop = false;
+        if (j >= n && !final_win) drop = true;
+        else if (me < p.rk_lines) {
+            drop = (p.rk_drop[me >> 5] >> (me & 31u)) & 1u;
+            if (me >= counted) fp += rk_fp(p, ws, i, me);
+        }
+        if (drop) rm_drop_run(p, i, n);
+    }
+    for (int o = 16; o; o >>= 1) fp += __shfl_xor_sync(0xFFFFFFFFu, fp, o);
+    if ((threadIdx.x & 31u) == 0 && fp) atomicAdd(&p.rk_cnt[RK_FP2], fp);
+}
+
+// Owner: the received records sorted by (tag, key, ord).  The first of each (tag, key) segment is the first occurrence;
+// every other one is a loser and goes back to its rank.
+static __global__ void __launch_bounds__(256) k_rm_decide(const uint4 *b0, const uint4 *b1, const unsigned *final_buf, u64 n, uint4 *lose,
+                                                          unsigned long long *cnt) {
+    const uint4 *r = *final_buf ? b1 : b0;
+    const u32 lane = threadIdx.x & 31u;
+    u32 c_uniq = 0, c_dup = 0;
+    const u64 n_round = (n + 31) & ~(u64)31;
+    for (u64 i = (u64)blockIdx.x * 256u + threadIdx.x; i < n_round; i += (u64)gridDim.x * 256u) {
+        bool loser = false;
+        uint4 x = make_uint4(0, 0, 0, 0);
+        if (i < n) {
+            x = r[i];
+            if (i > 0) { const uint4 y = r[i - 1]; loser = x.x == y.x && x.y == y.y && (x.w >> 31) == (y.w >> 31); }
+            if (loser) ++c_dup; else ++c_uniq;
+        }
+        const u32 b = __ballot_sync(0xFFFFFFFFu, loser);
+        unsigned long long base = 0;
+        if (lane == 0 && b) { base = atomicAdd(&cnt[RK_LOSE], (unsigned long long)__popc(b)); atomicAdd(&cnt[RK_LOSE + 1], (unsigned long long)__popc(b)); }
+        base = __shfl_sync(0xFFFFFFFFu, base, 0);
+        if (loser) lose[base + __popc(b & ((1u << lane) - 1u))] = x;
+    }
+    c_uniq = __reduce_add_sync(0xFFFFFFFFu, c_uniq); c_dup = __reduce_add_sync(0xFFFFFFFFu, c_dup);
+    if (lane == 0) { if (c_uniq) atomicAdd(&cnt[RK_UNIQ], (unsigned long long)c_uniq); if (c_dup) atomicAdd(&cnt[RK_DUP], (unsigned long long)c_dup); }
+}
+
+// Origin: the drop bit of every run head in `rec` (losers back from the owners, or this rank's own discards)
+static __global__ void __launch_bounds__(256) k_rm_settle(const uint4 *rec, u64 n, u32 rank, int check_rank, u64 lines, u32 *drop,
+                                                          unsigned long long *cnt) {
+    for (u64 i = (u64)blockIdx.x * 256u + threadIdx.x; i < n; i += (u64)gridDim.x * 256u) {
+        const uint4 x = rec[i];
+        const u64 ord = (u64)x.w << 32 | x.z, line = ord & RK_LINE_MASK;
+        if (line >= lines || (check_rank && ((ord >> 40) & 63u) != rank)) { atomicAdd(&cnt[RK_BAD], 1ull); continue; }
+        atomicOr(&drop[line >> 5], 1u << (line & 31u));
     }
 }
 

@@ -43,6 +43,28 @@ __device__ __forceinline__ u32 ld_acquire_sys_u32(const u32 *p) { u32 v; asm vol
 // part != NULL: the pairs are the `part[1]` records that END at index part[0] of `p` (both written on the device by the
 // producer, e.g. one sam2pairs window), and nothing is published: several such launches make up one epoch, closed by
 // k_xchg_publish.  part == NULL: p[0, n) is the rank's whole contribution and the last CTA publishes the epoch itself.
+//
+// Who owns a 16-byte record is a policy: the packed pairs' owner (above), the owner of a SAM-space krmdup key record
+// {key, ord} (mix(key, tag) mod world; the sender stamps its rank into ord on the way out), or the rank named in such a
+// record's ord (the way back to the record's origin).
+struct XcOwnPair {
+    static __device__ __forceinline__ u32 owner(const uint4 &r, u32 world, u32 res) { return xc_owner_hash(r.z & 0xFFFFu, r.z >> 16, r.x / res) % world; }
+    static __device__ __forceinline__ uint4 out(const uint4 &r, u32) { return r; }
+};
+struct XcOwnKey {                        // ord = tag << 63 | rank << 40 | line (s2p.cu, mk_s2p_rmdup_*)
+    static __device__ __forceinline__ u32 owner(const uint4 &r, u32 world, u32) {
+        u64 k = ((u64)r.y << 32 | r.x) ^ ((u64)(r.w >> 31) * 0x9E3779B97F4A7C15ull);
+        k ^= k >> 33; k *= 0xff51afd7ed558ccdull; k ^= k >> 33; k *= 0xc4ceb9fe1a85ec53ull; k ^= k >> 33;
+        return (u32)(k % world);
+    }
+    static __device__ __forceinline__ uint4 out(uint4 r, u32 rank) { r.w |= rank << 8; return r; }
+};
+struct XcOwnRank {
+    static __device__ __forceinline__ u32 owner(const uint4 &r, u32 world, u32) { return ((r.w >> 8) & (XC_MAX_WORLD - 1)) % world; }
+    static __device__ __forceinline__ uint4 out(const uint4 &r, u32) { return r; }
+};
+
+template <class Own>
 __global__ void __launch_bounds__(XC_T) k_xchg_scatter(const mk_pair *p, u64 n, const unsigned long long *part, XchgPeers peers, XchgCtrl *mine,
                                                         u32 world, u32 rank, u32 res, u32 epoch, u64 half_cap) {
     __shared__ uint4 s_pair[XC_TILE];
@@ -62,7 +84,8 @@ __global__ void __launch_bounds__(XC_T) k_xchg_scatter(const mk_pair *p, u64 n, 
             d[k] = 0xFFFFFFFFu;
             if (i < n) {
                 r[k] = ((const uint4 *)p)[i];
-                d[k] = xc_owner_hash(r[k].z & 0xFFFFu, r[k].z >> 16, r[k].x / res) % world;
+                d[k] = Own::owner(r[k], world, res);
+                r[k] = Own::out(r[k], rank);
                 atomicAdd(&s_cnt[d[k]], 1u);
             }
         }
@@ -112,7 +135,9 @@ __global__ void k_xchg_publish(XchgPeers peers, XchgCtrl *mine, u32 world, u32 r
     if (tid < world) st_release_sys_u32(&peers.ctrl[tid]->flag[rank], epoch);
 }
 
-// wait until every rank has delivered `epoch`, then publish the count
+// wait until every rank has delivered `epoch`, then publish the count.  A rank may already have published the next epoch
+// (one host thread driving several ranks of a two-step exchange, mk_s2p_rmdup_decide): it only does so after it has waited
+// for this epoch itself, so a flag at or past `epoch` means this epoch's data is in place.
 // (bounded: a peer that died or failed never publishes; after `timeout_ns` the wait gives up and reports which rank is missing
 // instead of hanging the GPU)
 __device__ __forceinline__ unsigned long long global_ns() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }
@@ -123,7 +148,7 @@ __global__ void k_xchg_wait(XchgCtrl *mine, u32 world, u32 epoch, unsigned long 
     __syncthreads();
     if (tid < world) {
         const unsigned long long t0 = global_ns();
-        while (ld_acquire_sys_u32(&mine->flag[tid]) != epoch) {
+        while ((int)(ld_acquire_sys_u32(&mine->flag[tid]) - epoch) < 0) {
             __nanosleep(200);
             if (global_ns() - t0 > timeout_ns) { atomicMax(&out[2], (unsigned long long)tid + 1ull); break; }
         }
@@ -230,7 +255,7 @@ extern "C" int mk_xchg_scatter_device(mk_xchg *x, const mk_pair *d_pairs, size_t
     x->epoch += 1;
     const u64 n_tiles = (n + XC_TILE - 1) / XC_TILE;
     const int grid = (int)std::max<u64>(1, std::min<u64>(n_tiles, (u64)x->sms * 4));
-    k_xchg_scatter<<<grid, XC_T, 0, (cudaStream_t)stream>>>(d_pairs, n, nullptr, x->peers, x->ctrl.as<XchgCtrl>(), (u32)x->world, (u32)x->rank, res, x->epoch, x->half_cap);
+    k_xchg_scatter<XcOwnPair><<<grid, XC_T, 0, (cudaStream_t)stream>>>(d_pairs, n, nullptr, x->peers, x->ctrl.as<XchgCtrl>(), (u32)x->world, (u32)x->rank, res, x->epoch, x->half_cap);
     x->launches += 1;
     MK_CUDA(cudaGetLastError());
     return MK_OK;
@@ -248,7 +273,7 @@ extern "C" int mk_xchg_begin(mk_xchg *x) {
 extern "C" int mk_xchg_scatter_part_device(mk_xchg *x, const mk_pair *d_base, const uint64_t *d_part, uint32_t res, void *stream) {
     if (!x || !d_base || !d_part || res == 0 || x->epoch == 0) { mk_set_error("mk_xchg_scatter_part_device: bad argument"); return MK_ERR_ARG; }
     MK_CUDA(cudaSetDevice(x->device));
-    k_xchg_scatter<<<x->sms * 2, XC_T, 0, (cudaStream_t)stream>>>(d_base, 0, (const unsigned long long *)d_part, x->peers, x->ctrl.as<XchgCtrl>(),
+    k_xchg_scatter<XcOwnPair><<<x->sms * 2, XC_T, 0, (cudaStream_t)stream>>>(d_base, 0, (const unsigned long long *)d_part, x->peers, x->ctrl.as<XchgCtrl>(),
                                                                   (u32)x->world, (u32)x->rank, res, x->epoch, x->half_cap);
     x->launches += 1;
     MK_CUDA(cudaGetLastError());
@@ -283,5 +308,24 @@ extern "C" int mk_xchg_finish_device(mk_xchg *x, mk_pair **d_recv, size_t *n_rec
     if (h[1] || h[0] > x->half_cap) { mk_set_error("mk_xchg_finish_device: rank %d was sent %llu pairs, capacity %zu", x->rank, h[0], x->half_cap); return MK_ERR_CAPACITY; }
     return MK_OK;
 }
+
+// 16-byte records of the multi-rank SAM-space krmdup (s2p.cu): owner 1 = the key's owner, 2 = the rank in the record's
+// ord.  d_part == NULL: the n records at d_rec are the rank's whole contribution to a new epoch, published at the end;
+// else one part of the epoch opened by mk_xchg_begin, as mk_xchg_scatter_part_device.
+int xchg_scatter_records(mk_xchg *x, const void *d_rec, u64 n, const unsigned long long *d_part, int owner, cudaStream_t s) {
+    if (!x || (owner != 1 && owner != 2)) { mk_set_error("xchg_scatter_records: bad argument"); return MK_ERR_ARG; }
+    if (!x->connected) { mk_set_error("xchg_scatter_records: mk_xchg_connect first"); return MK_ERR_STATE; }
+    MK_CUDA(cudaSetDevice(x->device));
+    if (!d_part) x->epoch += 1;
+    else if (x->epoch == 0) { mk_set_error("xchg_scatter_records: mk_xchg_begin first"); return MK_ERR_STATE; }
+    const u64 n_tiles = (n + XC_TILE - 1) / XC_TILE;
+    const int grid = d_part ? x->sms * 2 : (int)std::max<u64>(1, std::min<u64>(n_tiles, (u64)x->sms * 4));
+    auto k = owner == 1 ? k_xchg_scatter<XcOwnKey> : k_xchg_scatter<XcOwnRank>;
+    k<<<grid, XC_T, 0, s>>>((const mk_pair *)d_rec, n, d_part, x->peers, x->ctrl.as<XchgCtrl>(), (u32)x->world, (u32)x->rank, 1u, x->epoch, x->half_cap);
+    x->launches += 1;
+    MK_CUDA(cudaGetLastError());
+    return MK_OK;
+}
+void xchg_world_rank(const mk_xchg *x, int *world, int *rank) { *world = x->world; *rank = x->rank; }
 
 extern "C" uint64_t mk_xchg_launch_count(mk_xchg *x) { return x ? x->launches : 0; }
